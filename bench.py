@@ -14,7 +14,7 @@ A "step" is one pass of the hot path over one batch: reset every stream to its i
              loop and (b) SMs x 128 x 2 x max clock; plus the output stream's share of the measured HBM peak
   cpu_baseline : the reference C++ (oracle/_ref) on the host cores, one process per core, bounded sample
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--streams S] [--seconds T]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--streams S] [--seconds T] [--dump-outputs DIR]
 N>1 is launched with torch.distributed.run (one rank per GPU).
 """
 import argparse
@@ -64,7 +64,51 @@ def parse_args():
     ap.add_argument("--pull-players", type=int, default=148, help="--workload pull: players of the batched-pull leg")
     ap.add_argument("--long-seconds", type=float, default=3600.0)
     ap.add_argument("--long-rate", type=int, default=44100)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed (rank 0) as DIR/<name>.npy in float32 / "
+                         "float64, at most 64 MB in all: a fixed, seeded sample where the output is larger, so that two builds "
+                         "can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm renders in worker processes and keeps no outputs")
+    return args
+
+
+DUMP_BYTES = 64 * 10**6
+
+
+def dump_outputs(path, arrays):
+    """Write {name: float32 / float64 array} as path/<name>.npy; together they stay within DUMP_BYTES."""
+    import numpy as np
+    assert all(a.dtype in (np.float32, np.float64) for a in arrays.values())
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_BYTES, "--dump-outputs: %d bytes exceed the %d-byte budget" % (total, DUMP_BYTES)
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
+def sample_pcm(d_out, count, written, seed, points=1 << 20):
+    """What a caller receives -- int16 rows on the device, row i valid up to written[i] -- as float32 / float64 arrays:
+    `written` of every row; `points` at a seeded sample of positions over all rows (`points_index` = row * count + sample);
+    whole `rows` of a seeded sample of rows (`rows_index`), as many as the rest of DUMP_BYTES holds.  Samples past a row's
+    written count are not output and read as 0."""
+    import numpy as np
+    import torch
+    rows_n, stride = d_out.shape
+    rng = np.random.default_rng(seed)
+    flat = np.sort(rng.choice(rows_n * count, size=min(points, rows_n * count), replace=False))
+    r, c = flat // count, flat % count
+    pts = d_out.view(-1)[torch.from_numpy(r * stride + c).to(d_out.device)].cpu().numpy().astype(np.float32)
+    pts[c >= written[r]] = 0
+    left = DUMP_BYTES - rows_n * 8 - flat.size * 12 - (1 << 20)
+    sel = np.sort(rng.choice(rows_n, size=max(0, min(rows_n, left // (count * 4 + 8))), replace=False))
+    rows = d_out[torch.from_numpy(sel).to(d_out.device), :count].cpu().numpy().astype(np.float32)
+    rows[np.arange(count)[None, :] >= written[sel][:, None]] = 0
+    return {"written": written.astype(np.float64), "points": pts, "points_index": flat.astype(np.float64),
+            "rows": rows, "rows_index": sel.astype(np.float64)}
 
 
 class ClockSampler:
@@ -207,6 +251,8 @@ def long_arm(args, rank, world, local_rank):
             times.append(ms)
     clocks = sampler.stop() if rank == 0 else None
     ms = sum(times) / len(times)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, sample_pcm(d_out[None, :], n, np.array([got]), args.seed))
     # e2e: host frames in, host int16 out, wall clock around the C-ABI call
     h_out = np.zeros(n, dtype=np.int16)
     t0 = time.perf_counter()
@@ -284,7 +330,7 @@ def pull_arm(args, rank, world, local_rank):
         import torch.distributed as dist
         dist.init_process_group("gloo")
     sr, pull = args.sample_rate, args.pull_samples
-    warm, steps = max(args.warmup, 3), max(args.steps, 50)
+    warm, steps = max(args.warmup, 3), args.steps
     secs = (warm + steps + 2) * pull / sr
     fr, m, f, nul, ux = workloads.random_stream(5_000_000 + rank, secs, sr, seed=args.seed)
     fb = workloads._concat(sr, [(fr, m, f, nul, ux)], [5_000_000 + rank])
@@ -308,18 +354,18 @@ def pull_arm(args, rank, world, local_rank):
             if i >= warm:
                 ts.append(dt)
         p.close()
-        return np.array(ts)
+        return np.array(ts), c
 
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    res = {}
+    res, last = {}, {}
     for name, prec in (("stream", player.PRECISION_STREAM), ("fp32_serial", player.PRECISION_FP32)):
-        res[name] = timed_pulls(lambda: player.SpeechPlayer(sr, precision=prec, noise=player.NOISE_PHILOX, seed=args.seed,
-                                                            streamId=5_000_000 + rank))
+        res[name], last[name] = timed_pulls(lambda: player.SpeechPlayer(sr, precision=prec, noise=player.NOISE_PHILOX,
+                                                                        seed=args.seed, streamId=5_000_000 + rank))
     # many interactive players in one launch (speechPlayer_synthesizeBatch over stream handles: one block per player)
     nb = args.pull_players
-    bsecs = (warm + 12) * pull / sr
+    bsecs = (warm + steps + 2) * pull / sr
     bstreams = [workloads.random_stream(6_000_000 + rank * nb + k, bsecs, sr, seed=args.seed) for k in range(nb)]
     bps = [player.SpeechPlayer(sr, precision=player.PRECISION_STREAM, noise=player.NOISE_PHILOX, seed=args.seed,
                                streamId=6_000_000 + rank * nb + k) for k in range(nb)]
@@ -327,7 +373,7 @@ def pull_arm(args, rank, world, local_rank):
         p_.queue_frames(fr_, m_, f_, ux_, nul_)
     bts = []
     bh, bout, bw = player.batch_handles(bps), np.zeros((nb, pull), dtype=np.int16), np.zeros(nb, dtype=np.uint32)
-    for i in range(warm + 10):
+    for i in range(warm + steps):
         t0 = time.perf_counter()
         bout, bw = player.synthesize_batch(bps, pull, out=bout, written=bw, handles=bh)  # (a caller's loop reuses its buffers)
         dt = time.perf_counter() - t0
@@ -338,6 +384,9 @@ def pull_arm(args, rank, world, local_rank):
         p_.close()
     bts = np.array(bts)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"pull": last["stream"].astype(np.float32), "pull_fp32_serial": last["fp32_serial"].astype(np.float32),
+                                         "batch": bout.astype(np.float32), "batch_written": bw.astype(np.float64)})
     ts = res["stream"]
     total_s = float(ts.sum())
     if world > 1:
@@ -350,11 +399,11 @@ def pull_arm(args, rank, world, local_rank):
             from oracle import oracle
             if oracle.have_ref():
                 ref = oracle.RefLib(philox=False)
-                rts = timed_pulls(lambda: ref.player(sr))
+                rts, _ = timed_pulls(lambda: ref.player(sr))
                 kind = "reference"
             else:
                 port = oracle.PortLib()
-                rts = timed_pulls(lambda: port.player(sr))
+                rts, _ = timed_pulls(lambda: port.player(sr))
                 kind = "port"
             cpu = {"value": pull / sr / float(np.median(rts)), "unit": "audio-seconds/s", "cores": 1, "kind": kind,
                    "sample": "the same %d pulls of %d samples on one player, one core" % (steps, pull),
@@ -372,7 +421,7 @@ def pull_arm(args, rank, world, local_rank):
                            "l2": "not applicable: one block, working set in shared memory"},
                 "latency_ms": {"median": float(np.median(ts)) * 1e3, "p95": float(np.percentile(ts, 95)) * 1e3, "max": float(ts.max()) * 1e3,
                                "fp32_serial_kernel_median": float(np.median(res["fp32_serial"])) * 1e3},
-                "batch_of_players": {"players": nb, "samples_per_call": pull, "ms_per_call_median": float(np.median(bts)) * 1e3,
+                "batch_of_players": {"players": nb, "samples_per_call": pull, "calls": steps, "ms_per_call_median": float(np.median(bts)) * 1e3,
                                      "audio_seconds_per_s": nb * pull / sr / float(np.median(bts)),
                                      "note": "speechPlayer_synthesizeBatch over %d stream handles: one launch, one block per player" % nb},
                 "roofline": {"bound": "latency", "achieved": achieved, "peak": peak_tf, "unit": "TFLOP/s", "frac": achieved / peak_tf,
@@ -529,6 +578,8 @@ def main():
     rendered_all = float(rendered_all.item())                            # samples rendered per step, all ranks
     value = rendered_all / sr * args.steps / (elapsed_ms * 1e-3)          # audio-seconds per wall-second, whole job
     samples_per_s_gpu = rendered * args.steps / (elapsed_ms * 1e-3)       # per GPU
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, sample_pcm(d_out, count, d_written.cpu().numpy(), args.seed))
 
     # ---- e2e: host buffers through the C-ABI (H2D of the frames + D2H of the int16 inside the timed region) ----
     e2e = None

@@ -20,16 +20,19 @@ REF_DIR = os.path.join(HERE, "_ref")
 REF_SO = os.path.join(REF_DIR, "libspeechPlayer_ref.so")
 REF_PHILOX_SO = os.path.join(REF_DIR, "libspeechPlayer_ref_philox.so")
 PORT_SO = os.path.join(HERE, "libklatt_oracle.so")
+# A checkout of the original NVSpeechPlayer to compile the reference from; the repository does not contain one, and what
+# needs the reference itself (rather than the committed goldens rendered by it) skips without it.
+REFERENCE = os.environ.get("NVSP_REFERENCE_DIR", "")
 NUM_PARAMS = 47
 
 NOISE_LIBC, NOISE_PHILOX, NOISE_REPLAY = 0, 1, 2
 
 
-def build(reference="/root/reference", quiet=True):
+def build(reference=REFERENCE, quiet=True):
     """Compile the port always, and the reference .so files when the reference tree is present."""
     out = subprocess.DEVNULL if quiet else None
     subprocess.check_call(["make", "-C", HERE, "port"], stdout=out)
-    if os.path.isdir(os.path.join(reference, "src")):
+    if reference and os.path.isdir(os.path.join(reference, "src")):
         subprocess.check_call(["make", "-C", HERE, "ref", "REF=" + reference], stdout=out)
     return have_ref()
 
@@ -71,7 +74,7 @@ class RefLib:
     def __init__(self, philox=False):
         path = REF_PHILOX_SO if philox else REF_SO
         if not os.path.exists(path):
-            raise FileNotFoundError(path + " missing: run `make -C oracle ref` where /root/reference exists")
+            raise FileNotFoundError(path + " missing: run `make -C oracle ref REF=<NVSpeechPlayer checkout>`")
         self.philox = philox
         L = self.lib = ctypes.CDLL(path)
         L.speechPlayer_initialize.restype = ctypes.c_void_p

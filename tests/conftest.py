@@ -49,13 +49,10 @@ def port():
 
 @pytest.fixture(scope="session")
 def reflib():
-    """The compiled reference with Philox noise; present only where oracle/_ref was built (or travelled)."""
+    """The compiled reference with Philox noise: oracle/_ref, built from the NVSpeechPlayer checkout NVSP_REFERENCE_DIR names."""
     from oracle import oracle
-    if not oracle.have_ref():
-        if os.path.isdir("/root/reference/src"):
-            oracle.build(quiet=True)
-        else:
-            pytest.skip("oracle/_ref not available")
+    if not oracle.have_ref() and not oracle.build(quiet=True):
+        pytest.skip("oracle/_ref not built and NVSP_REFERENCE_DIR names no NVSpeechPlayer checkout")
     return oracle.RefLib(philox=True)
 
 

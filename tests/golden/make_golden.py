@@ -1,7 +1,7 @@
 """Regenerate the committed golden fixtures from the REFERENCE ITSELF.
 
-Run in the build container only (needs /root/reference and oracle/_ref built by
-`make -C oracle ref`); the GPU box has neither and only reads the .npz files.
+Run where an NVSpeechPlayer checkout is at hand (NVSP_REFERENCE_DIR names it; oracle/_ref is built
+from it); the tests only read the .npz files.
 
   config1.npz    BASELINE config 1: sampleIpa.txt through the reference's UNCHANGED
                  ipa.py + speechPlayer.py (recipe test_speakIpa.py:20-27, 22 050 Hz,
@@ -14,6 +14,9 @@ Run in the build container only (needs /root/reference and oracle/_ref built by
   phonemes       nvspeechplayer_b200/data/phoneme_table.npz: the numeric content of the
                  reference's data.py (49 phonemes x 47 params + flags) used by the
                  vowel-chart and midi-sing workload generators.
+  random_streams.npz  the random-frame streams of scenarios.RANDOM_STREAMS rendered by the
+                 compiled reference (Philox noise); `make_golden.py random_streams` writes
+                 only this file and needs only the compiled reference.
 """
 import ctypes
 import hashlib
@@ -29,7 +32,7 @@ sys.path.insert(0, ROOT)
 from oracle import oracle  # noqa: E402
 from tests import scenarios  # noqa: E402
 
-REF = "/root/reference"
+REF = oracle.REFERENCE
 HERE = os.path.dirname(os.path.abspath(__file__))
 SEED, STREAM = 0xB200, 0
 
@@ -128,6 +131,17 @@ def scenario_goldens():
     np.savez_compressed(os.path.join(HERE, "scenarios.npz"), **out)
 
 
+def random_stream_goldens():
+    """scenarios.RANDOM_STREAMS through the compiled reference with Philox noise, every frame queued up front."""
+    ref_px = oracle.RefLib(philox=True)
+    out = {}
+    for sr, sid in scenarios.RANDOM_STREAMS:
+        fr, m, f, nul, ux = scenarios.random_stream(sid, scenarios.RANDOM_SECONDS, sr)
+        out["%d_%d" % (sr, sid)] = ref_px.render(sr, fr, m, f, nul, ux, seed=scenarios.RANDOM_SEED, stream=sid)
+        print("random stream %d @ %d Hz: %d samples" % (sid, sr, out["%d_%d" % (sr, sid)].size))
+    np.savez_compressed(os.path.join(HERE, "random_streams.npz"), **out)
+
+
 class _RefAdapter:
     def __init__(self, lib, sr):
         lib.seed(scenarios.SEED, scenarios.STREAM)
@@ -148,6 +162,8 @@ class _RefAdapter:
 
 if __name__ == "__main__":
     assert oracle.build(REF, quiet=True), "reference .so not built"
-    ipa_mod = config1()
-    phoneme_table(ipa_mod)
-    scenario_goldens()
+    if sys.argv[1:] != ["random_streams"]:  # the one step that needs only the compiled reference, not its Python files
+        ipa_mod = config1()
+        phoneme_table(ipa_mod)
+        scenario_goldens()
+    random_stream_goldens()

@@ -1,5 +1,5 @@
-"""Regenerate tests/golden/ipa_frames.npz from the REFERENCE's own ipa.py (build container only: needs /root/reference
-and oracle/_ref).  For every (text, speed, basePitch, inflection, clauseType) case it stores what
+"""Regenerate tests/golden/ipa_frames.npz from the REFERENCE's own ipa.py (needs an NVSpeechPlayer checkout named by
+NVSP_REFERENCE_DIR, and oracle/_ref built from it).  For every (text, speed, basePitch, inflection, clauseType) case it stores what
 ipa.generateFramesAndTiming yields -- the 47 frame values (zeros + isNull for silence), durationMs, fadeMs -- so that the
 native bulk producer (include/speechPlayer_ipa.h) can be checked value for value where the reference is absent.
 

@@ -15,6 +15,9 @@ import numpy as np
 from nvspeechplayer_b200.workloads import NUM_PARAMS, P, PARAM_NAMES, RANDOM_RANGES, random_stream  # noqa: F401
 
 SEED, STREAM = 0xB200, 7  # Philox noise key used for every scenario
+# random-frame streams (sample rate, stream id) of 1.5 s with Philox key (RANDOM_SEED, stream id): what the live port-vs-reference
+# test renders, and what `tests/golden/make_golden.py random_streams` records from the reference
+RANDOM_STREAMS, RANDOM_SECONDS, RANDOM_SEED = ((16000, 31), (22050, 32), (44100, 33)), 1.5, 99
 
 
 def _rand_frame(rng):

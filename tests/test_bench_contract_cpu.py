@@ -27,6 +27,46 @@ def test_reference_arm_prints_one_contract_line():
     assert d["vs_baseline"] is None
 
 
+def test_steps_below_one_are_refused():
+    r = subprocess.run([sys.executable, "bench.py", "--impl", "reference", "--steps", "0"], cwd=ROOT, capture_output=True, text=True,
+                       timeout=120)
+    assert r.returncode == 2 and r.stdout == "" and "--steps" in r.stderr, (r.returncode, r.stderr[-300:])
+
+
+def test_dump_outputs_sample_what_the_rows_hold(tmp_path, monkeypatch):
+    """--dump-outputs: the seeded sample of a batch output (here a host tensor) is exactly what the rows hold, zero past each
+    row's written count, the same for the same seed, and a sample of whole rows when the output exceeds the budget."""
+    import numpy as np
+    import torch
+    monkeypatch.setenv("NCCL_DEBUG", "WARN")
+    monkeypatch.syspath_prepend(ROOT)
+    import bench
+    rows_n, stride, count = 300, 1008, 1000
+    out = np.random.default_rng(5).integers(-32768, 32768, size=(rows_n, stride)).astype(np.int16)
+    written = np.full(rows_n, count, dtype=np.int32)
+    written[::7] = 500
+    got = bench.sample_pcm(torch.from_numpy(out), count, written, 0xB200, points=5000)
+    assert all(a.dtype in (np.float32, np.float64) for a in got.values())
+    r, c = (got["points_index"] // count).astype(int), (got["points_index"] % count).astype(int)
+    assert len(set(got["points_index"])) == 5000 and (c < count).all()
+    np.testing.assert_array_equal(got["points"], np.where(c < written[r], out[r, c], 0))
+    sel = got["rows_index"].astype(int)
+    assert len(sel) == rows_n  # a small output fits whole
+    np.testing.assert_array_equal(got["rows"], np.where(np.arange(count)[None, :] < written[sel][:, None], out[sel, :count], 0))
+    np.testing.assert_array_equal(got["written"], written)
+    again = bench.sample_pcm(torch.from_numpy(out), count, written, 0xB200, points=5000)
+    assert all(np.array_equal(got[k], again[k]) for k in got)
+    bench.dump_outputs(str(tmp_path), got)
+    assert sorted(os.listdir(tmp_path)) == sorted(k + ".npy" for k in got)
+    np.testing.assert_array_equal(np.load(tmp_path / "rows.npy"), got["rows"])
+    # an output larger than the budget: whole rows of a sample of the rows, and the total stays within the budget
+    monkeypatch.setattr(bench, "DUMP_BYTES", 2_000_000)
+    part = bench.sample_pcm(torch.from_numpy(out), count, written, 0xB200, points=5000)
+    sel = part["rows_index"].astype(int)
+    assert 0 < len(sel) < rows_n and sum(a.nbytes for a in part.values()) <= bench.DUMP_BYTES
+    np.testing.assert_array_equal(part["rows"], np.where(np.arange(count)[None, :] < written[sel][:, None], out[sel, :count], 0))
+
+
 def test_reference_arm_other_ranks_exit_quietly():
     """Under torchrun (N > 1) rank 0 alone runs the reference arm; the other ranks exit 0 without work and without output."""
     env = dict(os.environ, RANK="1", LOCAL_RANK="1", WORLD_SIZE="2", MASTER_ADDR="127.0.0.1", MASTER_PORT="29533")

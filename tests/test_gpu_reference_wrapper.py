@@ -7,8 +7,10 @@ import sys
 import numpy as np
 import pytest
 
+from oracle import oracle
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
+REF = oracle.REFERENCE
 
 
 @pytest.mark.gpu
@@ -28,7 +30,8 @@ def test_untyped_wrapper_renders_config1_like_the_reference(tmp_path, golden_con
     assert exact >= 0.9999 and d.max() <= 1
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "src")), reason="needs the reference checkout (build container only)")
+@pytest.mark.skipif(not (REF and os.path.isdir(os.path.join(REF, "src"))),
+                    reason="needs the reference's own Python files: an NVSpeechPlayer checkout in NVSP_REFERENCE_DIR")
 def test_reference_python_files_load_and_queue_against_the_engine_library(tmp_path):
     """The reference's real speechPlayer.py / ipa.py / data.py, unmodified, in a throw-away package next to the engine's
     speechPlayer.dll: import, construct, run sampleIpa.txt through ipa.generateFramesAndTiming and queue every frame.

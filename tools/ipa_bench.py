@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Frame-producer throughput: the native bulk producer (include/speechPlayer_ipa.h) against the reference's ipa.py
-(build container only for the reference leg: it imports /root/reference through tests/golden/make_golden.py).
+(the reference leg runs when NVSP_REFERENCE_DIR names an NVSpeechPlayer checkout, imported through tests/golden/make_golden.py).
 Workload: the eight lines of sampleIpa.txt, speed 0.6, repeated; audio-seconds = sum of max(M+1, F+2) ticks / 22 050."""
 import os
 import sys
@@ -23,7 +23,7 @@ for threads in (1, 0):
     audio = float(fb.timeline_samples().sum()) / 22050.0
     print("native producer, %s: %d clauses, %d frames in %.3f s = %.0f clauses/s, %.3g audio-seconds/s"
           % ("1 thread" if threads == 1 else "%d threads" % os.cpu_count(), len(texts), int(fb.offsets[-1]), dt, len(texts) / dt, audio / dt))
-if os.path.isdir("/root/reference"):
+if os.environ.get("NVSP_REFERENCE_DIR"):
     sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
     from make_golden import oracle, reference_package
     ref_ipa, sp = reference_package(oracle.REF_SO)
