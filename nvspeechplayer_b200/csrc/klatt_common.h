@@ -91,7 +91,10 @@ constexpr int kNumDirect = 16;   // frame params used directly by the DSP each t
 //                   and end, plus the per-tick complex ratio of the pole written as 1 - omega.  A linear fade of
 //                   (f, bw) makes the pole a complex geometric sequence.  Only SMALL quantities are stored (zeta,
 //                   omega), never b~2, c~-1;  a = |zeta|^2 and rho = 1-|pole|^2 = 2*Re(zeta) - a follow per tick.
-//   vibrato       : phase increment per tick as 2^-64-cycle fixed point (start, per-tick change, end)
+//   vibrato       : phase increment per tick as 2^-64-cycle fixed point (start, per-tick change, end), and the depth
+//                   0.06 * vibratoPitchOffset (start, per-tick change, end) in double: a depth rounded to FP32 is a
+//                   constant pitch error of up to 2^-24 relative for the whole request, which the FP64 glottal phase
+//                   integrates and never forgets -- after minutes a sawtooth wrap lands on the neighbouring tick
 constexpr int kCoarseTicks = 64;  // drift control: every 64 samples the per-tick pole recurrence is re-based on a
                                    // 64-tick recurrence, so rounding bias accumulates over F/64 + 127 steps, not F
 struct alignas(16) FadePlanF32 {
@@ -101,6 +104,7 @@ struct alignas(16) FadePlanF32 {
 	float Wre[kNumResonators], Wim[kNumResonators];  // the same ratio over kCoarseTicks ticks at once
 	float dir0[kNumDirect], dirStep[kNumDirect], dirFinal[kNumDirect];
 	int64_t vibInc0, vibIncStep, vibIncFinal;
+	double depth0, depthStep, depthFinal;
 	uint32_t n0InvFade, n0InvFinal;  // anti-resonator inverted (cfN0 != 0, reference speechWaveGenerator.cpp:120) during / after the fade
 };
 static_assert(sizeof(FadePlanF32) % 16 == 0, "plan records are read with 16-byte loads");
@@ -126,11 +130,12 @@ struct GenStateF32 {
 	float zim[kNumResonators];
 	float dir[kNumDirect];         // current value of the directly used params
 	float zc[2 * kNumResonators];  // coarse-recurrence state (zeta re/im) of the fade in progress
+	double depth;                  // current vibrato depth, 0.06 * vibratoPitchOffset (FadePlanF32: in double)
 	FadePlanF32 plan;              // plan of the fade in progress when it was made inline (no precomputed plans)
 };
 
 // The same two blocks WITHOUT what a pre-queued (planned) FP32 stream never touches -- the three 47-double frames of the
-// frame manager and the inline fade plan: 544 bytes instead of 2.4 KB.  The block scheduler (klatt_f32_block.cu) keeps the
+// frame manager and the inline fade plan: 560 bytes instead of 2.4 KB.  The block scheduler (klatt_f32_block.cu) keeps the
 // streams of a call in a dense array of these (65 536 streams: 31 MB, resident in the 126 MB L2) and switches a stream
 // between the hold, fade and general loops every 64..128 ticks; members keep the names of the full structures so the
 // render bodies of klatt_f32_core.cuh work on either.
@@ -150,6 +155,8 @@ struct GenStateF32Lite {
 	float y[kNumResonators], d[kNumResonators], zre[kNumResonators], zim[kNumResonators];
 	float dir[kNumDirect];
 	float zc[2 * kNumResonators];
+	double depth;
+	uint32_t pad[2];
 };
 struct alignas(8) StreamStateLite {  // (8, not 16: the copies staged in shared memory sit on an 8-byte aligned stride)
 	FrameMgrLite fm;

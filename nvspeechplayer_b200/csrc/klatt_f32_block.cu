@@ -11,7 +11,7 @@
 //
 // Here a stream belongs to ONE thread block for the whole call (block b owns streams b, b + grid, b + 2 grid, ...), one
 // block of 16 warps = 8 workers per SM:
-//   * its state lives in a dense array of 544-byte StreamStateLite records (35 MB for 65 536 streams: L2-resident; only the
+//   * its state lives in a dense array of 560-byte StreamStateLite records (35 MB for 65 536 streams: L2-resident; only the
 //     owning SM ever touches a record, so plain cached loads are coherent and a fence.cta orders a hand-over).  A worker
 //     copies the 32 records of a cell into shared memory with coalesced 16-byte accesses, the render loops load and store
 //     their state THERE, and the records go back the same way (the first version let every lane read its own record word
@@ -38,8 +38,8 @@ constexpr int kBlkThreads = 512, kBlkWorkers = kBlkThreads / 64;
 constexpr uint32_t kClsHold = 0, kClsFade = 1, kClsGen = 2, kClsDone = 3, kClsExit = 4;
 constexpr uint32_t kCellTicks = kCoarseTicks;  // fade and general cells
 constexpr uint32_t kNoStream = 0xffffu;
-constexpr uint32_t kRecBytes = sizeof(StreamStateLite), kRecPieces = kRecBytes / 16;  // 544 B = 34 pieces of 16 bytes
-constexpr uint32_t kStageStride = kRecBytes + 8;  // bytes between the staged records of neighbouring lanes: 138 words, 2-way conflicts at most
+constexpr uint32_t kRecBytes = sizeof(StreamStateLite), kRecPieces = kRecBytes / 16;  // 560 B = 35 pieces of 16 bytes
+constexpr uint32_t kStageStride = kRecBytes + 8;  // bytes between the staged records of neighbouring lanes: 142 words, 2-way conflicts at most
 constexpr uint32_t kStageBytes = 32 * kStageStride;  // per worker
 
 struct BlockCtl {
@@ -123,6 +123,7 @@ klatt_block_import_kernel(const StreamDesc *__restrict__ descs, uint32_t numStre
 		for (int r = 0; r < kNumResonators; ++r) { L.f32.y[r] = gs.y[r]; L.f32.d[r] = gs.d[r]; L.f32.zre[r] = gs.zre[r]; L.f32.zim[r] = gs.zim[r]; }
 		for (int i = 0; i < kNumDirect; ++i) L.f32.dir[i] = gs.dir[i];
 		for (int i = 0; i < 2 * kNumResonators; ++i) L.f32.zc[i] = gs.zc[i];
+		L.f32.depth = gs.depth;
 	} else {  // init_states_kernel's fresh player (engine.cu)
 		L.fm.lastUserIndex = -1; L.fm.curIsNull = 1; L.fm.oldIsNull = 1;
 	}
@@ -150,6 +151,7 @@ klatt_block_export_kernel(const StreamDesc *__restrict__ descs, uint32_t numStre
 	for (int r = 0; r < kNumResonators; ++r) { gs.y[r] = L.f32.y[r]; gs.d[r] = L.f32.d[r]; gs.zre[r] = L.f32.zre[r]; gs.zim[r] = L.f32.zim[r]; }
 	for (int i = 0; i < kNumDirect; ++i) gs.dir[i] = L.f32.dir[i];
 	for (int i = 0; i < 2 * kNumResonators; ++i) gs.zc[i] = L.f32.zc[i];
+	gs.depth = L.f32.depth;
 	if (samplesWritten) samplesWritten[s] = L.f32.callPos;
 	if (results) {
 		StreamResult res;

@@ -18,7 +18,12 @@
 //    per request by planFade() in double.
 //  * pitch and glottal phase stay FP64 (src/speechWaveGenerator.cpp:55,74): the sawtooth turns phase error into
 //    full-scale error (a wrap that lands one sample early rings through every resonator), FP32 phase gives
-//    ~11 dB SNR.  Vibrato phase and its increment are 64-bit fixed point: exact accumulation, no drift.
+//    ~11 dB SNR.  Vibrato phase and its increment are 64-bit fixed point: exact accumulation, no drift.  The
+//    vibrato depth (0.06 * vibratoPitchOffset, lerped through fades) is FP64 too: the phase is never reset, so it
+//    integrates a constant pitch error for as long as the stream lives, and a depth rounded to FP32 (2^-24 relative)
+//    moved wraps to the neighbouring tick after 2-3 minutes of audio (61 dB SNR over 10 minutes, 92 dB in FP64).
+//    Only the vibrato sine is FP32: its gain is divided out of the depth (vibratoDepth), and its rounding changes from tick
+//    to tick and does not add up.
 //  * two-pole sections run in DELTA FORM:  d' = (1-rho)*d + a*(x - y);  y' = y + d'
 //    (a = |1-pole|^2, rho = 1-|pole|^2), algebraically the reference's  y' = a*x + b*y + c*y1  (b = 2 - rho - a,
 //    c = rho - 1; src :116-131) but only the SMALL quantities a, rho, d are represented, instead of cancelling
@@ -43,7 +48,8 @@
 
 namespace klatt {
 
-// slots of GenStateF32::dir
+// slots of GenStateF32::dir (dVibratoPitchOffset keeps the pair layout; the render paths carry the vibrato depth in
+// double instead: GenStateF32::depth, FadePlanF32::depth*)
 enum Direct : int {
 	dVibratoPitchOffset = 0, dVoiceTurbulenceAmplitude, dGlottalOpenQuotient, dVoiceAmplitude,
 	dAspirationAmplitude, dCaNP, dPa1, dPa2, dPa3, dPa4, dPa5, dPa6, dFricationAmplitude, dParallelBypass,
@@ -97,6 +103,14 @@ KLATT_HD int64_t vibratoIncrement(double speed, double srInv) {
 	return (int64_t)(t * 18446744073709551616.0);
 }
 
+// vibratoPitchOffset -> the depth the FP32 vibrato sine is multiplied by: pitch * (1 + sinTurns(t) * depth) is the reference's
+// pitch * (1 + sin(2*pi*t) * 0.06 * vibratoPitchOffset) (src/speechWaveGenerator.cpp:73).  The float coefficients of sinTurns
+// (2*pi itself is 2.8e-8 high in FP32) make its fundamental 3.861e-8 larger than sin's, and a gain error of the vibrato is a
+// pitch error the glottal phase integrates like a wrong depth (tests/test_long_stream_numerics_cpu.py measures the gain of
+// the compiled sinTurns); the depth divides it out.
+constexpr double kSinTurnsGain = 1.0 + 3.861e-8;
+KLATT_HD double vibratoDepth(double vibratoPitchOffset) { return vibratoPitchOffset * (0.06 / kSinTurnsGain); }
+
 KLATT_HD void planFade(const double *o, const double *n, uint32_t F, int sampleRate, FadePlanF32 &p) {
 	const double srInv = 1.0 / (double)sampleRate;
 	const double invF = 1.0 / (double)F;
@@ -106,6 +120,11 @@ KLATT_HD void planFade(const double *o, const double *n, uint32_t F, int sampleR
 		p.vibInc0 = vibratoIncrement(v0, srInv);
 		p.vibIncFinal = vibratoIncrement(v0 + ((v1 - v0) * 1.0), srInv);
 		p.vibIncStep = (p.vibIncFinal - p.vibInc0) / (int64_t)F;
+		double d0 = o[kVibratoPitchOffset], d1 = n[kVibratoPitchOffset];
+		if (d1 != d1) d1 = d0;
+		p.depth0 = vibratoDepth(d0);
+		p.depthStep = vibratoDepth((d1 - d0) * invF);
+		p.depthFinal = vibratoDepth(d0 + ((d1 - d0) * 1.0));
 	}
 	for (int i = 0; i < kNumDirect; ++i) {
 		double a = o[directParam(i)], b = n[directParam(i)];
@@ -207,8 +226,7 @@ KLATT_HD constexpr bool directOfParallel(int i) {
 	return i == dFricationAmplitude || (i >= dPa1 && i <= dPa6) || i == dParallelBypass || i == dPreFormantGain;
 }
 template <int ROLE> KLATT_HD constexpr bool roleUsesDirect(int i) {
-	return (RoleTraits<ROLE>::hasC && directOfCascade(i)) || (RoleTraits<ROLE>::hasP && directOfParallel(i)) ||
-	       (RoleTraits<ROLE>::hasO && i == dVibratoPitchOffset);
+	return (RoleTraits<ROLE>::hasC && directOfCascade(i)) || (RoleTraits<ROLE>::hasP && directOfParallel(i));
 }
 
 // hand-over between the two sides when they share a thread: plain members
@@ -303,12 +321,13 @@ struct DspState {  // what every tick reads AND writes
 	int64_t vibInc;
 	double pitchPos;         // glottal phase in cycles, FP64 like the reference's (parallel side)
 	double pitch, pitchInc;  // cur.voicePitch and its per-tick increment (parallel side)
+	double depth;            // vibrato depth 0.06 * cur.vibratoPitchOffset (the oscillators' side)
 };
 
 struct CoefF32 {  // what a tick only reads: a pure function of (zeta, direct params)
 	F2 a[kNumPairs], nrho[kNumPairs];  // |1 - pole|^2 and -(1 - |pole|^2)
 	float invA0;  // 1/a of the anti-resonator
-	float vpo, vta, goq, va, aa, caNP, bypass;
+	float vta, goq, va, aa, caNP, bypass;
 	F2 pa[3];
 	float halfGain, fricGain, og4000;
 	bool n0Inv;
@@ -352,7 +371,6 @@ KLATT_HD void buildCoef(CoefF32 &C, const F2 *u, const F2 *v, const F2 *dir, boo
 		C.bypass = half(dir, dParallelBypass);
 		C.fricGain = ((0.3f * kDrawScale) * half(dir, dFricationAmplitude)) * C.halfGain;
 	}
-	if (T::hasO) C.vpo = half(dir, dVibratoPitchOffset);
 }
 
 // one tick of the pole recurrences: zeta' = zeta + omega - zeta*omega (a no-op when omega == 0), on nz = -zeta:
@@ -527,7 +545,7 @@ KLATT_HD double divideBySampleRate(double x, double srD, double srInv) {
 // its other phases (pole recurrences, coefficients, the parallel bank), which do not depend on them; oscillatorSide()
 // below is the same segments back to back -- same operations, same bits.
 struct OscChain {
-	float t, u, q, vib;
+	float t, u, q;
 	double m, quot, pos;
 	KLATT_HD void seg1(DspState &S) {  // vibrato phase -> folded quarter-period argument
 		S.vibratoPos += (uint64_t)S.vibInc;
@@ -545,10 +563,9 @@ struct OscChain {
 		q = fmaf(u, q, -41.34170150756836f);
 		q = fmaf(t * u, q, t * 6.2831854820251465f);
 	}
-	KLATT_HD void seg3(DspState &S, float vpo) {  // pitch glide, pitch * (1 + vibrato)
-		vib = (q * 0.06f) * vpo;
+	KLATT_HD void seg3(DspState &S) {  // pitch glide, pitch * (1 + vibrato), the vibrato in FP64 from the FP32 sine
 		S.pitch += S.pitchInc;
-		m = S.pitch * ((double)vib + 1.0);
+		m = S.pitch * fma((double)q, S.depth, 1.0);
 	}
 	KLATT_HD void seg4(double srD, double srInv) { quot = divideBySampleRate(m, srD, srInv); }
 	KLATT_HD void seg5(DspState &S) {
@@ -560,7 +577,7 @@ struct OscChain {
 
 KLATT_HD float oscillatorSide(DspState &S, const CoefF32 &C, double srD, double srInv) {
 	OscChain o;
-	o.seg1(S); o.seg2(); o.seg3(S, C.vpo); o.seg4(srD, srInv); o.seg5(S);
+	o.seg1(S); o.seg2(); o.seg3(S); o.seg4(srD, srInv); o.seg5(S);
 	return o.seg6();
 }
 
@@ -643,7 +660,7 @@ KLATT_HD void loadDspState(DspState &S, const GS &gs) {
 	if (T::hasP) S.fricLast = gs.fricLast;
 	if (T::hasO) {
 		S.vibratoPos = gs.vibratoPos; S.vibInc = gs.vibInc;
-		S.pitchPos = gs.pitchPos; S.pitch = gs.pitch; S.pitchInc = gs.pitchInc;
+		S.pitchPos = gs.pitchPos; S.pitch = gs.pitch; S.pitchInc = gs.pitchInc; S.depth = gs.depth;
 	}
 }
 template <int ROLE, class GS>
@@ -655,7 +672,7 @@ KLATT_HD void storeDspState(GS &gs, const DspState &S) {
 	if (T::hasP) gs.fricLast = S.fricLast;
 	if (T::hasO) {
 		gs.vibratoPos = S.vibratoPos; gs.vibInc = S.vibInc;
-		gs.pitchPos = S.pitchPos; gs.pitch = S.pitch; gs.pitchInc = S.pitchInc;
+		gs.pitchPos = S.pitchPos; gs.pitch = S.pitch; gs.pitchInc = S.pitchInc; gs.depth = S.depth;
 	}
 }
 
@@ -781,6 +798,7 @@ KLATT_HD uint32_t renderGeneralF32T(FM &fm, GS &gs, const StreamDesc &desc, int 
 	F2 dir0[kNumDirectPairs], dstep[kNumDirectPairs];
 	float kf = 0.0f, kfStep = 0.0f;
 	int64_t vibIncStep = 0;
+	double depthStep = 0.0;  // S.depth advances by it on every tick (an FP64 sum: ~F ulps off the lerp, far below FP32's 2^-24)
 #pragma unroll
 	for (int r = T::R0; r < T::R1; ++r) { half(u, r) = -gs.zre[r]; half(v, r) = -gs.zim[r]; half(wr, r) = 0.0f; half(wi, r) = 0.0f; }
 #pragma unroll
@@ -819,6 +837,7 @@ KLATT_HD uint32_t renderGeneralF32T(FM &fm, GS &gs, const StreamDesc &desc, int 
 			kf = (float)counter;
 			kfStep = 1.0f;
 			vibIncStep = plan->vibIncStep;
+			depthStep = plan->depthStep;
 		}
 	}
 	uint32_t coarseAt = hasNew ? gs.coarseAt : 0x80000000u;
@@ -857,6 +876,7 @@ KLATT_HD uint32_t renderGeneralF32T(FM &fm, GS &gs, const StreamDesc &desc, int 
 						kf = 0.0f; kfStep = 1.0f;
 						if (T::hasO) {
 							S.vibInc = plan->vibInc0; vibIncStep = plan->vibIncStep;
+							S.depth = plan->depth0; depthStep = plan->depthStep;
 							const double pitchOld = gs.pitchOld, pitchNew = gs.pitchNew;
 							S.pitch = pitchOld;
 							S.pitchInc = (pitchNew != pitchNew) ? 0.0 : (pitchNew - pitchOld) / (double)newF;
@@ -879,6 +899,7 @@ KLATT_HD uint32_t renderGeneralF32T(FM &fm, GS &gs, const StreamDesc &desc, int 
 							S.pitch = (pitchNew != pitchNew) ? pitchOld : pitchOld + ((pitchNew - pitchOld) * 1.0);
 							S.pitchInc = 0.0;
 							S.vibInc = plan->vibIncFinal; vibIncStep = 0;
+							S.depth = plan->depthFinal; depthStep = 0.0;
 						}
 						nextEvent = newF + 1;
 					}
@@ -967,7 +988,7 @@ KLATT_HD uint32_t renderGeneralF32T(FM &fm, GS &gs, const StreamDesc &desc, int 
 			const bool oscHere = T::hasO && !T::hasC;  // the parallel warp of a pair carries the oscillators
 			OscChain osc;
 			kf += kfStep;
-			if (T::hasO) S.vibInc += vibIncStep;
+			if (T::hasO) { S.vibInc += vibIncStep; S.depth += depthStep; }
 			if (KLATT_UNLIKELY((gen & (uint64_t)(kCoarseTicks - 1)) == 0 && kfStep != 0.0f)) {
 				// drift control, on a grid of ABSOLUTE sample indices (identical for every chunking of the render, and
 				// the same loop iteration for every lane of a batch that started together): the poles of this tick come
@@ -1001,7 +1022,7 @@ KLATT_HD uint32_t renderGeneralF32T(FM &fm, GS &gs, const StreamDesc &desc, int 
 #pragma unroll
 				for (int k = 0; k < kNumDirectPairs; ++k)
 					if (roleUsesDirectPair<ROLE>(k)) dir[k] = fma2(kf2, dstep[k], dir0[k]);
-				if (oscHere) osc.seg3(S, half(dir, dVibratoPitchOffset));
+				if (oscHere) osc.seg3(S);
 				buildCoef<ROLE>(C, u, v, dir, n0Inv);
 			}
 			if (oscHere) osc.seg4(srD, srInv);
@@ -1104,6 +1125,7 @@ KLATT_HD void renderFadeF32T(FM &fm, GS &gs, const StreamDesc &desc, int sampleR
 		}
 	float kf = (float)counter;
 	const int64_t vibIncStep = plan->vibIncStep;
+	const double depthStep = plan->depthStep;
 	const bool n0Inv = gs.n0Inv != 0;
 	uint64_t gen = gs.samplesGenerated;
 	const uint64_t streamId = desc.streamId;
@@ -1145,7 +1167,7 @@ KLATT_HD void renderFadeF32T(FM &fm, GS &gs, const StreamDesc &desc, int sampleR
 					OscChain osc;
 					counter++;
 					kf += 1.0f;
-					if (T::hasO) S.vibInc += vibIncStep;
+					if (T::hasO) { S.vibInc += vibIncStep; S.depth += depthStep; }
 					if (t + k + h != 0) stepPoles<ROLE>(u, v, wr, wi);
 					if (oscHere) { osc.seg1(S); osc.seg2(); }
 					CoefF32 C;
@@ -1155,7 +1177,7 @@ KLATT_HD void renderFadeF32T(FM &fm, GS &gs, const StreamDesc &desc, int sampleR
 #pragma unroll
 						for (int q = 0; q < kNumDirectPairs; ++q)
 							if (roleUsesDirectPair<ROLE>(q)) dir[q] = fma2(kf2, dstep[q], dir0[q]);
-						if (oscHere) osc.seg3(S, half(dir, dVibratoPitchOffset));
+						if (oscHere) osc.seg3(S);
 						buildCoef<ROLE>(C, u, v, dir, n0Inv);
 					}
 					if (oscHere) osc.seg4(srD, srInv);

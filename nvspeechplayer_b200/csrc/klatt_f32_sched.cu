@@ -15,7 +15,7 @@
 #include "out_writer.cuh"
 #include "klatt_f32_pair.cuh"
 
-// KLATT_SCHED_LITE (default 1, round 2): the streams of a call live in a dense array of 544-byte StreamStateLite records
+// KLATT_SCHED_LITE (default 1, round 2): the streams of a call live in a dense array of 560-byte StreamStateLite records
 // (klatt_common.h; 35 MB for 65 536 streams: L2-resident) instead of the 2.4 KB AoS blocks; a worker copies the 32 records of
 // its chunk into shared memory with coalesced 16-byte ld.global.cg, the render loops load and store their state (and the
 // drift-control record zc, every 64 fade ticks) THERE, and the records go back with st.global.cg before the fence and the

@@ -129,6 +129,19 @@ struct DirWalk {
 	}
 };
 
+// the vibrato depth 0.06 * vibratoPitchOffset along the stream, in double like the serial kernels' (klatt_common.h FadePlanF32)
+struct DepthWalk {
+	double prevFinal, d0, ds, dF;
+	__device__ void load(const LongStream &L, uint32_t j) {
+		prevFinal = j > 0 ? L.plans[j - 1].depthFinal : 0.0;
+		const FadePlanF32 &p = L.plans[j];
+		d0 = p.depth0; ds = p.depthStep; dF = p.depthFinal;
+	}
+	__device__ __forceinline__ double at(uint32_t c, uint32_t F) const {
+		return c == 0 ? prevFinal : (c < F ? fma((double)(float)c, ds, d0) : dF);
+	}
+};
+
 // zeta = 1 - pole of one section along the stream
 struct PoleWalk {
 	float zr, zi, wr, wi;
@@ -410,14 +423,15 @@ klatt_long_timeline_kernel(LongStream L) {
 struct SourceWalk {
 	Cursor cur;
 	VibWalk vw;
-	DirWalk vpo, vta, goq, va, aa, fa, pfg;
+	DepthWalk depth;
+	DirWalk vta, goq, va, aa, fa, pfg;
 	uint64_t vibPos;
 	uint32_t loaded;
 	double pPop, pOld, pNew, pInc;  // pitch of the request in force: stale pop-tick value, fade end points, hold glide
 	double pitchHold;               // cur.voicePitch while holding, accumulated like the reference does (src/frame.cpp:77)
 	__device__ void loadReq(const LongStream &L, bool full) {
 		vw.load(L, cur.j);
-		vpo.load(L, cur.j, dVibratoPitchOffset);
+		depth.load(L, cur.j);
 		if (full) {
 			vta.load(L, cur.j, dVoiceTurbulenceAmplitude); goq.load(L, cur.j, dGlottalOpenQuotient);
 			va.load(L, cur.j, dVoiceAmplitude); aa.load(L, cur.j, dAspirationAmplitude);
@@ -436,21 +450,22 @@ struct SourceWalk {
 		// in the middle of a hold: the value the previous tick used, (c-1) - F - 1 additions after the landing
 		if (cur.c >= cur.F + 2) pitchHold = glideExact(landing(), pInc, (uint64_t)(cur.c - cur.F - 2));
 	}
-	// The increment of the glottal phase on this tick, exactly the double the serial kernel adds (klatt_f32_core.cuh OscChain:
-	// vibrato sine in FP32, pitch * (1 + vibrato) and the correctly rounded division by the sample rate in FP64; reference
-	// src/speechWaveGenerator.cpp:73-74).  cur.voicePitch: stale on the pop tick, old+(new-old)*ratio in the fade
+	// The increment of the glottal phase on this tick, the double the serial kernel adds (klatt_f32_core.cuh OscChain:
+	// vibrato sine in FP32, its depth, pitch * (1 + vibrato) and the correctly rounded division by the sample rate in FP64; reference
+	// src/speechWaveGenerator.cpp:73-74).  In a fade the serial kernels sum the depth's steps where this evaluates the depth in
+	// closed form: the two differ by a few FP64 ulps.  cur.voicePitch: stale on the pop tick, old+(new-old)*ratio in the fade
 	// (src/frame.cpp:49-52), the landing value on the landing and swap ticks, then += inc per tick (:77).
 	__device__ __forceinline__ double quotOfTick(double srD, double srInv) {
 		const uint32_t c = cur.c, F = cur.F;
 		vibPos += (uint64_t)vw.inc(c, F);
 		float vph = (float)(int32_t)(uint32_t)(vibPos >> 32) * 2.3283064365386963e-10f;
-		float vib = (sinTurns(vph) * 0.06f) * vpo.at(c, F);
+		const double vib1 = fma((double)sinTurns(vph), depth.at(c, F), 1.0);
 		double pitch;
 		if (c == 0) pitch = pPop;
 		else if (c < F) pitch = (pNew != pNew) ? pOld : pOld + ((pNew - pOld) * ((double)c / (double)F));
 		else if (c <= F + 1) { pitch = landing(); pitchHold = pitch; }
 		else { pitchHold += pInc; pitch = pitchHold; }
-		const double m = pitch * ((double)vib + 1.0);
+		const double m = pitch * vib1;
 		return divideBySampleRate(m, srD, srInv);
 	}
 	__device__ __forceinline__ void next(const LongStream &L, bool full) {

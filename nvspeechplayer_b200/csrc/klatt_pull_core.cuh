@@ -36,6 +36,7 @@ struct alignas(16) PullSeg {
 	double pitchInc;                        // hold glide (frame.cpp:77,98)
 	uint64_t vibPosAtPop;                   // vibrato phase before the pop tick, 2^-64 cycles
 	int64_t vibIncStale;                    // vibrato increment on the pop tick
+	double depthStale;                      // vibrato depth 0.06 * vibratoPitchOffset on the pop tick
 	float dirStale[kNumDirect];             // direct params on the pop tick (curFrame is not touched there, frame.cpp:55-72)
 	float zStaleRe[kNumResonators], zStaleIm[kNumResonators];
 	uint32_t n0InvStale;
@@ -43,7 +44,7 @@ struct alignas(16) PullSeg {
 	uint32_t c0;         // sampleCounter on the run's first tick (0 = the pop tick)
 	uint32_t tickStart;  // first tick of the run, counted from the start of the pull
 	uint32_t count;
-	uint32_t pad[3];
+	uint32_t pad[1];
 };
 static_assert(sizeof(PullSeg) % 16 == 0, "segments are copied as 16-byte words");
 
@@ -120,6 +121,11 @@ KLATT_HD double pullPitchAt(const PullSeg &s, uint32_t c) {
 
 KLATT_HD float pullDirAt(const PullSeg &s, int slot, uint32_t c) {
 	return c == 0 ? s.dirStale[slot] : (c < s.F ? fmaf((float)c, s.plan.dirStep[slot], s.plan.dir0[slot]) : s.plan.dirFinal[slot]);
+}
+
+// the vibrato depth 0.06 * vibratoPitchOffset on tick (seg, c), in double (klatt_common.h FadePlanF32)
+KLATT_HD double pullDepthAt(const PullSeg &s, uint32_t c) {
+	return c == 0 ? s.depthStale : (c < s.F ? fma((double)(float)c, s.plan.depthStep, s.plan.depth0) : s.plan.depthFinal);
 }
 
 KLATT_HD bool pullN0InvAt(const PullSeg &s, uint32_t c) {
@@ -274,8 +280,7 @@ struct PullOsc {  // vibrato + pitch along the pull
 		const PullSeg &S = X.segs[cur.s];
 		vibPos += (uint64_t)pullVibInc(S, cur.c);
 		float vph = (float)(int32_t)(uint32_t)(vibPos >> 32) * 2.3283064365386963e-10f;
-		float vib = (sinTurns(vph) * 0.06f) * pullDirAt(S, dVibratoPitchOffset, cur.c);
-		double m = pitch(S) * ((double)vib + 1.0);
+		double m = pitch(S) * fma((double)sinTurns(vph), pullDepthAt(S, cur.c), 1.0);
 		return divideBySampleRate(m, srD, srInv);
 	}
 	KLATT_HD void next(const PullCtx &X) {

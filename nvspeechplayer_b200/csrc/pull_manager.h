@@ -166,6 +166,7 @@ private:
 		for (int i = 0; i < kNumDirect; ++i) info.dirStale[i] = (float)cur[directParam(i)];
 		info.n0InvStale = cur[kCfN0] != 0;
 		info.vibIncStale = vibratoIncrement(cur[kVibratoSpeed], srInv);
+		info.depthStale = vibratoDepth(cur[kVibratoPitchOffset]);
 		info.vibPosAtPop = vibPos;
 		info.pitchStale = cur[kVoicePitch];
 		info.pitchOld = reqOld[kVoicePitch];

@@ -437,3 +437,9 @@ extern "C" void hostsim_pull_pitch_walk(double pitchOld, double pitchNew, double
 		out[i] = w.pitch(seg);
 	}
 }
+
+// the vibrato sine of every FP32 path (klatt_f32_core.cuh sinTurns) and the depth that multiplies it
+extern "C" void hostsim_sin_turns(const float *t, uint32_t n, float *out) {
+	for (uint32_t i = 0; i < n; ++i) out[i] = sinTurns(t[i]);
+}
+extern "C" double hostsim_vibrato_depth(double vibratoPitchOffset) { return vibratoDepth(vibratoPitchOffset); }

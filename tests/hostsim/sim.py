@@ -148,3 +148,21 @@ def phase(inc, pos0, mode):
     carry = ctypes.c_double(0)
     visited = L.hostsim_phase(inc.ctypes.data, len(inc), float(pos0), int(mode), out.ctypes.data, ctypes.byref(carry))
     return out, carry.value, visited
+
+
+def sin_turns(t):
+    """sinTurns (the FP32 vibrato sine of every FP32 path) of float32 phases in turns, |t| <= 0.5"""
+    L = lib()
+    L.hostsim_sin_turns.argtypes = [ctypes.c_void_p, ctypes.c_uint, ctypes.c_void_p]
+    t = np.ascontiguousarray(t, dtype=np.float32)
+    out = np.empty_like(t)
+    L.hostsim_sin_turns(t.ctypes.data, len(t), out.ctypes.data)
+    return out
+
+
+def vibrato_depth(vibrato_pitch_offset):
+    """what the FP32 paths multiply the vibrato sine by for a frame's vibratoPitchOffset"""
+    L = lib()
+    L.hostsim_vibrato_depth.restype = ctypes.c_double
+    L.hostsim_vibrato_depth.argtypes = [ctypes.c_double]
+    return L.hostsim_vibrato_depth(float(vibrato_pitch_offset))

@@ -38,3 +38,45 @@ def assert_f32_parity(got, want, what="", within=F32_WITHIN_1LSB, snr_db=F32_SNR
     short_and_tight = len(want) <= 10000 and mx <= 1
     assert snr >= snr_db or quiet or short_and_tight, "%s: SNR %.1f dB (max %g)" % (what, snr, mx)
     return w1, exact, snr, mx
+
+
+def clusters(got, want, gap=2000):
+    """Runs of samples off by more than 1 LSB, split where two of them are more than `gap` samples apart:
+    [(first index, length, peak |d|)]."""
+    n = min(len(got), len(want))
+    d = np.abs(np.asarray(got[:n], dtype=np.int64) - np.asarray(want[:n], dtype=np.int64))
+    bad = np.nonzero(d > 1)[0]
+    if len(bad) == 0:
+        return []
+    runs = np.split(bad, np.nonzero(np.diff(bad) > gap)[0] + 1)
+    return [(int(r[0]), int(r[-1] - r[0] + 1), int(d[r[0]:r[-1] + 1].max())) for r in runs]
+
+
+def where_in_queue(index, min_dur, fade_dur):
+    """(request, tick in that request, "pop" / "fade" / "hold") of output sample `index` of a queue rendered from a fresh
+    player: request j occupies max(M+1, F+2) ticks (F = max(fadeDuration, 1)); its tick 0 pops it, ticks 1..F-1 fade."""
+    m = np.asarray(min_dur, dtype=np.int64)
+    f = np.maximum(np.asarray(fade_dur, dtype=np.int64), 1)
+    start = np.concatenate([[0], np.cumsum(np.maximum(m + 1, f + 2))])
+    j = int(np.searchsorted(start, index, side="right") - 1)
+    c = int(index - start[j])
+    return j, c, "pop" if c == 0 else ("fade" if c < f[min(j, len(f) - 1)] else "hold")
+
+
+def assert_whole_stream(got, want, what, max_abs, snr_db, min_dur=None, fade_dur=None):
+    """Maximum |difference| and SNR over the WHOLE stream (a long render must not hide a burst in its average).  On failure
+    the message lists every cluster of samples off by more than 1 LSB (first index, length, peak), and, given the queue
+    (min_dur, fade_dur), the request, tick and phase each cluster starts in."""
+    assert len(got) == len(want), "%s: %d vs %d samples" % (what, len(got), len(want))
+    w1, exact, snr, mx = metrics(got, want)
+    print("parity %-44s n=%8d  <=1LSB %.6f  exact %.6f  SNR %6.1f dB  max|d| %g  (whole stream)" % (what, len(want), w1, exact, snr, mx))
+    if mx <= max_abs and snr >= snr_db:
+        return w1, exact, snr, mx
+    lines = []
+    for first, length, peak in clusters(got, want):
+        line = "  at sample %d: %d samples, peak %d" % (first, length, peak)
+        if min_dur is not None and fade_dur is not None:
+            line += "  request %d tick %d (%s)" % where_in_queue(first, min_dur, fade_dur)
+        lines.append(line)
+    raise AssertionError("%s: SNR %.1f dB (bar %.1f), max|d| %g (bar %g), %d clusters of |d| > 1:\n%s"
+                         % (what, snr, snr_db, mx, max_abs, len(lines), "\n".join(lines)))
