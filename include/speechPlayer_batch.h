@@ -141,6 +141,29 @@ long long speechPlayer_synthesizeLong(int sampleRate, const speechPlayer_frame_t
                                       unsigned long long maxSamples, int outOnDevice, double *renderMs,
                                       unsigned long long *kernelLaunches);
 
+/* Many pre-queued streams rendered with parallelism in time (the long-utterance path above), all streams' chunks in one
+ * launch sequence (streams are taken in consecutive groups of at most NVSP_LONG_BATCH_TICKS ticks, default 2^28).
+ * Inputs are HOST arrays in the layout of speechPlayer_batchSetFramesHost: stream s owns requests [offsets[s], offsets[s+1]).
+ * Stream s renders what speechPlayer_synthesizeLong(sampleRate, <its requests>, seed, streamIds[s], chunkTicks,
+ * maxSamples[s]) renders (Philox noise keyed (seed, streamIds[s]); streamIds NULL = 0..N-1).  Its glottal phase and its
+ * excitation are bit for bit the same; the start state of a resonator chunk comes from a double-precision scan whose
+ * association depends on where the stream sits among the scan's blocks, so a sample may in rare cases differ by a last-bit
+ * rounding from the solo render.  That is the only source of difference.
+ *   chunkTicks   : 0 = 1024, halved (down to 64) while a group has too few chunks to fill the GPU
+ *   maxSamples   : HOST u64 [numStreams] cap per stream, or NULL = the whole queue
+ *   outOffsets   : HOST int64 [numStreams + 1], filled: stream s's samples are out[outOffsets[s] .. outOffsets[s+1])
+ *   out          : packed int16 (HOST, or DEVICE when outOnDevice); NULL = size query only (no device work, no device needed)
+ *   serialPhase  : HOST u8 [numStreams] or NULL: 1 where that stream's glottal phase took the serial fallback
+ *   renderMs     : (optional) device time of the groups' launch sequences, summed
+ * Returns the total samples written (= outOffsets[numStreams]) or -1 (speechPlayer_lastError()). */
+long long speechPlayer_synthesizeLongBatch(int sampleRate, unsigned int numStreams, const int64_t *offsets,
+                                           const speechPlayer_frame_t *frames, const unsigned int *minFrameDuration,
+                                           const unsigned int *fadeDuration, const unsigned char *isNull, uint64_t seed,
+                                           const uint64_t *streamIds, unsigned int chunkTicks,
+                                           const unsigned long long *maxSamples, sample *out, int64_t *outOffsets,
+                                           int outOnDevice, unsigned char *serialPhase, double *renderMs,
+                                           unsigned long long *kernelLaunches);
+
 /* Pure host helper (no device needed): samples a fully pre-queued stream yields,
  * sum_j max(M_j+1, max(F_j,1)+2)  -- the occupancy law of the reference frame manager (src/frame.cpp:41-80). */
 unsigned long long speechPlayer_timelineSamples(const unsigned int *minFrameDuration,

@@ -1,6 +1,8 @@
-// klatt_long: the long-utterance path.  ONE pre-queued stream is cut into chunks of L ticks and every chunk is
-// rendered by its own thread, all chunks at once.  What a chunk needs from its past is recovered in closed form
-// or by a scan instead of by running the past:
+// klatt_long: the long-utterance path.  Pre-queued streams are cut into chunks of L ticks and every chunk is rendered by
+// its own thread, all chunks of all streams of a launch at once (LongTable: one stream for speechPlayer_synthesizeLong,
+// many for speechPlayer_synthesizeLongBatch).  A chunk kernel maps its chunk to (stream, chunk of the stream) and works in
+// that stream's own ticks; every scan restarts at a stream's first chunk.  What a chunk needs from its past is recovered
+// in closed form or by a scan instead of by running the past:
 //
 //   frame manager   the occupancy law max(M+1, F+2) (reference src/frame.cpp:41-80) gives every request its first
 //                   tick by a prefix sum; a chunk finds its request by bisection and its position in the fade / hold
@@ -37,6 +39,8 @@
 
 namespace klatt {
 
+// One stream of a launch: pointers into the flat arrays of all the launch's requests at this stream's offset.  (Mirrored
+// field for field in engine.cu, which builds the table on the host.)
 struct LongStream {
 	const double *frames;      // [nReq][47]
 	const uint32_t *minDur, *fadeDur;
@@ -45,15 +49,49 @@ struct LongStream {
 	uint32_t nReq;
 	int sampleRate;
 	uint64_t seed, streamId;
+	uint64_t cap;              // ticks rendered: the timeline is cut here (start[nReq] = min(ticks the queue yields, cap))
+	uint64_t outBase;          // where the stream's tick 0 goes in the launch's packed int16 output
 	// made by klatt_long_timeline_kernel
-	uint64_t *start;        // [nReq+1] tick of each request's pop tick; start[nReq] = ticks the stream yields
+	uint64_t *start;        // [nReq+1] tick of each request's pop tick; start[nReq] = ticks rendered
 	int32_t *prevReal;      // [nReq] last non-NULL request before j, or -1
 	double *pitchPop;       // [nReq] cur.voicePitch on the pop tick (stale value)
 	double *pitchOld, *pitchNew, *pitchInc;  // [nReq] fade end points and hold glide
 	uint64_t *vibPosStart;  // [nReq] vibrato phase before the pop tick
 };
 
+// The streams of one launch.  Stream s owns the chunks [chunkBase[s], chunkBase[s+1]) (chunkBase: exclusive scan of
+// ceil(ticks_s / L)); its tick t lives at VIRTUAL tick chunkBase[s] * L + t of the signal arrays, so every chunk starts on
+// a multiple of L as it does for one stream, and the gap between two streams is under L ticks.
+struct LongTable {
+	const LongStream *streams;   // [numStreams]
+	const uint32_t *chunkBase;   // [numStreams + 1]
+	uint32_t numStreams;
+	LongStream one;              // streams[0] by value: a one-stream launch reads its stream from the parameter bank
+};
+
 namespace {
+
+// Every chunk kernel is instantiated twice from the same code: MULTI = false for a one-stream launch (the stream's fields
+// are kernel parameters, as the per-tick walks want them: reading them from a table in global memory made config 4 24 % slower) and
+// MULTI = true for a table of streams.
+// the stream that owns chunk ch: the last s with chunkBase[s] <= ch (empty streams own no chunk)
+template <bool MULTI>
+__device__ __forceinline__ uint32_t streamOfChunk(const LongTable &T, uint32_t ch) {
+	if (!MULTI) return 0;
+	uint32_t lo = 0, hi = T.numStreams;
+	while (hi - lo > 1) {
+		const uint32_t mid = (lo + hi) >> 1;
+		if (T.chunkBase[mid] <= ch) lo = mid; else hi = mid;
+	}
+	return lo;
+}
+template <bool MULTI>
+__device__ __forceinline__ const LongStream &streamAt(const LongTable &T, uint32_t s) { return MULTI ? T.streams[s] : T.one; }
+// first chunk of stream s, and one past its last
+template <bool MULTI>
+__device__ __forceinline__ uint32_t chunkBegin(const LongTable &T, uint32_t s) { return MULTI ? T.chunkBase[s] : 0u; }
+template <bool MULTI>
+__device__ __forceinline__ uint32_t chunkEnd(const LongTable &T, uint32_t s, uint32_t numChunks) { return MULTI ? T.chunkBase[s + 1] : numChunks; }
 
 constexpr int kWarmTicks = 64;
 
@@ -264,8 +302,11 @@ __device__ __forceinline__ uint64_t tileScanAdd(uint64_t v, uint64_t *buf) {
 	return buf[tid];
 }
 
+// one block per stream: block s walks streams[s]
+template <bool MULTI>
 __global__ void __launch_bounds__(kTimelineTile)
-klatt_long_timeline_kernel(LongStream L) {
+klatt_long_timeline_kernel(LongTable T) {
+	const LongStream &L = streamAt<MULTI>(T, blockIdx.x);
 	__shared__ uint64_t scanBuf[kTimelineTile];
 	__shared__ uint8_t sNull[kTimelineTile];
 	__shared__ double sP0[kTimelineTile], sPNew[kTimelineTile], sInc[kTimelineTile];  // the frame's voicePitch, new.voicePitch after :71 (real requests), voicePitchInc
@@ -414,7 +455,7 @@ klatt_long_timeline_kernel(LongStream L) {
 		if (in) { L.pitchPop[j] = oPop[tid]; L.pitchOld[j] = oOld[tid]; L.pitchNew[j] = oNew[tid]; L.pitchInc[j] = oInc[tid]; }
 		__syncthreads();
 	}
-	if (tid == 0) L.start[L.nReq] = tBase;
+	if (tid == 0) L.start[L.nReq] = tBase < L.cap ? tBase : L.cap;
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -491,12 +532,15 @@ struct PhaseSrc {
 };
 
 // pass 1: the phase every chunk advances by (fraction of a cycle, 2^-64 fixed point: exact sums, used to LOCATE the anchors)
+template <bool MULTI>
 __global__ void __launch_bounds__(128)
-klatt_long_phase_kernel(LongStream L, uint32_t chunkTicks, uint32_t numChunks, uint64_t *__restrict__ advance) {
+klatt_long_phase_kernel(LongTable T, uint32_t chunkTicks, uint32_t numChunks, uint64_t *__restrict__ advance) {
 	const uint32_t ch = blockIdx.x * blockDim.x + threadIdx.x;
 	if (ch >= numChunks) return;
+	const uint32_t s = streamOfChunk<MULTI>(T, ch);
+	const LongStream &L = streamAt<MULTI>(T, s);
 	const uint64_t total = L.start[L.nReq];
-	const uint64_t t0 = (uint64_t)ch * chunkTicks;
+	const uint64_t t0 = (uint64_t)(ch - chunkBegin<MULTI>(T, s)) * chunkTicks;
 	const uint64_t t1 = (t0 + chunkTicks < total) ? t0 + chunkTicks : total;
 	PhaseSrc src(L, t0);
 	uint64_t pos = 0, fi;
@@ -509,7 +553,8 @@ klatt_long_phase_kernel(LongStream L, uint32_t chunkTicks, uint32_t numChunks, u
 }
 
 // exclusive scan of the per-chunk phase advances: 64-bit integer sums modulo one cycle, exact.  One block; every thread
-// sums a contiguous run, the run totals are scanned with warp shuffles, the runs are replayed from their prefix.
+// sums a contiguous run, the run totals are scanned with warp shuffles, the runs are replayed from their prefix.  The scan
+// runs over the chunks of all streams; a stream's own prefix is this one minus the value at its first chunk (exact mod 2^64).
 __global__ void __launch_bounds__(1024)
 klatt_long_phase_scan_kernel(const uint64_t *__restrict__ advance, uint32_t numChunks, uint64_t *__restrict__ startPhase) {
 	__shared__ uint64_t warpTotal[32];
@@ -545,69 +590,102 @@ klatt_long_phase_scan_kernel(const uint64_t *__restrict__ advance, uint32_t numC
 }
 
 // speculative pass: anchors, the two runs per chunk, the offset map of every chunk (klatt_long_phase.cuh)
+template <bool MULTI>
 __global__ void __launch_bounds__(128)
-klatt_long_spec_kernel(LongStream L, uint32_t chunkTicks, uint32_t numChunks, const uint64_t *__restrict__ startPhase,
+klatt_long_spec_kernel(LongTable T, uint32_t chunkTicks, uint32_t numChunks, const uint64_t *__restrict__ startPhase,
                        PhaseChunk *__restrict__ chunks, uint32_t *__restrict__ fail) {
 	const uint32_t ch = blockIdx.x * blockDim.x + threadIdx.x;
 	if (ch >= numChunks) return;
+	const uint32_t s = streamOfChunk<MULTI>(T, ch), cb = chunkBegin<MULTI>(T, s);
+	const LongStream &L = streamAt<MULTI>(T, s);
 	const uint64_t total = L.start[L.nReq];
-	PhaseSrc src(L, (uint64_t)ch * chunkTicks);
+	PhaseSrc src(L, (uint64_t)(ch - cb) * chunkTicks);
 	PhaseChunk pc;
-	// a run may extend over up to 15 anchorless chunks (zero pitch, silence); beyond that the call takes the fallback
-	if (!phaseSpeculateChunk(src, ch, chunkTicks, total, startPhase[ch], 16ull * chunkTicks, pc)) atomicOr(fail, 1u);
+	// a run may extend over up to 15 anchorless chunks (zero pitch, silence); beyond that the stream takes the fallback
+	if (!phaseSpeculateChunk(src, ch - cb, chunkTicks, total, startPhase[ch] - startPhase[cb], 16ull * chunkTicks, pc))
+		atomicOr(fail + s, 1u);
 	chunks[ch] = pc;
 }
 
-// exclusive scan of the offset maps in chunk order: startP[c] = the TRUE phase entering tick chunks[c].anchor
+// exclusive scan of the offset maps in chunk order, restarted at every stream's first chunk: startP[c] = the TRUE phase
+// entering tick chunks[c].anchor.  (A restart is not a map of the m -> m + a[m & 3] family, so the scan is SEGMENTED: an
+// element is (head, map), and a head discards whatever came before it.  Exact integer arithmetic either way.)
+struct SegPhaseMap {
+	PhaseMap m;
+	int head;  // the segment of this element starts inside it
+};
+__device__ __forceinline__ SegPhaseMap segCombine(const SegPhaseMap &first, const SegPhaseMap &second) {
+	if (second.head) return second;
+	SegPhaseMap r;
+	r.m = phaseMapCompose(second.m, first.m);
+	r.head = first.head;
+	return r;
+}
+
+template <bool MULTI>
 __global__ void __launch_bounds__(1024)
-klatt_long_phase_map_scan_kernel(const PhaseChunk *__restrict__ chunks, uint32_t numChunks, double *__restrict__ startP) {
-	__shared__ PhaseMap warpTotal[32];
+klatt_long_phase_map_scan_kernel(LongTable T, const PhaseChunk *__restrict__ chunks, uint32_t numChunks, double *__restrict__ startP) {
+	__shared__ SegPhaseMap warpTotal[32];
 	const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
 	const uint32_t per = (numChunks + 1023) / 1024;
 	const uint32_t c0 = (uint32_t)tid * per < numChunks ? (uint32_t)tid * per : numChunks;
 	const uint32_t c1 = c0 + per < numChunks ? c0 + per : numChunks;
-	PhaseMap run = phaseMapIdentity();
-	for (uint32_t c = c0; c < c1; ++c) run = phaseMapCompose(chunks[c].map, run);
-	auto shfl = [](const PhaseMap &m, int delta) {
-		PhaseMap r;
+	// the stream of chunk c0; the run then moves on stream by stream (c is a stream's first chunk iff c == chunkBase[s])
+	const uint32_t s0 = c0 < numChunks ? streamOfChunk<MULTI>(T, c0) : 0;
+	SegPhaseMap run{phaseMapIdentity(), 0};
+	for (uint32_t c = c0, s = s0; c < c1; ++c) {
+		while (chunkEnd<MULTI>(T, s, numChunks) <= c) ++s;
+		run = segCombine(run, SegPhaseMap{chunks[c].map, c == chunkBegin<MULTI>(T, s)});
+	}
+	auto shfl = [](const SegPhaseMap &m, int delta) {
+		SegPhaseMap r;
 #pragma unroll
-		for (int i = 0; i < kPhaseRuns; ++i) r.a[i] = __shfl_up_sync(0xffffffffu, m.a[i], delta);
+		for (int i = 0; i < kPhaseRuns; ++i) r.m.a[i] = __shfl_up_sync(0xffffffffu, m.m.a[i], delta);
+		r.head = __shfl_up_sync(0xffffffffu, m.head, delta);
 		return r;
 	};
-	PhaseMap inc = run;
+	SegPhaseMap inc = run;
 #pragma unroll
 	for (int delta = 1; delta < 32; delta <<= 1) {
-		PhaseMap up = shfl(inc, delta);
-		if (lane >= delta) inc = phaseMapCompose(inc, up);
+		SegPhaseMap up = shfl(inc, delta);
+		if (lane >= delta) inc = segCombine(up, inc);
 	}
 	if (lane == 31) warpTotal[warp] = inc;
 	__syncthreads();
 	if (warp == 0) {
-		PhaseMap w = warpTotal[lane];
+		SegPhaseMap w = warpTotal[lane];
 #pragma unroll
 		for (int delta = 1; delta < 32; delta <<= 1) {
-			PhaseMap up = shfl(w, delta);
-			if (lane >= delta) w = phaseMapCompose(w, up);
+			SegPhaseMap up = shfl(w, delta);
+			if (lane >= delta) w = segCombine(up, w);
 		}
 		warpTotal[lane] = w;
 	}
 	__syncthreads();
-	PhaseMap prev = shfl(inc, 1);
-	PhaseMap pre = lane == 0 ? phaseMapIdentity() : prev;
-	if (warp > 0) pre = phaseMapCompose(pre, warpTotal[warp - 1]);
-	// the stream starts at offset 0 of chunk 0's anchor (phase 0 exactly): the offset at chunk c's anchor is pre(0)
-	for (uint32_t c = c0; c < c1; ++c) {
+	SegPhaseMap prev = shfl(inc, 1);
+	SegPhaseMap pre = lane == 0 ? SegPhaseMap{phaseMapIdentity(), 0} : prev;
+	if (warp > 0) pre = segCombine(warpTotal[warp - 1], pre);
+	// every stream starts at offset 0 of its first chunk's anchor (phase 0 exactly): the offset at chunk c's anchor is pre(0)
+	PhaseMap p = pre.m;
+	for (uint32_t c = c0, s = s0; c < c1; ++c) {
+		while (chunkEnd<MULTI>(T, s, numChunks) <= c) ++s;
+		if (c == chunkBegin<MULTI>(T, s)) p = phaseMapIdentity();
 		const PhaseChunk pc = chunks[c];
-		startP[c] = pc.anchor == kNoAnchor ? 0.0 : phaseFromOffset(pc.s0, phaseMapApply(pre, 0));
-		pre = phaseMapCompose(pc.map, pre);
+		startP[c] = pc.anchor == kNoAnchor ? 0.0 : phaseFromOffset(pc.s0, phaseMapApply(p, 0));
+		p = phaseMapCompose(pc.map, p);
 	}
 }
 
-// serial fallback: ONE thread runs the plain recurrence over the whole stream and hands every chunk its true start (slow:
-// one tick after the other; taken only when the speculative pass could not anchor a chunk or failed its own check)
-__global__ void klatt_long_phase_serial_kernel(LongStream L, uint32_t chunkTicks, uint32_t numChunks, PhaseChunk *__restrict__ chunks,
-                                               double *__restrict__ startP) {
-	if (blockIdx.x != 0 || threadIdx.x != 0) return;
+// serial fallback: one thread per stream whose fail flag is set runs the plain recurrence over that whole stream and hands
+// every chunk of it its true start (slow: one tick after the other; taken only for a stream whose speculative pass could not
+// anchor a chunk or failed its own check).  The other streams' chunks are left as they are.
+template <bool MULTI>
+__global__ void klatt_long_phase_serial_kernel(LongTable T, uint32_t chunkTicks, uint32_t allChunks, const uint32_t *__restrict__ fail,
+                                               PhaseChunk *__restrict__ chunks, double *__restrict__ startP) {
+	const uint32_t s = blockIdx.x * blockDim.x + threadIdx.x;
+	if (s >= T.numStreams || !fail[s]) return;
+	const LongStream &L = streamAt<MULTI>(T, s);
+	const uint32_t cb = chunkBegin<MULTI>(T, s), numChunks = chunkEnd<MULTI>(T, s, allChunks) - cb;
 	const uint64_t total = L.start[L.nReq];
 	PhaseSrc src(L, 0);
 	double pos = 0.0, quot;
@@ -616,8 +694,8 @@ __global__ void klatt_long_phase_serial_kernel(LongStream L, uint32_t chunkTicks
 		const uint64_t t0 = (uint64_t)c * chunkTicks, t1 = (t0 + chunkTicks < total) ? t0 + chunkTicks : total;
 		PhaseChunk pc;
 		pc.anchor = t0; pc.next = t1; pc.s0 = pos; pc.map = phaseMapIdentity();
-		chunks[c] = pc;
-		startP[c] = pos;
+		chunks[cb + c] = pc;
+		startP[cb + c] = pos;
 		for (uint64_t t = t0; t < t1; ++t) {
 			src.tick(quot, fi);
 			pos = phaseStep(pos, quot);
@@ -628,14 +706,20 @@ __global__ void klatt_long_phase_serial_kernel(LongStream L, uint32_t chunkTicks
 // pass 2: the two excitation signals of every tick: cascade input ci (:204, :148) and parallel input pin (:206, :171).
 // Chunk ch owns the ticks [anchor, next) of its phase run and renders them from the true start phase; the run must end on
 // the next run's start, bit for bit, or `fail` is raised (the construction is verified, not trusted).
+template <bool MULTI>
 __global__ void __launch_bounds__(128)
-klatt_long_source_kernel(LongStream L, uint32_t chunkTicks, uint32_t numChunks, const PhaseChunk *__restrict__ chunks,
+klatt_long_source_kernel(LongTable T, uint32_t chunkTicks, uint32_t numChunks, const PhaseChunk *__restrict__ chunks,
                          const double *__restrict__ startP, uint32_t *__restrict__ fail, float *__restrict__ ci,
                          float *__restrict__ pin) {
 	const uint32_t ch = blockIdx.x * blockDim.x + threadIdx.x;
 	if (ch >= numChunks) return;
 	const PhaseChunk pc = chunks[ch];
 	if (pc.anchor == kNoAnchor) return;
+	const uint32_t s = streamOfChunk<MULTI>(T, ch), cb = chunkBegin<MULTI>(T, s);
+	const LongStream &L = streamAt<MULTI>(T, s);
+	// the stream's ticks in the signal arrays (the phase runs are in the stream's own ticks)
+	ci += (size_t)cb * chunkTicks;
+	pin += (size_t)cb * chunkTicks;
 	const uint64_t total = L.start[L.nReq];
 	const uint64_t t0 = pc.anchor, t1 = pc.next;
 	const double srD = (double)L.sampleRate, srInv = 1.0 / srD;
@@ -671,8 +755,8 @@ klatt_long_source_kernel(LongStream L, uint32_t chunkTicks, uint32_t numChunks, 
 		w.next(L, true);
 	}
 	if (t1 < total) {  // the chunk whose run starts at t1 must have been handed exactly the value this run arrives with
-		const uint32_t nx = (uint32_t)(t1 / chunkTicks);
-		if (nx >= numChunks || chunks[nx].anchor != t1 || startP[nx] != pos) atomicOr(fail, 1u);
+		const uint32_t nx = cb + (uint32_t)(t1 / chunkTicks);
+		if (nx >= chunkEnd<MULTI>(T, s, numChunks) || chunks[nx].anchor != t1 || startP[nx] != pos) atomicOr(fail + s, 1u);
 	}
 }
 
@@ -703,9 +787,9 @@ struct Affine {
 // its row ([32][33]: conflict-free either way).
 constexpr int kStageBlock = 64;   // threads: two warps, one tile each (+ one for the parallel-bank signal in the last stage)
 constexpr int kTile = 32;
-template <int STAGE, int PASS>
+template <int STAGE, int PASS, bool MULTI>
 __global__ void __launch_bounds__(kStageBlock)
-klatt_long_stage_kernel(LongStream L, uint32_t chunkTicks, uint32_t numChunks, int res, const float *__restrict__ in,
+klatt_long_stage_kernel(LongTable T, uint32_t chunkTicks, uint32_t numChunks, int res, const float *__restrict__ in,
                         const float *__restrict__ par, Affine *__restrict__ maps, const float2 *__restrict__ startState,
                         float *__restrict__ out, int16_t *__restrict__ pcm) {
 	constexpr int NR = StageTraits<STAGE>::NR;
@@ -715,13 +799,25 @@ klatt_long_stage_kernel(LongStream L, uint32_t chunkTicks, uint32_t numChunks, i
 	// (the output tile IS the input tile: a thread overwrites tick q of its own row after it has consumed it -- one tile per
 	// warp instead of two lets twice as many warps share an SM, and these kernels are bound by the latency of their recurrences)
 	float (*tOut)[kTile][kTile + 1] = tIn;
+	// per row of the warp's tiles (= per lane's chunk): ticks in the chunk, and where its tick 0 goes in the int16 output.  A
+	// warp may hold chunks of several streams; the signal arrays are addressed in virtual ticks (chunk c at c * chunkTicks).
+	__shared__ uint32_t sLen[kStageBlock / 32][kTile];
+	__shared__ uint64_t sPcm[kHasPar ? kStageBlock / 32 : 1][kTile];
 	const uint32_t lane = threadIdx.x & 31u, wib = threadIdx.x >> 5;
 	const uint32_t ch = blockIdx.x * blockDim.x + threadIdx.x;
 	const uint32_t warpChunk0 = ch - lane;  // first chunk of this warp
 	const bool live = ch < numChunks;
+	const uint32_t s = live ? streamOfChunk<MULTI>(T, ch) : 0, cb = chunkBegin<MULTI>(T, s);
+	const LongStream &L = streamAt<MULTI>(T, s);
 	const uint64_t total = L.start[L.nReq];
-	const uint64_t t0 = live ? (uint64_t)ch * chunkTicks : total;
-	const uint64_t t1 = (t0 + chunkTicks < total) ? t0 + chunkTicks : total;
+	const uint64_t t0 = live ? (uint64_t)(ch - cb) * chunkTicks : 0;  // in the stream's own ticks
+	const uint64_t t1 = live ? ((t0 + chunkTicks < total) ? t0 + chunkTicks : total) : 0;
+	const bool lastOfStream = live && ch + 1 == chunkEnd<MULTI>(T, s, numChunks);
+	if (MULTI) {
+		sLen[wib][lane] = (uint32_t)(t1 - t0);
+		if (kHasPar) sPcm[kHasPar ? wib : 0][lane] = L.outBase + t0;
+		__syncwarp();
+	}
 	Cursor cur;
 	PoleWalk pw[NR], pw0;  // pw0: the FIR anti-resonator of the nasal stage
 	DirWalk mix[NR], extra;  // parallel: pa1..6 + bypass; nasal: caNP; last: outputGain
@@ -754,8 +850,9 @@ klatt_long_stage_kernel(LongStream L, uint32_t chunkTicks, uint32_t numChunks, i
 			for (int k = 0; k < NR; ++k) { float2 s = startState[(size_t)ch * NR + k]; y[k] = s.x; d[k] = s.y; }
 		}
 		if (STAGE == kStageNasal) {
-			if (t0 >= 1) in1 = in[t0 - 1];
-			if (t0 >= 2) in2 = in[t0 - 2];
+			const size_t v0 = (size_t)cb * chunkTicks + t0;
+			if (t0 >= 1) in1 = in[v0 - 1];
+			if (t0 >= 2) in2 = in[v0 - 2];
 		}
 	}
 	for (uint32_t tile = 0; tile < chunkTicks; tile += kTile) {
@@ -763,7 +860,7 @@ klatt_long_stage_kernel(LongStream L, uint32_t chunkTicks, uint32_t numChunks, i
 #pragma unroll 4
 		for (int r = 0; r < kTile; ++r) {
 			const uint64_t g = (uint64_t)(warpChunk0 + r) * chunkTicks + tile + lane;
-			const bool ok = warpChunk0 + r < numChunks && g < total;
+			const bool ok = MULTI ? tile + lane < sLen[wib][r] : (warpChunk0 + r < numChunks && g < total);
 			tIn[wib][r][lane] = ok ? in[g] : 0.0f;
 			if (kHasPar) tPar[wib][r][lane] = ok ? par[g] : 0.0f;
 		}
@@ -881,9 +978,9 @@ klatt_long_stage_kernel(LongStream L, uint32_t chunkTicks, uint32_t numChunks, i
 #pragma unroll 4
 			for (int r = 0; r < kTile; ++r) {
 				const uint64_t g = (uint64_t)(warpChunk0 + r) * chunkTicks + tile + lane;
-				if (warpChunk0 + r < numChunks && g < total) {
+				if (MULTI ? tile + lane < sLen[wib][r] : (warpChunk0 + r < numChunks && g < total)) {
 					const float o = tOut[wib][r][lane];
-					if (STAGE == kStageLast) pcm[g] = (int16_t)(int)o;
+					if (STAGE == kStageLast) pcm[MULTI ? sPcm[kHasPar ? wib : 0][r] + tile + lane : g] = (int16_t)(int)o;
 					else out[g] = o;
 				}
 			}
@@ -891,10 +988,13 @@ klatt_long_stage_kernel(LongStream L, uint32_t chunkTicks, uint32_t numChunks, i
 		}
 	}
 	if (PASS == 1 && live) {
+		// The last chunk of a stream leaves the zero map (P = 0, z = 0): the scan's prefix at the next stream's first chunk is
+		// then exactly the zero state it starts from, with no change to the scan.  (Nothing reads a stream's last map otherwise.)
 #pragma unroll
 		for (int k = 0; k < NR; ++k) {
 			Affine m;
 			m.p00 = p00[k]; m.p01 = p01[k]; m.p10 = p10[k]; m.p11 = p11[k]; m.zy = y[k]; m.zd = d[k];
+			if (lastOfStream) m = Affine{0.0f, 0.0f, 0.0f, 0.0f, 0.0f, 0.0f};
 			maps[(size_t)ch * NR + k] = m;
 		}
 	}
@@ -1035,57 +1135,84 @@ cudaError_t launchKlattPlan(const int64_t *offsets, uint32_t numStreams, uint64_
                             const uint32_t *fadeDur, const uint8_t *isNull, int sampleRate, FadePlanF32 *plans,
                             cudaStream_t stream);
 
-cudaError_t launchKlattLongTimeline(const LongStream &L, cudaStream_t stream) {
-	klatt_long_timeline_kernel<<<1, kTimelineTile, 0, stream>>>(L);
+cudaError_t launchKlattLongTimeline(const LongTable &T, cudaStream_t stream) {
+	if (T.numStreams > 1) klatt_long_timeline_kernel<true><<<T.numStreams, kTimelineTile, 0, stream>>>(T);
+	else klatt_long_timeline_kernel<false><<<1, kTimelineTile, 0, stream>>>(T);
 	return cudaGetLastError();
 }
 
-// signals: five float arrays of totalTicks (+ padding): ci, pin, par, xa, xb.  maps / startState: numChunks * 6.
-// phase scratch: advance / startPhase [numChunks] u64, chunks [numChunks] PhaseChunk, startP [numChunks] double, fail u32.
-// serialPhase: skip the speculative passes and run the plain recurrence on one thread (the fallback).
-cudaError_t launchKlattLongRender(const LongStream &L, uint64_t totalTicks, uint32_t chunkTicks, uint64_t *advance,
-                                  uint64_t *startPhase, PhaseChunk *chunks, double *startP, uint32_t *fail, bool serialPhase,
-                                  float *ci, float *pin, float *par, float *xa, float *xb, Affine *maps,
-                                  float2 *startState, void *scanScratch, int16_t *pcm, unsigned long long *launchCounter, cudaStream_t stream) {
-	if (totalTicks == 0) return cudaSuccess;
-	const uint32_t numChunks = (uint32_t)((totalTicks + chunkTicks - 1) / chunkTicks);
+// The glottal phase of every chunk: the speculative passes (fail[s] is raised for a stream whose chunks could not be
+// anchored), or, with `serial`, the plain recurrence on one thread for each stream whose fail[s] is set.
+// phase scratch: advance / startPhase [numChunks] u64, chunks [numChunks] PhaseChunk, startP [numChunks] double, fail [numStreams].
+template <bool MULTI>
+static cudaError_t longPhase(const LongTable &T, uint32_t numChunks, uint32_t chunkTicks, uint64_t *advance, uint64_t *startPhase,
+                                 PhaseChunk *chunks, double *startP, uint32_t *fail, bool serial, unsigned long long *launchCounter,
+                                 cudaStream_t stream) {
+	if (numChunks == 0) return cudaSuccess;
 	const dim3 grid((numChunks + 127) / 128), block(128);
-	const dim3 sgrid((numChunks + kStageBlock - 1) / kStageBlock), sblock(kStageBlock);
-	cudaError_t e = cudaMemsetAsync(fail, 0, sizeof(uint32_t), stream);
-	if (e != cudaSuccess) return e;
-	if (serialPhase) {
-		klatt_long_phase_serial_kernel<<<1, 1, 0, stream>>>(L, chunkTicks, numChunks, chunks, startP);
+	if (serial) {
+		klatt_long_phase_serial_kernel<MULTI><<<(T.numStreams + 31) / 32, 32, 0, stream>>>(T, chunkTicks, numChunks, fail, chunks, startP);
 		if (launchCounter) *launchCounter += 1;
 	} else {
-		klatt_long_phase_kernel<<<grid, block, 0, stream>>>(L, chunkTicks, numChunks, advance);
+		klatt_long_phase_kernel<MULTI><<<grid, block, 0, stream>>>(T, chunkTicks, numChunks, advance);
 		klatt_long_phase_scan_kernel<<<1, 1024, 0, stream>>>(advance, numChunks, startPhase);
-		klatt_long_spec_kernel<<<grid, block, 0, stream>>>(L, chunkTicks, numChunks, startPhase, chunks, fail);
-		klatt_long_phase_map_scan_kernel<<<1, 1024, 0, stream>>>(chunks, numChunks, startP);
+		klatt_long_spec_kernel<MULTI><<<grid, block, 0, stream>>>(T, chunkTicks, numChunks, startPhase, chunks, fail);
+		klatt_long_phase_map_scan_kernel<MULTI><<<1, 1024, 0, stream>>>(T, chunks, numChunks, startP);
 		if (launchCounter) *launchCounter += 4;
 	}
-	klatt_long_source_kernel<<<grid, block, 0, stream>>>(L, chunkTicks, numChunks, chunks, startP, fail, ci, pin);
+	return cudaGetLastError();
+}
+
+// The source pass (which checks the phase runs and raises fail[s] on a miss) and the resonator stages, into the int16 output.
+// signals: five float arrays of numChunks * chunkTicks virtual ticks (+ padding): ci, pin, par, xa, xb.  maps / startState:
+// numChunks * 6.  pcm: the packed output, stream s from streams[s].outBase.
+template <bool MULTI>
+static cudaError_t longSynth(const LongTable &T, uint32_t numChunks, uint32_t chunkTicks, const PhaseChunk *chunks,
+                                 const double *startP, uint32_t *fail, float *ci, float *pin, float *par, float *xa, float *xb,
+                                 Affine *maps, float2 *startState, void *scanScratch, int16_t *pcm, unsigned long long *launchCounter,
+                                 cudaStream_t stream) {
+	if (numChunks == 0) return cudaSuccess;
+	const dim3 grid((numChunks + 127) / 128), block(128);
+	const dim3 sgrid((numChunks + kStageBlock - 1) / kStageBlock), sblock(kStageBlock);
+	klatt_long_source_kernel<MULTI><<<grid, block, 0, stream>>>(T, chunkTicks, numChunks, chunks, startP, fail, ci, pin);
 	// parallel bank
-	klatt_long_stage_kernel<kStageParallel, 1><<<sgrid, sblock, 0, stream>>>(L, chunkTicks, numChunks, 0, pin, nullptr, maps, nullptr, nullptr, nullptr);
+	klatt_long_stage_kernel<kStageParallel, 1, MULTI><<<sgrid, sblock, 0, stream>>>(T, chunkTicks, numChunks, 0, pin, nullptr, maps, nullptr, nullptr, nullptr);
 	launchLongScan(maps, numChunks, 6, scanScratch, startState, stream);
-	klatt_long_stage_kernel<kStageParallel, 2><<<sgrid, sblock, 0, stream>>>(L, chunkTicks, numChunks, 0, pin, nullptr, nullptr, startState, par, nullptr);
+	klatt_long_stage_kernel<kStageParallel, 2, MULTI><<<sgrid, sblock, 0, stream>>>(T, chunkTicks, numChunks, 0, pin, nullptr, nullptr, startState, par, nullptr);
 	// rN0 + rNP
-	klatt_long_stage_kernel<kStageNasal, 1><<<sgrid, sblock, 0, stream>>>(L, chunkTicks, numChunks, kResNP, ci, nullptr, maps, nullptr, nullptr, nullptr);
+	klatt_long_stage_kernel<kStageNasal, 1, MULTI><<<sgrid, sblock, 0, stream>>>(T, chunkTicks, numChunks, kResNP, ci, nullptr, maps, nullptr, nullptr, nullptr);
 	launchLongScan(maps, numChunks, 1, scanScratch, startState, stream);
-	klatt_long_stage_kernel<kStageNasal, 2><<<sgrid, sblock, 0, stream>>>(L, chunkTicks, numChunks, kResNP, ci, nullptr, nullptr, startState, xa, nullptr);
+	klatt_long_stage_kernel<kStageNasal, 2, MULTI><<<sgrid, sblock, 0, stream>>>(T, chunkTicks, numChunks, kResNP, ci, nullptr, nullptr, startState, xa, nullptr);
 	// r6 .. r2
 	float *src = xa, *dst = xb;
 	for (int r = kResCascade; r < kResParallel - 1; ++r) {
-		klatt_long_stage_kernel<kStageCascade, 1><<<sgrid, sblock, 0, stream>>>(L, chunkTicks, numChunks, r, src, nullptr, maps, nullptr, nullptr, nullptr);
+		klatt_long_stage_kernel<kStageCascade, 1, MULTI><<<sgrid, sblock, 0, stream>>>(T, chunkTicks, numChunks, r, src, nullptr, maps, nullptr, nullptr, nullptr);
 		launchLongScan(maps, numChunks, 1, scanScratch, startState, stream);
-		klatt_long_stage_kernel<kStageCascade, 2><<<sgrid, sblock, 0, stream>>>(L, chunkTicks, numChunks, r, src, nullptr, nullptr, startState, dst, nullptr);
+		klatt_long_stage_kernel<kStageCascade, 2, MULTI><<<sgrid, sblock, 0, stream>>>(T, chunkTicks, numChunks, r, src, nullptr, nullptr, startState, dst, nullptr);
 		float *tmp = src; src = dst; dst = tmp;
 	}
 	// r1 + output
-	klatt_long_stage_kernel<kStageLast, 1><<<sgrid, sblock, 0, stream>>>(L, chunkTicks, numChunks, kResParallel - 1, src, par, maps, nullptr, nullptr, nullptr);
+	klatt_long_stage_kernel<kStageLast, 1, MULTI><<<sgrid, sblock, 0, stream>>>(T, chunkTicks, numChunks, kResParallel - 1, src, par, maps, nullptr, nullptr, nullptr);
 	launchLongScan(maps, numChunks, 1, scanScratch, startState, stream);
-	klatt_long_stage_kernel<kStageLast, 2><<<sgrid, sblock, 0, stream>>>(L, chunkTicks, numChunks, kResParallel - 1, src, par, nullptr, startState, nullptr, pcm);
+	klatt_long_stage_kernel<kStageLast, 2, MULTI><<<sgrid, sblock, 0, stream>>>(T, chunkTicks, numChunks, kResParallel - 1, src, par, nullptr, startState, nullptr, pcm);
 	if (launchCounter) *launchCounter += 1 + 5 * 8;
 	return cudaGetLastError();
+}
+
+cudaError_t launchKlattLongPhase(const LongTable &T, uint32_t numChunks, uint32_t chunkTicks, uint64_t *advance, uint64_t *startPhase,
+                                 PhaseChunk *chunks, double *startP, uint32_t *fail, bool serial, unsigned long long *launchCounter,
+                                 cudaStream_t stream) {
+	return T.numStreams > 1 ? longPhase<true>(T, numChunks, chunkTicks, advance, startPhase, chunks, startP, fail, serial, launchCounter, stream)
+	                        : longPhase<false>(T, numChunks, chunkTicks, advance, startPhase, chunks, startP, fail, serial, launchCounter, stream);
+}
+
+cudaError_t launchKlattLongSynth(const LongTable &T, uint32_t numChunks, uint32_t chunkTicks, const PhaseChunk *chunks,
+                                 const double *startP, uint32_t *fail, float *ci, float *pin, float *par, float *xa, float *xb,
+                                 Affine *maps, float2 *startState, void *scanScratch, int16_t *pcm, unsigned long long *launchCounter,
+                                 cudaStream_t stream) {
+	return T.numStreams > 1
+	           ? longSynth<true>(T, numChunks, chunkTicks, chunks, startP, fail, ci, pin, par, xa, xb, maps, startState, scanScratch, pcm, launchCounter, stream)
+	           : longSynth<false>(T, numChunks, chunkTicks, chunks, startP, fail, ci, pin, par, xa, xb, maps, startState, scanScratch, pcm, launchCounter, stream);
 }
 
 }  // namespace klatt

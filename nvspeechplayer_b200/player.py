@@ -111,6 +111,8 @@ def load_library():
     L.speechPlayer_multiBatchGetLastIndices.argtypes = [vp, vp]
     L.speechPlayer_synthesizeLong.restype = ctypes.c_longlong
     L.speechPlayer_synthesizeLong.argtypes = [i32, vp, vp, vp, vp, u32, u64, u64, u32, vp, ctypes.c_ulonglong, i32, vp, vp]
+    L.speechPlayer_synthesizeLongBatch.restype = ctypes.c_longlong
+    L.speechPlayer_synthesizeLongBatch.argtypes = [i32, u32, vp, vp, vp, vp, vp, u64, vp, u32, vp, vp, vp, i32, vp, vp, vp]
     _lib = L
     return L
 
@@ -260,6 +262,58 @@ def synthesize_long(sample_rate, frames, min_dur, fade_dur, is_null=None, seed=0
                                         chunk_ticks, _ptr(out), max_samples, 0, ctypes.byref(ms), ctypes.byref(launches))
     _check(got, "speechPlayer_synthesizeLong")
     return out[:got], ms.value, launches.value
+
+
+def synthesize_long_batch(fb, seed=0xB200, chunk_ticks=0, max_samples=None, device_out=None):
+    """speechPlayer_synthesizeLongBatch: every stream of ``fb`` (a workloads.FrameBatch of whole, pre-queued queues) rendered
+    with parallelism in time, all streams' chunks in one launch sequence.  Row s is what ``synthesize_long`` renders for
+    stream s with noise stream ``fb.stream_ids[s]``.  ``max_samples``: None, one cap for all streams, or one per stream.
+    Returns (packed int16 samples, out_offsets int64 [N+1], serial_phase uint8 [N], render_ms, kernel_launches); stream s is
+    ``samples[out_offsets[s]:out_offsets[s+1]]`` (``split_rows``).  With ``device_out`` (a raw device address of at least
+    ``long_batch_size(...)`` int16) the samples stay in HBM and the first element is the total sample count."""
+    L = load_library()
+    n = fb.num_streams
+    offsets = np.ascontiguousarray(fb.offsets, dtype=np.int64)
+    frames = np.ascontiguousarray(fb.frames, dtype=np.float64).reshape(-1, NUM_PARAMS)
+    m = np.ascontiguousarray(fb.min_dur, dtype=np.uint32)
+    f = np.ascontiguousarray(fb.fade_dur, dtype=np.uint32)
+    nul = np.ascontiguousarray(fb.is_null, dtype=np.uint8)
+    ids = np.ascontiguousarray(fb.stream_ids, dtype=np.uint64)
+    caps = None if max_samples is None else np.ascontiguousarray(np.broadcast_to(np.asarray(max_samples, dtype=np.uint64), (n,)))
+    out_offsets = np.zeros(n + 1, dtype=np.int64)
+    serial = np.zeros(n, dtype=np.uint8)
+    ms, launches = ctypes.c_double(0), ctypes.c_ulonglong(0)
+
+    def call(out_ptr, on_device):
+        return L.speechPlayer_synthesizeLongBatch(fb.sample_rate, n, _ptr(offsets), _ptr(frames), _ptr(m), _ptr(f), _ptr(nul), seed,
+                                                  _ptr(ids), chunk_ticks, _ptr(caps), out_ptr, _ptr(out_offsets), on_device,
+                                                  _ptr(serial), ctypes.byref(ms), ctypes.byref(launches))
+    if device_out is not None:
+        got = _check(call(device_out, 1), "speechPlayer_synthesizeLongBatch")
+        return got, out_offsets, serial, ms.value, launches.value
+    total = _check(call(None, 0), "speechPlayer_synthesizeLongBatch")
+    out = np.zeros(max(total, 1), dtype=np.int16)
+    got = _check(call(_ptr(out), 0), "speechPlayer_synthesizeLongBatch")
+    return out[:got], out_offsets, serial, ms.value, launches.value
+
+
+def long_batch_size(fb, max_samples=None):
+    """(total samples, out_offsets) of synthesize_long_batch for ``fb``: a size query, no device needed."""
+    L = load_library()
+    n = fb.num_streams
+    offsets = np.ascontiguousarray(fb.offsets, dtype=np.int64)
+    m = np.ascontiguousarray(fb.min_dur, dtype=np.uint32)
+    f = np.ascontiguousarray(fb.fade_dur, dtype=np.uint32)
+    caps = None if max_samples is None else np.ascontiguousarray(np.broadcast_to(np.asarray(max_samples, dtype=np.uint64), (n,)))
+    out_offsets = np.zeros(n + 1, dtype=np.int64)
+    got = L.speechPlayer_synthesizeLongBatch(fb.sample_rate, n, _ptr(offsets), None, _ptr(m), _ptr(f), None, 0, None, 0, _ptr(caps),
+                                             None, _ptr(out_offsets), 0, None, None, None)
+    return _check(got, "speechPlayer_synthesizeLongBatch"), out_offsets
+
+
+def split_rows(samples, out_offsets):
+    """The packed output of synthesize_long_batch as one array (a view) per stream."""
+    return [samples[int(out_offsets[s]):int(out_offsets[s + 1])] for s in range(len(out_offsets) - 1)]
 
 
 class Batch(object):
