@@ -1,4 +1,4 @@
-// Host-side helper threads (plain C++, no CUDA): see HostPool below.  Used by engine.cu for the batched pull; tests/hostsim
+// Host-side helper threads (plain C++, no CUDA): see HostPool below.  Used by api_player.cu for the batched pull; tests/hostsim
 // builds it on the CPU (tests/test_host_pool_cpu.py).
 #pragma once
 #include <algorithm>

@@ -22,6 +22,7 @@
 #include "klatt_f32_core.cuh"
 #include "out_writer.cuh"
 #include "klatt_f32_pair.cuh"
+#include "launch.h"
 
 namespace klatt {
 

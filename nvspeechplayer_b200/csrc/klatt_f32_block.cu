@@ -31,6 +31,7 @@
 #include "klatt_f32_core.cuh"
 #include "out_writer.cuh"
 #include "klatt_f32_pair.cuh"
+#include "launch.h"
 
 namespace klatt {
 
@@ -124,7 +125,7 @@ klatt_block_import_kernel(const StreamDesc *__restrict__ descs, uint32_t numStre
 		for (int i = 0; i < kNumDirect; ++i) L.f32.dir[i] = gs.dir[i];
 		for (int i = 0; i < 2 * kNumResonators; ++i) L.f32.zc[i] = gs.zc[i];
 		L.f32.depth = gs.depth;
-	} else {  // init_states_kernel's fresh player (engine.cu)
+	} else {  // init_states_kernel's fresh player (host.cu)
 		L.fm.lastUserIndex = -1; L.fm.curIsNull = 1; L.fm.oldIsNull = 1;
 	}
 	lite[s] = L;

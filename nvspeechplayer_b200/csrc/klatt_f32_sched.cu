@@ -14,6 +14,7 @@
 #include "klatt_f32_core.cuh"
 #include "out_writer.cuh"
 #include "klatt_f32_pair.cuh"
+#include "launch.h"
 
 // KLATT_SCHED_LITE (default 1, round 2): the streams of a call live in a dense array of 560-byte StreamStateLite records
 // (klatt_common.h; 35 MB for 65 536 streams: L2-resident) instead of the 2.4 KB AoS blocks; a worker copies the 32 records of
@@ -30,12 +31,6 @@
 #endif
 
 namespace klatt {
-
-cudaError_t launchKlattLiteImport(const StreamDesc *descs, uint32_t numStreams, uint32_t numDummies, void *lite, cudaStream_t stream);
-cudaError_t launchKlattLiteExport(const StreamDesc *descs, uint32_t numStreams, const void *lite, uint32_t *samplesWritten, StreamResult *results,
-                                  cudaStream_t stream);
-cudaError_t launchKlattFinalize(const StreamDesc *descs, uint32_t numStreams, uint32_t *samplesWritten, StreamResult *results,
-                                cudaStream_t stream);
 
 #ifdef KLATT_SCHED_PROFILE
 #define PROF_LAP(acc) { long long t1 = clock64(); acc += t1 - t0; t0 = t1; }

@@ -22,6 +22,7 @@
 #include "klatt_common.h"
 #include "philox.cuh"
 #include "out_writer.cuh"
+#include "launch.h"
 
 namespace klatt {
 

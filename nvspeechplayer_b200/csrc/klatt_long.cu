@@ -36,38 +36,9 @@
 #include "klatt_common.h"
 #include "klatt_f32_core.cuh"
 #include "klatt_long_phase.cuh"
+#include "launch.h"
 
 namespace klatt {
-
-// One stream of a launch: pointers into the flat arrays of all the launch's requests at this stream's offset.  (Mirrored
-// field for field in engine.cu, which builds the table on the host.)
-struct LongStream {
-	const double *frames;      // [nReq][47]
-	const uint32_t *minDur, *fadeDur;
-	const uint8_t *isNull;     // may be null
-	const FadePlanF32 *plans;  // [nReq]
-	uint32_t nReq;
-	int sampleRate;
-	uint64_t seed, streamId;
-	uint64_t cap;              // ticks rendered: the timeline is cut here (start[nReq] = min(ticks the queue yields, cap))
-	uint64_t outBase;          // where the stream's tick 0 goes in the launch's packed int16 output
-	// made by klatt_long_timeline_kernel
-	uint64_t *start;        // [nReq+1] tick of each request's pop tick; start[nReq] = ticks rendered
-	int32_t *prevReal;      // [nReq] last non-NULL request before j, or -1
-	double *pitchPop;       // [nReq] cur.voicePitch on the pop tick (stale value)
-	double *pitchOld, *pitchNew, *pitchInc;  // [nReq] fade end points and hold glide
-	uint64_t *vibPosStart;  // [nReq] vibrato phase before the pop tick
-};
-
-// The streams of one launch.  Stream s owns the chunks [chunkBase[s], chunkBase[s+1]) (chunkBase: exclusive scan of
-// ceil(ticks_s / L)); its tick t lives at VIRTUAL tick chunkBase[s] * L + t of the signal arrays, so every chunk starts on
-// a multiple of L as it does for one stream, and the gap between two streams is under L ticks.
-struct LongTable {
-	const LongStream *streams;   // [numStreams]
-	const uint32_t *chunkBase;   // [numStreams + 1]
-	uint32_t numStreams;
-	LongStream one;              // streams[0] by value: a one-stream launch reads its stream from the parameter bank
-};
 
 namespace {
 
@@ -769,11 +740,6 @@ template <int STAGE> struct StageTraits {
 	static constexpr int NR = STAGE == kStageParallel ? 6 : 1;  // scanned sections
 };
 
-// affine map of one section over one chunk, (y, d)_end = P (y, d)_start + z, row-major P
-struct Affine {
-	float p00, p01, p10, p11, zy, zd;
-};
-
 // One chunk of one stage.  PASS 1: from zero state, also accumulate P.  PASS 2: from the scanned start state, write
 // the stage's output signal (or, for the last stage, the int16 samples).
 //   kStageParallel: in = pin, sections 8..13, out = par (:170-180)
@@ -1129,12 +1095,8 @@ static void launchLongScan(const Affine *maps, uint32_t numChunks, int numSectio
 size_t klattLongScanScratchBytes(uint64_t numChunks) { return sizeof(AffineD) * 6 * (size_t)((numChunks + kScanBlock - 1) / kScanBlock); }
 
 // ---------------------------------------------------------------------------------------------------------------
-// launcher: everything device-resident; scratch sized by the caller (see engine.cu)
+// launchers (launch.h)
 // ---------------------------------------------------------------------------------------------------------------
-cudaError_t launchKlattPlan(const int64_t *offsets, uint32_t numStreams, uint64_t totalRequests, const double *frames,
-                            const uint32_t *fadeDur, const uint8_t *isNull, int sampleRate, FadePlanF32 *plans,
-                            cudaStream_t stream);
-
 cudaError_t launchKlattLongTimeline(const LongTable &T, cudaStream_t stream) {
 	if (T.numStreams > 1) klatt_long_timeline_kernel<true><<<T.numStreams, kTimelineTile, 0, stream>>>(T);
 	else klatt_long_timeline_kernel<false><<<1, kTimelineTile, 0, stream>>>(T);

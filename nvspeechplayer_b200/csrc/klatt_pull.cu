@@ -9,6 +9,7 @@
 #include <cuda_runtime.h>
 #include "klatt_common.h"
 #include "klatt_pull_core.cuh"
+#include "launch.h"
 
 namespace klatt {
 

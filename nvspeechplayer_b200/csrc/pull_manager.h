@@ -11,7 +11,7 @@
 //   drain  src/frame.cpp:73-75   nothing queued when the hold runs out: no sample, the caller gets a short count
 //   purge  src/frame.cpp:103-112 queue dropped, a fade in progress frozen into the old request, next tick pops
 //
-// Header-only and host-only; included by engine.cu and by the host build of the kernel arithmetic under tests/hostsim.
+// Header-only and host-only; included by api_player.cu and by the host build of the kernel arithmetic under tests/hostsim.
 #pragma once
 #include <stdint.h>
 #include <string.h>

@@ -20,7 +20,7 @@ def weak_shard(streams_per_rank, rank):
 
 def balanced_ranges(ticks_per_stream, shards):
     """first[shards + 1] of contiguous stream ranges whose tick sums are balanced -- the rule speechPlayer_multiBatchSetFramesHost
-    applies (engine.cu): with upto = running sum of (ticks + 1), shard d starts at the first stream where upto reaches d / shards
+    applies (api_batch.cu): with upto = running sum of (ticks + 1), shard d starts at the first stream where upto reaches d / shards
     of the total.  tests/test_gpu_multibatch.py holds the library to this function."""
     import numpy as np
     t = np.asarray(ticks_per_stream, dtype=np.uint64) + np.uint64(1)

@@ -4,7 +4,7 @@
 //
 //   shapes:  contig : one cudaMemcpyAsync of B bytes (device -> pinned host)
 //            2d     : cudaMemcpy2DAsync of the engine's gather shape: `rows` rows of `width` bytes out of a device
-//                     staging buffer (pitch = width) into a host buffer of pitch `hostPitch` (engine.cu renderToHost:
+//                     staging buffer (pitch = width) into a host buffer of pitch `hostPitch` (host.cu renderToHost:
 //                     65 536 rows, 2 s slices of a 10 s row -> width 88 200 B, host pitch 441 000 B)
 //            2dtight: the same rows into a host buffer of pitch == width (what a [chunk][stream]-blocked host layout
 //                     would see)
