@@ -12,7 +12,8 @@
  *
  * The reference spends ~1 us per frame in ctypes calls alone and renders ~5e3 audio-seconds per second per core through
  * this pipeline (SURVEY.md 8f); the arrays this producer fills are the ones speechPlayer_batchSetFramesHost takes.
- * Host code only: no CUDA device is needed for these calls.
+ * The table calls and speechPlayer_ipaFrames are host code only: no CUDA device is needed for them.
+ * speechPlayer_ipaFramesDevice runs the same rules on the GPU and fills the arrays speechPlayer_batchSetFramesDevice takes.
  */
 #ifndef NVSP_B200_SPEECHPLAYER_IPA_H
 #define NVSP_B200_SPEECHPLAYER_IPA_H
@@ -62,6 +63,29 @@ long long speechPlayer_ipaFrames(const speechPlayer_ipaTable_t *table, const cha
                                  speechPlayer_frame_t *frames, unsigned int *minDur, unsigned int *fadeDur,
                                  unsigned char *isNull, double *durationMs, double *fadeMs,
                                  unsigned long long capacity, unsigned int numThreads);
+
+/* The same producer on the calling thread's current CUDA device, bit for bit speechPlayer_ipaFrames.  Only the UTF-8
+ * bytes and the per-text parameters cross PCIe; the frames are written in device memory.
+ *
+ * Inputs are HOST memory and the caller's to reuse once the call returns:
+ *   text + textOffsets [numTexts+1]  packed UTF-8: text i is the bytes [textOffsets[i], textOffsets[i+1]) of text, ending
+ *                                    early at its first NUL byte (offsets must not decrease)
+ *   speed / basePitch / inflection / clauseType, sampleRate, trailingSilenceMs: as speechPlayer_ipaFrames
+ * Outputs are DEVICE memory on the current device; any may be NULL:
+ *   dOffsets [numTexts+1] int64                                        -- always written when non-NULL
+ *   dFrames [capacity][47] double, dMinDur / dFadeDur [capacity] uint32, dIsNull [capacity] uint8,
+ *   dDurationMs / dFadeMs [capacity] double, dTimelineSamples [numTexts] uint64 (samples each text yields, the sum of
+ *   max(M + 1, max(F, 1) + 2) that speechPlayer_timelineSamples computes)  -- written only when capacity >= the total
+ * The call synchronises once (to learn the total) and returns with the rows still being written on cudaStream, so a
+ * speechPlayer_batchSetFramesDevice on the same stream may follow without a synchronisation.  Returns the total number
+ * of frames, or -1 (speechPlayer_lastError()): bad arguments, no device (there is no CPU fallback), or a pitch percent
+ * without a precomputed factor. */
+long long speechPlayer_ipaFramesDevice(const speechPlayer_ipaTable_t *table, const char *text, const int64_t *textOffsets,
+                                       unsigned int numTexts, const double *speed, const double *basePitch,
+                                       const double *inflection, const char *clauseType, int sampleRate,
+                                       double trailingSilenceMs, void *dOffsets, void *dFrames, void *dMinDur,
+                                       void *dFadeDur, void *dIsNull, void *dDurationMs, void *dFadeMs,
+                                       void *dTimelineSamples, unsigned long long capacity, void *cudaStream);
 
 #ifdef __cplusplus
 }

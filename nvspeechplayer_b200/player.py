@@ -340,8 +340,19 @@ class Batch(object):
                                                        _ptr(fb.user_index), _ptr(fb.is_null), cuda_stream),
                "speechPlayer_batchSetFramesHost")
 
-    def set_frames_device(self, d_offsets, d_frames, d_min, d_fade, d_user_index=None, d_is_null=None, cuda_stream=None):
-        """Arguments are raw device addresses (ints), e.g. tensor.data_ptr()."""
+    def set_frames_device(self, d_offsets, d_frames=None, d_min=None, d_fade=None, d_user_index=None, d_is_null=None, cuda_stream=None):
+        """Arguments are raw device addresses (ints), e.g. tensor.data_ptr(); or d_offsets is an ipa.DeviceFrameBatch, whose
+        tensors the batch then keeps alive for as long as it uses them."""
+        if hasattr(d_offsets, "min_dur") and hasattr(d_offsets, "timeline_samples"):
+            db = d_offsets
+            assert db.num_streams == self.num_streams
+            if cuda_stream is not None and hasattr(cuda_stream, "cuda_stream"):
+                cuda_stream = cuda_stream.cuda_stream
+            _check(self._L.speechPlayer_batchSetFramesDevice(self._h, db.offsets.data_ptr(), db.frames.data_ptr(), db.min_dur.data_ptr(),
+                                                             db.fade_dur.data_ptr(), None, db.is_null.data_ptr(), cuda_stream),
+                   "speechPlayer_batchSetFramesDevice")
+            self._keep = db
+            return
         _check(self._L.speechPlayer_batchSetFramesDevice(self._h, d_offsets, d_frames, d_min, d_fade, d_user_index, d_is_null,
                                                          cuda_stream), "speechPlayer_batchSetFramesDevice")
 
