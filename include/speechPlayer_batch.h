@@ -164,6 +164,27 @@ long long speechPlayer_synthesizeLongBatch(int sampleRate, unsigned int numStrea
                                            int outOnDevice, unsigned char *serialPhase, double *renderMs,
                                            unsigned long long *kernelLaunches);
 
+/* The same call for queues that are already in device memory, e.g. written by speechPlayer_ipaFramesDevice or by a model on
+ * the GPU: stream s renders exactly what speechPlayer_synthesizeLongBatch renders for the same queues, bit for bit, and
+ * outOffsets and serialPhase are the same.  Nothing of the queues is uploaded; they are read in place.
+ *   dOffsets, dFrames, dMinDur, dFadeDur, dIsNull : DEVICE pointers of the current device, in the layout of
+ *                  speechPlayer_batchSetFramesDevice (int64 [N+1], double [total][47], u32, u32, u8 or NULL).  dFrames,
+ *                  dMinDur and dFadeDur are required when the queues hold any request.  The arrays are only read, and must
+ *                  stay valid and unchanged until the call returns.
+ *   the others   : as for speechPlayer_synthesizeLongBatch (host arrays; out is HOST, or DEVICE when outOnDevice)
+ *   cudaStream   : every copy, event and launch of the call goes on it, so the call is ordered after work already queued
+ *                  there (the producer of the queues) without synchronisation by the caller; NULL = the default stream
+ * The offsets are copied back and checked by the host entry's rules before any kernel reads the queues, then one kernel
+ * counts each stream's ticks (the occupancy law) and they are copied back: out = NULL is still a size query, but it needs
+ * the device.  kernelLaunches counts that kernel too.  The call synchronises cudaStream before it returns.
+ * Returns the total samples written (= outOffsets[numStreams]) or -1 (speechPlayer_lastError()). */
+long long speechPlayer_synthesizeLongBatchDevice(int sampleRate, unsigned int numStreams, const void *dOffsets, const void *dFrames,
+                                                 const void *dMinDur, const void *dFadeDur, const void *dIsNull, uint64_t seed,
+                                                 const uint64_t *streamIds, unsigned int chunkTicks,
+                                                 const unsigned long long *maxSamples, sample *out, int64_t *outOffsets,
+                                                 int outOnDevice, unsigned char *serialPhase, double *renderMs,
+                                                 unsigned long long *kernelLaunches, void *cudaStream);
+
 /* Pure host helper (no device needed): samples a fully pre-queued stream yields,
  * sum_j max(M_j+1, max(F_j,1)+2)  -- the occupancy law of the reference frame manager (src/frame.cpp:41-80). */
 unsigned long long speechPlayer_timelineSamples(const unsigned int *minFrameDuration,

@@ -1095,8 +1095,49 @@ static void launchLongScan(const Affine *maps, uint32_t numChunks, int numSectio
 size_t klattLongScanScratchBytes(uint64_t numChunks) { return sizeof(AffineD) * 6 * (size_t)((numChunks + kScanBlock - 1) / kScanBlock); }
 
 // ---------------------------------------------------------------------------------------------------------------
+// ticks of device-resident queues (speechPlayer_synthesizeLongBatchDevice): the occupancy law of timelineTicks (host.h),
+// sum over a stream's requests of max(M + 1, max(F, 1) + 2), one block per stream.  Integer sums: exact in any order.
+// ---------------------------------------------------------------------------------------------------------------
+constexpr int kTicksBlock = 256;
+constexpr uint32_t kTicksMaxBlocks = 1u << 20;  // more streams than this: each block takes every kTicksMaxBlocks-th stream
+
+__global__ void __launch_bounds__(kTicksBlock)
+klatt_long_ticks_kernel(const int64_t *__restrict__ offsets, uint32_t numStreams, const uint32_t *__restrict__ minDur,
+                        const uint32_t *__restrict__ fadeDur, uint64_t *__restrict__ ticks) {
+	__shared__ unsigned long long warpSum[kTicksBlock / 32];
+	const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+	for (uint32_t s = blockIdx.x; s < numStreams; s += gridDim.x) {
+		const int64_t end = offsets[s + 1];
+		unsigned long long t = 0;
+		for (int64_t j = offsets[s] + threadIdx.x; j < end; j += kTicksBlock) {
+			const unsigned long long m = minDur[j], f = fadeDur[j] > 1u ? fadeDur[j] : 1u;
+			t += m + 1 > f + 2 ? m + 1 : f + 2;
+		}
+#pragma unroll
+		for (int d = 16; d > 0; d >>= 1) t += __shfl_down_sync(0xffffffffu, t, d);
+		if (lane == 0) warpSum[warp] = t;
+		__syncthreads();
+		if (warp == 0) {
+			t = lane < kTicksBlock / 32 ? warpSum[lane] : 0;
+#pragma unroll
+			for (int d = 16; d > 0; d >>= 1) t += __shfl_down_sync(0xffffffffu, t, d);
+			if (lane == 0) ticks[s] = t;
+		}
+		__syncthreads();  // warpSum is rewritten for the block's next stream
+	}
+}
+
+// ---------------------------------------------------------------------------------------------------------------
 // launchers (launch.h)
 // ---------------------------------------------------------------------------------------------------------------
+cudaError_t launchKlattLongTicks(const int64_t *offsets, uint32_t numStreams, const uint32_t *minDur, const uint32_t *fadeDur,
+                                 uint64_t *ticks, cudaStream_t stream) {
+	if (numStreams == 0) return cudaSuccess;
+	klatt_long_ticks_kernel<<<numStreams < kTicksMaxBlocks ? numStreams : kTicksMaxBlocks, kTicksBlock, 0, stream>>>(offsets, numStreams, minDur,
+	                                                                                                             fadeDur, ticks);
+	return cudaGetLastError();
+}
+
 cudaError_t launchKlattLongTimeline(const LongTable &T, cudaStream_t stream) {
 	if (T.numStreams > 1) klatt_long_timeline_kernel<true><<<T.numStreams, kTimelineTile, 0, stream>>>(T);
 	else klatt_long_timeline_kernel<false><<<1, kTimelineTile, 0, stream>>>(T);

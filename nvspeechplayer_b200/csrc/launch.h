@@ -98,6 +98,10 @@ struct Affine {
 };
 
 // Launchers: everything device-resident, scratch sized by the caller (api_long.cu).
+// ticks[s] = the ticks stream s's whole queue yields (the occupancy law of timelineTicks, host.h); offsets [numStreams + 1]
+// as validated by the host
+cudaError_t launchKlattLongTicks(const int64_t *offsets, uint32_t numStreams, const uint32_t *minDur, const uint32_t *fadeDur,
+                                 uint64_t *ticks, cudaStream_t stream);
 cudaError_t launchKlattLongTimeline(const LongTable &T, cudaStream_t stream);
 cudaError_t launchKlattLongPhase(const LongTable &T, uint32_t numChunks, uint32_t chunkTicks, uint64_t *advance, uint64_t *startPhase,
                                  PhaseChunk *chunks, double *startP, uint32_t *fail, bool serial, unsigned long long *launchCounter,

@@ -113,6 +113,8 @@ def load_library():
     L.speechPlayer_synthesizeLong.argtypes = [i32, vp, vp, vp, vp, u32, u64, u64, u32, vp, ctypes.c_ulonglong, i32, vp, vp]
     L.speechPlayer_synthesizeLongBatch.restype = ctypes.c_longlong
     L.speechPlayer_synthesizeLongBatch.argtypes = [i32, u32, vp, vp, vp, vp, vp, u64, vp, u32, vp, vp, vp, i32, vp, vp, vp]
+    L.speechPlayer_synthesizeLongBatchDevice.restype = ctypes.c_longlong
+    L.speechPlayer_synthesizeLongBatchDevice.argtypes = [i32, u32, vp, vp, vp, vp, vp, u64, vp, u32, vp, vp, vp, i32, vp, vp, vp, vp]
     _lib = L
     return L
 
@@ -264,51 +266,95 @@ def synthesize_long(sample_rate, frames, min_dur, fade_dur, is_null=None, seed=0
     return out[:got], ms.value, launches.value
 
 
-def synthesize_long_batch(fb, seed=0xB200, chunk_ticks=0, max_samples=None, device_out=None):
+def _device_queues(fb):
+    """(offsets, frames, min_dur, fade_dur, is_null) of ``fb`` when its queues are torch CUDA tensors -- an ipa.DeviceFrameBatch,
+    or any object with workloads.FrameBatch's queue fields as tensors (is_null may be None) -- else None."""
+    if not getattr(fb.offsets, "is_cuda", False):
+        return None
+    import torch
+    q = (fb.offsets, fb.frames, fb.min_dur, fb.fade_dur, getattr(fb, "is_null", None))
+    want = ((torch.int64,), (torch.float64,), (torch.int32, torch.uint32), (torch.int32, torch.uint32), (torch.uint8, torch.bool))
+    for name, t, dtypes in zip(("offsets", "frames", "min_dur", "fade_dur", "is_null"), q, want):
+        if t is None and name == "is_null":
+            continue
+        if not (getattr(t, "is_cuda", False) and t.device == fb.offsets.device and t.dtype in dtypes and t.is_contiguous()):
+            raise ValueError("device queues: %s must be a contiguous %s tensor on %s" % (name, " or ".join(map(str, dtypes)),
+                                                                                          fb.offsets.device))
+    if fb.frames.numel() != 47 * fb.min_dur.numel():
+        raise ValueError("device queues: frames must hold 47 values per request")
+    return q
+
+
+def _long_batch_entry(fb, seed, stream_ids, chunk_ticks, caps, out_offsets, serial, ms, launches, cuda_stream):
+    """(call(out, on_device), entry name): speechPlayer_synthesizeLongBatch for ``fb``'s host queues, or
+    speechPlayer_synthesizeLongBatchDevice for queues in device memory (on ``cuda_stream``, default: the device's current torch
+    stream).  The closure holds the queue arrays, so they live as long as it."""
+    L = load_library()
+    n = fb.num_streams
+    rest = lambda out, on_device: (seed, _ptr(stream_ids), chunk_ticks, _ptr(caps), out, _ptr(out_offsets), on_device, _ptr(serial),
+                                   None if ms is None else ctypes.byref(ms), None if launches is None else ctypes.byref(launches))
+    dq = _device_queues(fb)
+    if dq is None:
+        offsets = np.ascontiguousarray(fb.offsets, dtype=np.int64)
+        frames = np.ascontiguousarray(fb.frames, dtype=np.float64).reshape(-1, NUM_PARAMS)
+        m = np.ascontiguousarray(fb.min_dur, dtype=np.uint32)
+        f = np.ascontiguousarray(fb.fade_dur, dtype=np.uint32)
+        nul = None if fb.is_null is None else np.ascontiguousarray(fb.is_null, dtype=np.uint8)
+        return (lambda out, on_device: L.speechPlayer_synthesizeLongBatch(fb.sample_rate, n, _ptr(offsets), _ptr(frames), _ptr(m), _ptr(f),
+                                                                          _ptr(nul), *rest(out, on_device))), "speechPlayer_synthesizeLongBatch"
+    import torch
+    dev = dq[0].device
+    if cuda_stream is None:
+        cuda_stream = torch.cuda.current_stream(dev)
+    handle = cuda_stream.cuda_stream if hasattr(cuda_stream, "cuda_stream") else cuda_stream
+    ptrs = [None if t is None else (t.data_ptr() or None) for t in dq]
+
+    def call(out, on_device):
+        with torch.cuda.device(dev):
+            return L.speechPlayer_synthesizeLongBatchDevice(fb.sample_rate, n, *ptrs, *rest(out, on_device), handle)
+    return call, "speechPlayer_synthesizeLongBatchDevice"
+
+
+def _caps(max_samples, n):
+    return None if max_samples is None else np.ascontiguousarray(np.broadcast_to(np.asarray(max_samples, dtype=np.uint64), (n,)))
+
+
+def synthesize_long_batch(fb, seed=0xB200, chunk_ticks=0, max_samples=None, device_out=None, stream_ids=None, cuda_stream=None):
     """speechPlayer_synthesizeLongBatch: every stream of ``fb`` (a workloads.FrameBatch of whole, pre-queued queues) rendered
     with parallelism in time, all streams' chunks in one launch sequence.  Row s is what ``synthesize_long`` renders for
-    stream s with noise stream ``fb.stream_ids[s]``.  ``max_samples``: None, one cap for all streams, or one per stream.
+    stream s with noise stream ``stream_ids[s]`` (default: ``fb.stream_ids``, or 0..N-1 when ``fb`` has none).
+    ``max_samples``: None, one cap for all streams, or one per stream.
+    ``fb`` may hold its queues in device memory: an ipa.DeviceFrameBatch, or a FrameBatch-like object whose offsets, frames,
+    min_dur, fade_dur (and is_null, or None) are CUDA tensors.  They are then rendered in place by
+    speechPlayer_synthesizeLongBatchDevice on ``cuda_stream`` (a torch.cuda.Stream or raw handle; default: the device's current
+    torch stream), after whatever is queued there -- the producer of the queues needs no synchronisation -- and bit for bit as
+    the host route renders the same queues.
     Returns (packed int16 samples, out_offsets int64 [N+1], serial_phase uint8 [N], render_ms, kernel_launches); stream s is
     ``samples[out_offsets[s]:out_offsets[s+1]]`` (``split_rows``).  With ``device_out`` (a raw device address of at least
     ``long_batch_size(...)`` int16) the samples stay in HBM and the first element is the total sample count."""
-    L = load_library()
     n = fb.num_streams
-    offsets = np.ascontiguousarray(fb.offsets, dtype=np.int64)
-    frames = np.ascontiguousarray(fb.frames, dtype=np.float64).reshape(-1, NUM_PARAMS)
-    m = np.ascontiguousarray(fb.min_dur, dtype=np.uint32)
-    f = np.ascontiguousarray(fb.fade_dur, dtype=np.uint32)
-    nul = np.ascontiguousarray(fb.is_null, dtype=np.uint8)
-    ids = np.ascontiguousarray(fb.stream_ids, dtype=np.uint64)
-    caps = None if max_samples is None else np.ascontiguousarray(np.broadcast_to(np.asarray(max_samples, dtype=np.uint64), (n,)))
+    ids = getattr(fb, "stream_ids", None) if stream_ids is None else stream_ids
+    ids = None if ids is None else np.ascontiguousarray(ids, dtype=np.uint64)
     out_offsets = np.zeros(n + 1, dtype=np.int64)
     serial = np.zeros(n, dtype=np.uint8)
     ms, launches = ctypes.c_double(0), ctypes.c_ulonglong(0)
-
-    def call(out_ptr, on_device):
-        return L.speechPlayer_synthesizeLongBatch(fb.sample_rate, n, _ptr(offsets), _ptr(frames), _ptr(m), _ptr(f), _ptr(nul), seed,
-                                                  _ptr(ids), chunk_ticks, _ptr(caps), out_ptr, _ptr(out_offsets), on_device,
-                                                  _ptr(serial), ctypes.byref(ms), ctypes.byref(launches))
+    call, what = _long_batch_entry(fb, seed, ids, chunk_ticks, _caps(max_samples, n), out_offsets, serial, ms, launches, cuda_stream)
     if device_out is not None:
-        got = _check(call(device_out, 1), "speechPlayer_synthesizeLongBatch")
+        got = _check(call(device_out, 1), what)
         return got, out_offsets, serial, ms.value, launches.value
-    total = _check(call(None, 0), "speechPlayer_synthesizeLongBatch")
+    total = _check(call(None, 0), what)
     out = np.zeros(max(total, 1), dtype=np.int16)
-    got = _check(call(_ptr(out), 0), "speechPlayer_synthesizeLongBatch")
+    got = _check(call(_ptr(out), 0), what)
     return out[:got], out_offsets, serial, ms.value, launches.value
 
 
-def long_batch_size(fb, max_samples=None):
-    """(total samples, out_offsets) of synthesize_long_batch for ``fb``: a size query, no device needed."""
-    L = load_library()
+def long_batch_size(fb, max_samples=None, cuda_stream=None):
+    """(total samples, out_offsets) of synthesize_long_batch for ``fb``: a size query.  Host queues need no device; queues in
+    device memory are sized on the device (on ``cuda_stream``, as synthesize_long_batch)."""
     n = fb.num_streams
-    offsets = np.ascontiguousarray(fb.offsets, dtype=np.int64)
-    m = np.ascontiguousarray(fb.min_dur, dtype=np.uint32)
-    f = np.ascontiguousarray(fb.fade_dur, dtype=np.uint32)
-    caps = None if max_samples is None else np.ascontiguousarray(np.broadcast_to(np.asarray(max_samples, dtype=np.uint64), (n,)))
     out_offsets = np.zeros(n + 1, dtype=np.int64)
-    got = L.speechPlayer_synthesizeLongBatch(fb.sample_rate, n, _ptr(offsets), None, _ptr(m), _ptr(f), None, 0, None, 0, _ptr(caps),
-                                             None, _ptr(out_offsets), 0, None, None, None)
-    return _check(got, "speechPlayer_synthesizeLongBatch"), out_offsets
+    call, what = _long_batch_entry(fb, 0, None, 0, _caps(max_samples, n), out_offsets, None, None, None, cuda_stream)
+    return _check(call(None, 0), what), out_offsets
 
 
 def split_rows(samples, out_offsets):
