@@ -109,6 +109,12 @@ struct alignas(16) FadePlanF32 {
 };
 static_assert(sizeof(FadePlanF32) % 16 == 0, "plan records are read with 16-byte loads");
 
+// affine map of one two-pole section over a run of ticks, (y, d)_end = P (y, d)_start + z, row-major P: what pass 1 of a
+// time-parallel stage leaves for the scan (klatt_tick_core.cuh)
+struct Affine {
+	float p00, p01, p10, p11, zy, zd;
+};
+
 struct GenStateF32 {
 	double pitchPos;               // glottal phase in cycles, FP64 and accumulated exactly like the reference does
 	double pitch;                  // cur.voicePitch

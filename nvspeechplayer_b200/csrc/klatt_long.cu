@@ -29,13 +29,15 @@
 //                   rN0+rNP, r6 ... r1; the last stage fuses the mix, gain, clamp and int16 store (:207-208).
 //
 // The arithmetic of a tick is the FP32 formulation of klatt_f32_core.cuh (delta-form sections, pole recurrences
-// during fades, FP64 pitch and phase); inside a fade the pole is re-based on its closed form every 64 ticks.  Parity
+// during fades, FP64 pitch and phase), stated once for this path and the pull path in klatt_tick_core.cuh; inside a fade
+// the pole is re-based on its closed form every 64 ticks (here: FP64 poleTerms of the frames' end points).  Parity
 // with the serial kernels is by tolerance (re-association), not bit for bit: the bar is the FP32 bar (<= 1 LSB on
 // >= 99.9 %, >= 60 dB SNR against the reference).
 #include <cuda_runtime.h>
 #include "klatt_common.h"
 #include "klatt_f32_core.cuh"
 #include "klatt_long_phase.cuh"
+#include "klatt_tick_core.cuh"
 #include "launch.h"
 
 namespace klatt {
@@ -134,7 +136,7 @@ struct DirWalk {
 		d0 = p.dir0[slot]; ds = p.dirStep[slot]; dF = p.dirFinal[slot];
 	}
 	__device__ __forceinline__ float at(uint32_t c, uint32_t F) const {
-		return c == 0 ? prevFinal : (c < F ? fmaf((float)c, ds, d0) : dF);
+		return dirLaw(c, F, prevFinal, d0, ds, dF);
 	}
 };
 
@@ -147,84 +149,26 @@ struct DepthWalk {
 		d0 = p.depth0; ds = p.depthStep; dF = p.depthFinal;
 	}
 	__device__ __forceinline__ double at(uint32_t c, uint32_t F) const {
-		return c == 0 ? prevFinal : (c < F ? fma((double)(float)c, ds, d0) : dF);
+		return depthLaw(c, F, prevFinal, d0, ds, dF);
 	}
 };
 
-// zeta = 1 - pole of one section along the stream
-struct PoleWalk {
-	float zr, zi, wr, wi;
-	__device__ void exact(const LongStream &L, uint32_t j, uint32_t k, uint32_t F, int r) {
-		double f0, f1, b0, b1;
-		fadeEnds(L, j, resFreqParam(r), f0, f1);
-		fadeEnds(L, j, resBwParam(r), b0, b1);
-		if (f1 != f1) f1 = f0;
-		if (b1 != b1) b1 = b0;
-		const double ratio = (double)k / (double)F;
-		poleTerms(f0 + ((f1 - f0) * ratio), b0 + ((b1 - b0) * ratio), 1.0 / (double)L.sampleRate, zr, zi);
-	}
-	// state as it is AFTER the tick before (j, c)
-	__device__ void seek(const LongStream &L, uint32_t j, uint32_t c, uint32_t F, int r) {
-		wr = wi = 0.0f;
-		if (c <= 1) {
-			if (j > 0) { zr = L.plans[j - 1].zFre[r]; zi = L.plans[j - 1].zFim[r]; }
-			else { zr = zi = 0.0f; }
-		} else if (c <= F) {  // ticks 1 .. c-1 of the fade are behind us
-			if (c - 1 < F) { exact(L, j, c - 1, F, r); wr = L.plans[j].wre[r]; wi = L.plans[j].wim[r]; }
-		} else {
-			zr = L.plans[j].zFre[r]; zi = L.plans[j].zFim[r];
-		}
-	}
-	// the update of tick (j, c): afterwards (zr, zi) is what the tick renders with
-	__device__ __forceinline__ void tick(const LongStream &L, uint32_t j, uint32_t c, uint32_t F, int r) {
-		if (c == 0 || c > F) return;  // pop tick: stale; after the landing: constant
-		if (c == F) {
-			zr = L.plans[j].zFre[r]; zi = L.plans[j].zFim[r]; wr = wi = 0.0f;
-			return;
-		}
-		if (c == 1) {
-			const FadePlanF32 &p = L.plans[j];
-			zr = p.z0re[r]; zi = p.z0im[r]; wr = p.wre[r]; wi = p.wim[r];
-		}
-		if ((c & (uint32_t)(kCoarseTicks - 1)) == 0) {
-			exact(L, j, c, F, r);  // drift control: back onto the closed form
-			return;
-		}
-		float tr = fmaf(-zr, wr, wr);
-		tr = fmaf(zi, wi, tr);
-		float ti = fmaf(-zr, wi, wi);
-		ti = fmaf(-zi, wr, ti);
-		zr += tr;
-		zi += ti;
-	}
-	// a plain interior fade tick (1 < c < F, not a multiple of kCoarseTicks): the last six operations of tick()
-	__device__ __forceinline__ void step() {
-		float tr = fmaf(-zr, wr, wr);
-		tr = fmaf(zi, wi, tr);
-		float ti = fmaf(-zr, wi, wi);
-		ti = fmaf(-zi, wr, ti);
-		zr += tr;
-		zi += ti;
-	}
-	__device__ __forceinline__ void coef(float &a, float &rho) const {
-		a = fmaf(zr, zr, zi * zi);
-		rho = fmaf(2.0f, zr, -a);
-	}
-};
-
-__device__ __forceinline__ bool n0InvAt(const LongStream &L, uint32_t j, uint32_t c, uint32_t F) {
-	if (c == 0) return j > 0 ? L.plans[j - 1].n0InvFinal != 0 : false;
-	return (c < F ? L.plans[j].n0InvFade : L.plans[j].n0InvFinal) != 0;
+// PoleWalk of section r along the stream: the closed form in double from the end points of request j's fade
+__device__ void longPoleExact(const LongStream &L, uint32_t j, uint32_t k, uint32_t F, int r, float &zr, float &zi) {
+	double f0, f1, b0, b1;
+	fadeEnds(L, j, resFreqParam(r), f0, f1);
+	fadeEnds(L, j, resBwParam(r), b0, b1);
+	if (f1 != f1) f1 = f0;
+	if (b1 != b1) b1 = b0;
+	const double ratio = (double)k / (double)F;
+	poleTerms(f0 + ((f1 - f0) * ratio), b0 + ((b1 - b0) * ratio), 1.0 / (double)L.sampleRate, zr, zi);
 }
-
-// cur.voicePitch on tick (j, c)
-__device__ __forceinline__ double pitchAt(const LongStream &L, uint32_t j, uint32_t c, uint32_t F) {
-	if (c == 0) return L.pitchPop[j];
-	const double o = L.pitchOld[j], n = L.pitchNew[j];
-	if (c < F) return (n != n) ? o : o + ((n - o) * ((double)c / (double)F));
-	const double landing = (n != n) ? o : o + ((n - o) * 1.0);
-	if (c <= F + 1) return landing;
-	return landing + (double)(c - F - 1) * L.pitchInc[j];
+__device__ void longPoleSeek(PoleWalk &w, const LongStream &L, uint32_t j, uint32_t c, uint32_t F, int r) {
+	w.seek(L.plans[j], c, F, r, j > 0 ? L.plans[j - 1].zFre[r] : 0.0f, j > 0 ? L.plans[j - 1].zFim[r] : 0.0f,
+	       [&](uint32_t k, float &zr, float &zi) { longPoleExact(L, j, k, F, r, zr, zi); });
+}
+__device__ __forceinline__ void longPoleTick(PoleWalk &w, const LongStream &L, uint32_t j, uint32_t c, uint32_t F, int r) {
+	w.tick(L.plans[j], c, F, r, [&](uint32_t k, float &zr, float &zi) { longPoleExact(L, j, k, F, r, zr, zi); });
 }
 
 // vibrato: per-tick increment on tick (j, c), and the phase after the ticks before (j, c)
@@ -234,18 +178,9 @@ struct VibWalk {
 		vPrev = j > 0 ? L.plans[j - 1].vibIncFinal : 0;
 		v0 = L.plans[j].vibInc0; vs = L.plans[j].vibIncStep; vF = L.plans[j].vibIncFinal;
 	}
-	__device__ __forceinline__ int64_t inc(uint32_t c, uint32_t F) const {
-		return c == 0 ? vPrev : (c < F ? v0 + (int64_t)c * vs : vF);
-	}
+	__device__ __forceinline__ int64_t inc(uint32_t c, uint32_t F) const { return vibIncLaw(c, F, vPrev, v0, vs, vF); }
 	// sum of inc(c') for c' in [0, c)
-	__device__ uint64_t before(uint32_t c, uint32_t F) const {
-		if (c == 0) return 0;
-		uint64_t s = (uint64_t)vPrev;
-		const uint64_t kmax = (c - 1 < F - 1) ? c - 1 : F - 1;  // fade ticks 1 .. kmax are behind us
-		s += kmax * (uint64_t)v0 + (uint64_t)vs * (kmax * (kmax + 1) / 2);
-		if (c > F) s += (uint64_t)(c - F) * (uint64_t)vF;
-		return s;
-	}
+	__device__ uint64_t before(uint32_t c, uint32_t F) const { return vibBeforeLaw(c, F, vPrev, v0, vs, vF); }
 };
 
 }  // namespace
@@ -370,7 +305,7 @@ klatt_long_timeline_kernel(LongTable T) {
 		if (in && !null) {
 			const double curGuess = realPrevInTile ? sPNew[rLocal] + (double)sHold[rLocal] * sInc[rLocal] : carryEnd;
 			const double pOld = prevNull ? myP0 : curGuess;   // :64-67 copies the frame BEFORE :71 moves new.voicePitch
-			const double landing = (myPNew != myPNew) ? pOld : pOld + ((myPNew - pOld) * 1.0);
+			const double landing = pitchLanding(pOld, myPNew);
 			gLanding[tid] = landing;
 			gEnd[tid] = glideExact(landing, myInc, myHold);  // hold ticks F+2 .. occ-1: one addition each (src/frame.cpp:77)
 		}
@@ -390,7 +325,7 @@ klatt_long_timeline_kernel(LongTable T) {
 				else {
 					pOldTrue = prevNull ? myP0 : curTrue;
 					pNewTrue = myPNew;
-					const double landing = (pNewTrue != pNewTrue) ? pOldTrue : pOldTrue + ((pNewTrue - pOldTrue) * 1.0);
+					const double landing = pitchLanding(pOldTrue, pNewTrue);
 					changed = __double_as_longlong(landing) != __double_as_longlong(gLanding[tid]);
 					if (changed) { gLanding[tid] = landing; newEnd = glideExact(landing, myInc, myHold); }
 				}
@@ -412,7 +347,7 @@ klatt_long_timeline_kernel(LongTable T) {
 					double pOld = pitchCur, pNew = nul ? pitchCur : sPNew[k];
 					if (!nul && (oldIsNull || base + k == 0)) pOld = sP0[k];
 					oOld[k] = pOld; oNew[k] = pNew; oInc[k] = sInc[k];
-					const double landing = (pNew != pNew) ? pOld : pOld + ((pNew - pOld) * 1.0);
+					const double landing = pitchLanding(pOld, pNew);
 					pitchCur = glideExact(landing, sInc[k], sHold[k]);
 					oldIsNull = nul;
 				}
@@ -440,7 +375,7 @@ struct SourceWalk {
 	uint64_t vibPos;
 	uint32_t loaded;
 	double pPop, pOld, pNew, pInc;  // pitch of the request in force: stale pop-tick value, fade end points, hold glide
-	double pitchHold;               // cur.voicePitch while holding, accumulated like the reference does (src/frame.cpp:77)
+	double pitchHold;               // cur.voicePitch on the tick before (pitchTick)
 	__device__ void loadReq(const LongStream &L, bool full) {
 		vw.load(L, cur.j);
 		depth.load(L, cur.j);
@@ -452,33 +387,21 @@ struct SourceWalk {
 		pPop = L.pitchPop[cur.j]; pOld = L.pitchOld[cur.j]; pNew = L.pitchNew[cur.j]; pInc = L.pitchInc[cur.j];
 		loaded = cur.j;
 	}
-	__device__ __forceinline__ double landing() const { return (pNew != pNew) ? pOld : pOld + ((pNew - pOld) * 1.0); }
 	__device__ void seek(const LongStream &L, uint64_t t, bool full) {
 		cur.seek(L, t);
 		pitchHold = 0.0;
 		if (cur.j >= L.nReq) { loaded = cur.j; return; }
 		loadReq(L, full);
 		vibPos = L.vibPosStart[cur.j] + vw.before(cur.c, cur.F);
-		// in the middle of a hold: the value the previous tick used, (c-1) - F - 1 additions after the landing
-		if (cur.c >= cur.F + 2) pitchHold = glideExact(landing(), pInc, (uint64_t)(cur.c - cur.F - 2));
+		// in the middle of a hold: the value the previous tick used
+		if (cur.c >= cur.F + 2) pitchHold = pitchLaw(cur.c - 1, cur.F, pPop, pOld, pNew, pInc);
 	}
-	// The increment of the glottal phase on this tick, the double the serial kernel adds (klatt_f32_core.cuh OscChain:
-	// vibrato sine in FP32, its depth, pitch * (1 + vibrato) and the correctly rounded division by the sample rate in FP64; reference
-	// src/speechWaveGenerator.cpp:73-74).  In a fade the serial kernels sum the depth's steps where this evaluates the depth in
-	// closed form: the two differ by a few FP64 ulps.  cur.voicePitch: stale on the pop tick, old+(new-old)*ratio in the fade
-	// (src/frame.cpp:49-52), the landing value on the landing and swap ticks, then += inc per tick (:77).
+	// The increment of the glottal phase on this tick, the double the serial kernel adds (klatt_f32_core.cuh OscChain).  In a
+	// fade the serial kernels sum the depth's steps where this evaluates the depth in closed form: the two differ by a few FP64
+	// ulps.
 	__device__ __forceinline__ double quotOfTick(double srD, double srInv) {
 		const uint32_t c = cur.c, F = cur.F;
-		vibPos += (uint64_t)vw.inc(c, F);
-		float vph = (float)(int32_t)(uint32_t)(vibPos >> 32) * 2.3283064365386963e-10f;
-		const double vib1 = fma((double)sinTurns(vph), depth.at(c, F), 1.0);
-		double pitch;
-		if (c == 0) pitch = pPop;
-		else if (c < F) pitch = (pNew != pNew) ? pOld : pOld + ((pNew - pOld) * ((double)c / (double)F));
-		else if (c <= F + 1) { pitch = landing(); pitchHold = pitch; }
-		else { pitchHold += pInc; pitch = pitchHold; }
-		const double m = pitch * vib1;
-		return divideBySampleRate(m, srD, srInv);
+		return glottalInc(vibPos, vw.inc(c, F), pitchTick(pitchHold, true, c, F, pPop, pOld, pNew, pInc), depth.at(c, F), srD, srInv);
 	}
 	__device__ __forceinline__ void next(const LongStream &L, bool full) {
 		cur.next(L);
@@ -698,9 +621,8 @@ klatt_long_source_kernel(LongTable T, uint32_t chunkTicks, uint32_t numChunks, c
 	float aspLast = 0.0f, fricLast = 0.0f;
 	for (uint64_t g = (t0 > (uint64_t)kWarmTicks ? t0 - kWarmTicks : 0); g < t0; ++g) {
 		Philox4 b = noiseBlock(L.seed, L.streamId, g >> 1);
-		const uint32_t wA = (g & 1) ? b.w[2] : b.w[0], wF = (g & 1) ? b.w[3] : b.w[1];
-		aspLast = fmaf(0.75f, aspLast, bitsToFloat(0x4B000000u | (wA >> 9)) - 8388608.0f);
-		fricLast = fmaf(0.75f, fricLast, bitsToFloat(0x4B000000u | (wF >> 9)) - 8388608.0f);
+		aspLast = colourNoise(aspLast, (g & 1) ? b.w[2] : b.w[0]);
+		fricLast = colourNoise(fricLast, (g & 1) ? b.w[3] : b.w[1]);
 	}
 	SourceWalk w;
 	w.seek(L, t0, true);
@@ -712,17 +634,8 @@ klatt_long_source_kernel(LongTable T, uint32_t chunkTicks, uint32_t numChunks, c
 		const uint32_t wA = (t & 1) ? blk.w[2] : blk.w[0], wF = (t & 1) ? blk.w[3] : blk.w[1];
 		const uint32_t c = w.cur.c, F = w.cur.F;
 		pos = phaseStep(pos, w.quotOfTick(srD, srInv));
-		const float voice = (float)pos;
-		aspLast = fmaf(0.75f, aspLast, bitsToFloat(0x4B000000u | (wA >> 9)) - 8388608.0f);
-		float asp = aspLast * (0.2f * kDrawScale);
-		float turb = asp * w.vta.at(c, F);
-		if (voice < w.goq.at(c, F)) turb *= 0.01f;
-		float v = (fmaf(voice, 2.0f, -1.0f) + turb) * w.va.at(c, F);
-		float src = fmaf(asp, w.aa.at(c, F), v);
-		const float halfGain = w.pfg.at(c, F) * 0.5f;
-		ci[t] = src * halfGain;
-		fricLast = fmaf(0.75f, fricLast, bitsToFloat(0x4B000000u | (wF >> 9)) - 8388608.0f);
-		pin[t] = fricLast * (((0.3f * kDrawScale) * w.fa.at(c, F)) * halfGain);
+		excitation((float)pos, wA, wF, w.vta.at(c, F), w.goq.at(c, F), w.va.at(c, F), w.aa.at(c, F), w.fa.at(c, F), w.pfg.at(c, F),
+		           aspLast, fricLast, ci[t], pin[t]);
 		w.next(L, true);
 	}
 	if (t1 < total) {  // the chunk whose run starts at t1 must have been handed exactly the value this run arrives with
@@ -734,18 +647,9 @@ klatt_long_source_kernel(LongTable T, uint32_t chunkTicks, uint32_t numChunks, c
 // ---------------------------------------------------------------------------------------------------------------
 // resonator stages
 // ---------------------------------------------------------------------------------------------------------------
-enum Stage : int { kStageParallel = 0, kStageNasal = 1, kStageCascade = 2, kStageLast = 3 };
-
-template <int STAGE> struct StageTraits {
-	static constexpr int NR = STAGE == kStageParallel ? 6 : 1;  // scanned sections
-};
-
-// One chunk of one stage.  PASS 1: from zero state, also accumulate P.  PASS 2: from the scanned start state, write
-// the stage's output signal (or, for the last stage, the int16 samples).
-//   kStageParallel: in = pin, sections 8..13, out = par (:170-180)
-//   kStageNasal   : in = ci, rN0 (FIR) then rNP (section 1), out = x after the caNP mix (:148-150)
-//   kStageCascade : in = x, section `res`, out = its output (:151-156)
-//   kStageLast    : like kStageCascade for r1, then (x + par) * outputGain * 4000, clamp, truncate (:207-208)
+// One chunk of one stage (klatt_tick_core.cuh StageTick).  PASS 1: from zero state, also accumulate P.  PASS 2: from the
+// scanned start state, write the stage's output signal (or, for the last stage, the int16 samples).  The parallel stage
+// reads pin and writes par, the nasal stage reads ci, the last stage also reads par.
 // Memory: thread i of a warp walks chunk (w + i), i.e. addresses chunkTicks * 4 bytes apart -- a warp-wide access to tick t
 // of 32 chunks touches 32 different sectors (round 1: 8 x the algorithmic traffic on the stores, long_scoreboard 28 cycles
 // per issue).  The signals therefore move through a shared-memory tile per warp: 32 chunks x 32 ticks, loaded and stored as
@@ -799,26 +703,23 @@ klatt_long_stage_kernel(LongTable T, uint32_t chunkTicks, uint32_t numChunks, in
 		}
 	};
 	uint32_t loaded = 0;
-	float y[NR], d[NR];
-	float p00[NR], p01[NR], p10[NR], p11[NR];
-#pragma unroll
-	for (int k = 0; k < NR; ++k) { y[k] = 0.0f; d[k] = 0.0f; p00[k] = 1.0f; p01[k] = 0.0f; p10[k] = 0.0f; p11[k] = 1.0f; }
-	float in1 = 0.0f, in2 = 0.0f;  // the FIR section needs the two inputs before the chunk
+	StageTick<STAGE, PASS> st;
+	st.start();  // (the FIR section needs the two inputs before the chunk)
 	if (live) {
 		cur.seek(L, t0);
 #pragma unroll
-		for (int k = 0; k < NR; ++k) pw[k].seek(L, cur.j, cur.c, cur.F, STAGE == kStageParallel ? kResParallel + k : res);
-		if (STAGE == kStageNasal) pw0.seek(L, cur.j, cur.c, cur.F, kResN0);
+		for (int k = 0; k < NR; ++k) longPoleSeek(pw[k], L, cur.j, cur.c, cur.F, STAGE == kStageParallel ? kResParallel + k : res);
+		if (STAGE == kStageNasal) longPoleSeek(pw0, L, cur.j, cur.c, cur.F, kResN0);
 		loadDirs();
 		loaded = cur.j;
 		if (PASS == 2) {
 #pragma unroll
-			for (int k = 0; k < NR; ++k) { float2 s = startState[(size_t)ch * NR + k]; y[k] = s.x; d[k] = s.y; }
+			for (int k = 0; k < NR; ++k) { float2 s = startState[(size_t)ch * NR + k]; st.y[k] = s.x; st.d[k] = s.y; }
 		}
 		if (STAGE == kStageNasal) {
 			const size_t v0 = (size_t)cb * chunkTicks + t0;
-			if (t0 >= 1) in1 = in[v0 - 1];
-			if (t0 >= 2) in2 = in[v0 - 2];
+			if (t0 >= 1) st.in1 = in[v0 - 1];
+			if (t0 >= 2) st.in2 = in[v0 - 2];
 		}
 	}
 	for (uint32_t tile = 0; tile < chunkTicks; tile += kTile) {
@@ -834,51 +735,10 @@ klatt_long_stage_kernel(LongTable T, uint32_t chunkTicks, uint32_t numChunks, in
 		if (live) {
 			const uint64_t tb = t0 + tile;
 			const int qEnd = (tb + kTile <= t1) ? kTile : (tb < t1 ? (int)(t1 - tb) : 0);
-			// One tick of the stage with the coefficients of that tick given: the FIR anti-resonator (nasal stage), the scanned
-			// sections, the affine map (pass 1), the stage's output (pass 2).
-			auto tickWith = [&](int q, const float *a, const float *rho, const float *mixv, float extraV, bool n0Inv, float a0, float rho0) {
-				float x = tIn[wib][lane][q];
-				const float xin = x;
-				if (STAGE == kStageNasal) {  // rN0 on inputs: src/speechWaveGenerator.cpp:129-135 with anti == true
-					const float dprev = in1 - in2;
-					const float dx = x - in1;
-					const float dx1 = fmaf(-rho0, dprev, dprev);
-					x = n0Inv ? fmaf(dx - dx1, fastRcp(a0), in1) : fmaf(a0, dx, dx1 + in1);
-					in2 = in1;
-					in1 = xin;
-				}
-				float acc = 0.0f;
-#pragma unroll
-				for (int k = 0; k < NR; ++k) {
-					float w = fmaf(-rho[k], d[k], d[k]);
-					w = fmaf(-a[k], y[k], w);
-					const float dn = fmaf(a[k], x, w);
-					d[k] = dn;
-					y[k] += dn;
-					if (PASS == 1) {  // P <- A P with A = [[1-a, 1-rho], [-a, 1-rho]] acting on (y, d)
-						const float g = 1.0f - rho[k];
-						const float n10 = fmaf(-a[k], p00[k], g * p10[k]), n11 = fmaf(-a[k], p01[k], g * p11[k]);
-						p00[k] += n10; p01[k] += n11;
-						p10[k] = n10; p11[k] = n11;
-					}
-					if (STAGE == kStageParallel) acc = fmaf(y[k] - x, mixv[k], acc);
-				}
-				if (PASS == 2) {
-					float o;
-					if (STAGE == kStageParallel) {
-						o = fmaf(x - acc, extraV, acc);
-					} else if (STAGE == kStageNasal) {
-						o = fmaf(y[0] - xin, extraV, xin);
-					} else if (STAGE == kStageCascade) {
-						o = y[0];
-					} else {
-						float sgn = (y[0] + tPar[kHasPar ? wib : 0][kHasPar ? lane : 0][q]) * (extraV * 4000.0f);
-						sgn = fminf(sgn, 32000.0f);
-						sgn = fmaxf(sgn, -32000.0f);
-						o = (float)(int)sgn;  // the int16 value, exactly representable
-					}
-					tOut[wib][lane][q] = o;
-				}
+			auto tickAt = [&](int q, StageCoefs<STAGE> &co) {
+				if (STAGE == kStageNasal) co.rcp0 = co.inv ? fastRcp(co.a0) : 0.0f;
+				const float o = st(tIn[wib][lane][q], kHasPar ? tPar[kHasPar ? wib : 0][kHasPar ? lane : 0][q] : 0.0f, co);
+				if (PASS == 2) tOut[wib][lane][q] = o;
 			};
 			// Events, not branches (as in the batch kernels): a tick that may change something -- the pop tick, the first fade
 			// tick, a drift-control point, the landing, the first tick of a tile -- runs the general code; the ticks that follow
@@ -886,23 +746,24 @@ klatt_long_stage_kernel(LongTable T, uint32_t chunkTicks, uint32_t numChunks, in
 			// plain pole steps) run a tight loop with no frame-manager logic.  Same operations on the same values per tick.
 			int q = 0;
 			while (q < qEnd) {
-				float a[NR], rho[NR], mixv[NR], a0 = 0.0f, rho0 = 0.0f, extraV = 0.0f;
-				bool n0Inv = false;
+				StageCoefs<STAGE> co;
+				co.extra = co.a0 = co.rho0 = co.rcp0 = 0.0f;
+				co.inv = false;
 				{
 					const uint32_t j = cur.j, c = cur.c, F = cur.F;
 					if (STAGE == kStageNasal) {
-						pw0.tick(L, j, c, F, kResN0);
-						pw0.coef(a0, rho0);
-						n0Inv = n0InvAt(L, j, c, F);
+						longPoleTick(pw0, L, j, c, F, kResN0);
+						pw0.coef(co.a0, co.rho0);
+						co.inv = n0InvLaw(c, F, j > 0 ? L.plans[j - 1].n0InvFinal : 0u, L.plans[j].n0InvFade, L.plans[j].n0InvFinal);
 					}
 #pragma unroll
 					for (int k = 0; k < NR; ++k) {
-						pw[k].tick(L, j, c, F, STAGE == kStageParallel ? kResParallel + k : res);
-						pw[k].coef(a[k], rho[k]);
-						mixv[k] = STAGE == kStageParallel ? mix[k].at(c, F) : 0.0f;
+						longPoleTick(pw[k], L, j, c, F, STAGE == kStageParallel ? kResParallel + k : res);
+						pw[k].coef(co.a[k], co.rho[k]);
+						co.mix[k] = STAGE == kStageParallel ? mix[k].at(c, F) : 0.0f;
 					}
-					if (STAGE != kStageCascade) extraV = extra.at(c, F);
-					tickWith(q, a, rho, mixv, extraV, n0Inv, a0, rho0);
+					if (STAGE != kStageCascade) co.extra = extra.at(c, F);
+					tickAt(q, co);
 					++q;
 					cur.next(L);
 					if (cur.j != loaded && cur.j < L.nReq) { loadDirs(); loaded = cur.j; }
@@ -912,7 +773,7 @@ klatt_long_stage_kernel(LongTable T, uint32_t chunkTicks, uint32_t numChunks, in
 				if (c > F) {  // inside a hold: nothing moves until the request ends
 					uint32_t n = (uint32_t)(qEnd - q);
 					if ((uint64_t)n > cur.left) n = (uint32_t)cur.left;
-					for (uint32_t i = 0; i < n; ++i) tickWith(q + (int)i, a, rho, mixv, extraV, n0Inv, a0, rho0);
+					for (uint32_t i = 0; i < n; ++i) tickAt(q + (int)i, co);
 					q += (int)n;
 					cur.advance(L, n);
 					if (cur.j != loaded && cur.j < L.nReq) { loadDirs(); loaded = cur.j; }
@@ -923,15 +784,18 @@ klatt_long_stage_kernel(LongTable T, uint32_t chunkTicks, uint32_t numChunks, in
 					if (n > toGrid) n = toGrid;
 					for (uint32_t i = 0; i < n; ++i) {
 						const uint32_t ci = c + i;
-						if (STAGE == kStageNasal) { pw0.step(); pw0.coef(a0, rho0); }
+						if (STAGE == kStageNasal) {
+							pw0.step();
+							pw0.coef(co.a0, co.rho0);
+						}
 #pragma unroll
 						for (int k = 0; k < NR; ++k) {
 							pw[k].step();
-							pw[k].coef(a[k], rho[k]);
-							if (STAGE == kStageParallel) mixv[k] = mix[k].at(ci, F);
+							pw[k].coef(co.a[k], co.rho[k]);
+							if (STAGE == kStageParallel) co.mix[k] = mix[k].at(ci, F);
 						}
-						if (STAGE != kStageCascade) extraV = extra.at(ci, F);
-						tickWith(q + (int)i, a, rho, mixv, extraV, n0Inv, a0, rho0);
+						if (STAGE != kStageCascade) co.extra = extra.at(ci, F);
+						tickAt(q + (int)i, co);
 					}
 					q += (int)n;
 					cur.advance(L, n);  // (stays inside the request: n <= F - c < left)
@@ -958,10 +822,7 @@ klatt_long_stage_kernel(LongTable T, uint32_t chunkTicks, uint32_t numChunks, in
 		// then exactly the zero state it starts from, with no change to the scan.  (Nothing reads a stream's last map otherwise.)
 #pragma unroll
 		for (int k = 0; k < NR; ++k) {
-			Affine m;
-			m.p00 = p00[k]; m.p01 = p01[k]; m.p10 = p10[k]; m.p11 = p11[k]; m.zy = y[k]; m.zd = d[k];
-			if (lastOfStream) m = Affine{0.0f, 0.0f, 0.0f, 0.0f, 0.0f, 0.0f};
-			maps[(size_t)ch * NR + k] = m;
+			maps[(size_t)ch * NR + k] = lastOfStream ? Affine{0.0f, 0.0f, 0.0f, 0.0f, 0.0f, 0.0f} : st.map(k);
 		}
 	}
 }

@@ -122,15 +122,15 @@ __device__ uint64_t blockExclusiveU64(uint64_t own, uint64_t *warpSum) {
 
 template <int STAGE>
 __device__ __forceinline__ void runStage(const PullCtx &X, uint32_t ch, int res, PullAffineD *warpTotal) {
-	constexpr int NR = PullStageTraits<STAGE>::NR;
-	PullAffine maps[NR];
+	constexpr int NR = StageTraits<STAGE>::NR;
+	Affine maps[NR];
 	PullStart st[NR];
-	PullPole poles[NR + 1];
+	PoleWalk poles[NR + 1];
 	float fir[2] = {0.0f, 0.0f};
 	pullStage<STAGE, 1>(X, ch, res, maps, nullptr, fir, poles);
 #pragma unroll
 	for (int k = 0; k < NR; ++k) {
-		const int r = STAGE == kPullParallel ? kResParallel + k : res;
+		const int r = STAGE == kStageParallel ? kResParallel + k : res;
 		const PullAffineD pre = blockExclusive(pullToD(maps[k]), seedOf(X.state->y[r], X.state->d[r]), warpTotal);
 		st[k].y = (float)pre.zy;
 		st[k].d = (float)pre.zd;
@@ -215,13 +215,13 @@ __device__ __forceinline__ void pullBlock(PullCtx X, const PullSeg *__restrict__
 	__syncthreads();  // the FIR section of the nasal stage reads its neighbours' last two cascade inputs
 	mark(X, 4);
 
-	runStage<kPullParallel>(X, ch, 0, warpTotal);
+	runStage<kStageParallel>(X, ch, 0, warpTotal);
 	mark(X, 5);
-	runStage<kPullNasal>(X, ch, kResNP, warpTotal);
+	runStage<kStageNasal>(X, ch, kResNP, warpTotal);
 	mark(X, 6);
-	for (int r = kResCascade; r < kResParallel - 1; ++r) runStage<kPullCascade>(X, ch, r, warpTotal);
+	for (int r = kResCascade; r < kResParallel - 1; ++r) runStage<kStageCascade>(X, ch, r, warpTotal);
 	mark(X, 7);
-	runStage<kPullLast>(X, ch, kResParallel - 1, warpTotal);
+	runStage<kStageLast>(X, ch, kResParallel - 1, warpTotal);
 
 	__syncthreads();
 	{

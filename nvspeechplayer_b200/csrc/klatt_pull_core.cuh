@@ -2,7 +2,8 @@
 // (speechPlayer_synthesize(handle, n, buf), the call the NVDA audio thread makes, reference
 // nvdaAddon/synthDrivers/nvSpeechPlayer/__init__.py:56-82) rendered by ONE thread block, parallel in time, with the
 // state of the stream carried in and out.  It is klatt_long.cu's scheme (affine maps of the two-pole sections over a
-// chunk, composed by a scan) brought down to chunks of <= 16 ticks held in shared memory:
+// chunk, composed by a scan) brought down to chunks of <= 16 ticks held in shared memory, and the tick both render is
+// klatt_tick_core.cuh's:
 //
 //   host   the frame manager runs at REQUEST granularity in FP64, exactly as reference src/frame.cpp:41-115 (pop,
 //          NULL-frame rewrites, swap, hold glide, drain, purge): pull_manager.h.  For a pull it emits the runs of ticks
@@ -21,6 +22,7 @@
 #pragma once
 #include "klatt_common.h"
 #include "klatt_f32_core.cuh"
+#include "klatt_tick_core.cuh"
 
 namespace klatt {
 
@@ -85,52 +87,22 @@ struct PullBatchItem {
 	int16_t *pcmOut;
 };
 
-// affine map of one section over one chunk, (y, d)_end = P (y, d)_start + z, row-major P
-struct PullAffine {
-	float p00, p01, p10, p11, zy, zd;
-};
+// the pull path's names for the records of klatt_tick_core.cuh (the host model in tests/hostsim uses them)
+typedef Affine PullAffine;
+typedef PoleWalk PullPole;
+template <int STAGE> using PullStageTraits = StageTraits<STAGE>;
+constexpr int kPullParallel = kStageParallel, kPullNasal = kStageNasal, kPullCascade = kStageCascade, kPullLast = kStageLast;
+
 struct PullStart {
 	float y, d;
 };
 
-// vibrato: increment on tick (seg, c) and the sum of the increments of ticks [0, c) of the request
-KLATT_HD int64_t pullVibInc(const PullSeg &s, uint32_t c) {
-	return c == 0 ? s.vibIncStale : (c < s.F ? s.plan.vibInc0 + (int64_t)c * s.plan.vibIncStep : s.plan.vibIncFinal);
-}
+// the request laws of klatt_tick_core.cuh on tick (seg, c), with the values on the pop tick the segment carries
 KLATT_HD uint64_t pullVibBefore(const PullSeg &s, uint32_t c) {
-	if (c == 0) return 0;
-	uint64_t sum = (uint64_t)s.vibIncStale;
-	const uint64_t kmax = (c - 1 < s.F - 1) ? c - 1 : s.F - 1;  // fade ticks 1 .. kmax are behind us
-	sum += kmax * (uint64_t)s.plan.vibInc0 + (uint64_t)s.plan.vibIncStep * (kmax * (kmax + 1) / 2);
-	if (c > s.F) sum += (uint64_t)(c - s.F) * (uint64_t)s.plan.vibIncFinal;
-	return sum;
+	return vibBeforeLaw(c, s.F, s.vibIncStale, s.plan.vibInc0, s.plan.vibIncStep, s.plan.vibIncFinal);
 }
-
-// cur.voicePitch on tick (seg, c): stale on the pop tick, the fade (src/utils.h:20-23), the landing value on the landing
-// and the swap tick, then the hold glide: the reference adds voicePitchInc once per tick (src/frame.cpp:77), and a sum of
-// roundings is not a product -- glideExact (klatt_f32_core.cuh) reproduces the c - F - 1 additions bit for bit.  PullOsc
-// below walks a chunk tick by tick and only seeks this way; from one hold tick to the next it adds, as the reference does.
-KLATT_HD double pullPitchAt(const PullSeg &s, uint32_t c) {
-	if (c == 0) return s.pitchStale;
-	const double o = s.pitchOld, n = s.pitchNew;
-	if (c < s.F) return (n != n) ? o : o + ((n - o) * ((double)c / (double)s.F));
-	const double landing = (n != n) ? o : o + ((n - o) * 1.0);
-	if (c <= s.F + 1) return landing;
-	return glideExact(landing, s.pitchInc, (uint64_t)(c - s.F - 1));
-}
-
 KLATT_HD float pullDirAt(const PullSeg &s, int slot, uint32_t c) {
-	return c == 0 ? s.dirStale[slot] : (c < s.F ? fmaf((float)c, s.plan.dirStep[slot], s.plan.dir0[slot]) : s.plan.dirFinal[slot]);
-}
-
-// the vibrato depth 0.06 * vibratoPitchOffset on tick (seg, c), in double (klatt_common.h FadePlanF32)
-KLATT_HD double pullDepthAt(const PullSeg &s, uint32_t c) {
-	return c == 0 ? s.depthStale : (c < s.F ? fma((double)(float)c, s.plan.depthStep, s.plan.depth0) : s.plan.depthFinal);
-}
-
-KLATT_HD bool pullN0InvAt(const PullSeg &s, uint32_t c) {
-	if (c == 0) return s.n0InvStale != 0;
-	return (c < s.F ? s.plan.n0InvFade : s.plan.n0InvFinal) != 0;
+	return dirLaw(c, s.F, s.dirStale[slot], s.plan.dir0[slot], s.plan.dirStep[slot], s.plan.dirFinal[slot]);
 }
 
 // where a tick sits: segment, sampleCounter value on that tick, ticks of the segment still to come (this one included)
@@ -156,67 +128,31 @@ struct PullCursor {
 	}
 };
 
-// zeta = 1 - pole of one section along the pull (klatt_long.cu PoleWalk over segments)
-struct PullPole {
-	float zr, zi, wr, wi;
-	// zeta on fade tick k from the closed form of the pole.  The arguments are formed in double, the exponential and
-	// the sine / cosine in FP32 with the cancellation-free expressions of oneMinusExp(): zeta is kept in FP32 anyway, and
-	// 512 threads x 14 sections x (expm1 + sincos) in double was the largest fixed cost of a launch.
-	KLATT_HD void exact(const PullSeg &S, uint32_t k, int r, double srInv) {
-		const double PI = 3.14159265358979323846;
-		const double ratio = (double)((float)k / (float)S.F);
-		const double f0 = S.fb[r][0], f1 = S.fb[r][1], b0 = S.fb[r][2], b1 = S.fb[r][3];
-		const float x = (float)(-PI * (b0 + ((b1 - b0) * ratio)) * srInv);     // log of the pole radius
-		const float hth = (float)(PI * (f0 + ((f1 - f0) * ratio)) * srInv);    // half the pole angle
-		const float em1 = expm1f(x);
-		const float rad = 1.0f + em1;
-		float sh, ch;
-		sincosf(hth, &sh, &ch);
-		zr = fmaf((2.0f * rad) * sh, sh, -em1);
-		zi = -rad * ((2.0f * sh) * ch);
-	}
-	// state as it is AFTER the tick before (S, c)
-	KLATT_HD void seek(const PullSeg &S, uint32_t c, int r, double srInv) {
-		wr = wi = 0.0f;
-		if (c <= 1) {
-			zr = S.zStaleRe[r]; zi = S.zStaleIm[r];
-		} else if (c <= S.F) {  // ticks 1 .. c-1 of the fade are behind us
-			exact(S, c - 1, r, srInv);
-			wr = S.plan.wre[r]; wi = S.plan.wim[r];
-		} else {
-			zr = S.plan.zFre[r]; zi = S.plan.zFim[r];
-		}
-	}
-	// the update of tick (S, c): afterwards (zr, zi) is what the tick renders with
-	KLATT_HD void tick(const PullSeg &S, uint32_t c, int r, double srInv) {
-		if (c == 0) {  // pop tick: what was in force before
-			zr = S.zStaleRe[r]; zi = S.zStaleIm[r]; wr = wi = 0.0f;
-			return;
-		}
-		if (c > S.F) return;  // after the landing: constant
-		if (c == S.F) {
-			zr = S.plan.zFre[r]; zi = S.plan.zFim[r]; wr = wi = 0.0f;
-			return;
-		}
-		if (c == 1) {
-			zr = S.plan.z0re[r]; zi = S.plan.z0im[r]; wr = S.plan.wre[r]; wi = S.plan.wim[r];
-		}
-		if ((c & (uint32_t)(kCoarseTicks - 1)) == 0) {
-			exact(S, c, r, srInv);  // drift control: back onto the closed form
-			return;
-		}
-		float tr = fmaf(-zr, wr, wr);
-		tr = fmaf(zi, wi, tr);
-		float ti = fmaf(-zr, wi, wi);
-		ti = fmaf(-zi, wr, ti);
-		zr += tr;
-		zi += ti;
-	}
-	KLATT_HD void coef(float &a, float &rho) const {
-		a = fmaf(zr, zr, zi * zi);
-		rho = fmaf(2.0f, zr, -a);
-	}
-};
+// zeta of section r on fade tick k from the closed form of the pole (PoleWalk's `exact`).  The arguments are formed in
+// double, the exponential and the sine / cosine in FP32 with the cancellation-free expressions of oneMinusExp(): zeta is kept
+// in FP32 anyway, and 512 threads x 14 sections x (expm1 + sincos) in double was the largest fixed cost of a launch.
+KLATT_HD void pullPoleExact(const PullSeg &S, uint32_t k, int r, double srInv, float &zr, float &zi) {
+	const double PI = 3.14159265358979323846;
+	const double ratio = (double)((float)k / (float)S.F);
+	const double f0 = S.fb[r][0], f1 = S.fb[r][1], b0 = S.fb[r][2], b1 = S.fb[r][3];
+	const float x = (float)(-PI * (b0 + ((b1 - b0) * ratio)) * srInv);     // log of the pole radius
+	const float hth = (float)(PI * (f0 + ((f1 - f0) * ratio)) * srInv);    // half the pole angle
+	const float em1 = expm1f(x);
+	const float rad = 1.0f + em1;
+	float sh, ch;
+	sincosf(hth, &sh, &ch);
+	zr = fmaf((2.0f * rad) * sh, sh, -em1);
+	zi = -rad * ((2.0f * sh) * ch);
+}
+
+// PoleWalk of section r along the pull: the pop tick of a segment sets what was in force before it
+KLATT_HD void pullPoleSeek(PoleWalk &w, const PullSeg &S, uint32_t c, int r, double srInv) {
+	w.seek(S.plan, c, S.F, r, S.zStaleRe[r], S.zStaleIm[r], [&](uint32_t k, float &zr, float &zi) { pullPoleExact(S, k, r, srInv, zr, zi); });
+}
+KLATT_HD void pullPoleTick(PoleWalk &w, const PullSeg &S, uint32_t c, int r, double srInv) {
+	if (c == 0) w = PoleWalk{S.zStaleRe[r], S.zStaleIm[r], 0.0f, 0.0f};
+	else w.tick(S.plan, c, S.F, r, [&](uint32_t k, float &zr, float &zi) { pullPoleExact(S, k, r, srInv, zr, zi); });
+}
 
 KLATT_HD uint32_t pullIdx(const PullCtx &X, uint32_t t) { return (t % X.L) * (uint32_t)kPullThreads + t / X.L; }
 
@@ -233,7 +169,6 @@ KLATT_HD void pullNoiseWords(const PullCtx &X, uint64_t g, Philox4 &blk, uint64_
 		wF = (d0 + 1 < X.drawLen) ? ((uint32_t)X.draws[d0 + 1] << 1) : 0u;
 	}
 }
-KLATT_HD float pullDraw(uint32_t w) { return bitsToFloat(0x4B000000u | (w >> 9)) - 8388608.0f; }
 
 // ---------------------------------------------------------------------------------------------------------------
 // source (reference src/speechWaveGenerator.cpp:32-88, :204-206)
@@ -256,7 +191,7 @@ struct PullSourceSums {
 struct PullOsc {  // vibrato + pitch along the pull
 	PullCursor cur;
 	uint64_t vibPos;
-	double glide;                     // voicePitch on hold tick (glideSeg, glideC)
+	double glide;                     // voicePitch on tick (glideSeg, glideC), the last one pitch() rendered
 	uint32_t glideSeg, glideC;
 	KLATT_HD void seek(const PullCtx &X, uint32_t t) {
 		cur.seek(X, t);
@@ -264,24 +199,19 @@ struct PullOsc {  // vibrato + pitch along the pull
 		vibPos = S.vibPosAtPop + pullVibBefore(S, cur.c);
 		glide = 0.0; glideSeg = 0xffffffffu; glideC = 0;
 	}
-	// cur.voicePitch on the current tick: pullPitchAt, with the hold glide carried from tick to tick by the reference's own
-	// addition (src/frame.cpp:77)
+	// cur.voicePitch on the current tick (pitchTick)
 	KLATT_HD double pitch(const PullSeg &S) {
-		const uint32_t c = cur.c;
-		if (c <= S.F + 1u) return pullPitchAt(S, c);
-		if (glideSeg == cur.s && glideC + 1u == c) glide = glide + S.pitchInc;
-		else glide = pullPitchAt(S, c);
-		glideSeg = cur.s; glideC = c;
-		return glide;
+		const double p = pitchTick(glide, glideSeg == cur.s && glideC + 1u == cur.c, cur.c, S.F, S.pitchStale, S.pitchOld, S.pitchNew,
+		                           S.pitchInc);
+		glideSeg = cur.s; glideC = cur.c;
+		return p;
 	}
-	// what this tick adds to the glottal phase, in cycles: (pitch * vibrato) / sampleRate as the reference rounds it
-	// (src/speechWaveGenerator.cpp:72-74, :55)
+	// what this tick adds to the glottal phase, in cycles
 	KLATT_HD double phaseInc(const PullCtx &X, double srD, double srInv) {
 		const PullSeg &S = X.segs[cur.s];
-		vibPos += (uint64_t)pullVibInc(S, cur.c);
-		float vph = (float)(int32_t)(uint32_t)(vibPos >> 32) * 2.3283064365386963e-10f;
-		double m = pitch(S) * fma((double)sinTurns(vph), pullDepthAt(S, cur.c), 1.0);
-		return divideBySampleRate(m, srD, srInv);
+		const uint32_t c = cur.c;
+		return glottalInc(vibPos, vibIncLaw(c, S.F, S.vibIncStale, S.plan.vibInc0, S.plan.vibIncStep, S.plan.vibIncFinal), pitch(S),
+		                  depthLaw(c, S.F, S.depthStale, S.plan.depth0, S.plan.depthStep, S.plan.depthFinal), srD, srInv);
 	}
 	KLATT_HD void next(const PullCtx &X) {
 		const uint32_t was = cur.s;
@@ -313,8 +243,8 @@ KLATT_HD void pullSourcePass1(const PullCtx &X, uint32_t ch, PullSourceSums &out
 	for (uint32_t t = t0; t < t1; ++t, at += kPullThreads) {
 		uint32_t wA, wF;
 		pullNoiseWords(X, g0 + t, blk, blkIndex, wA, wF);
-		out.zAsp = fmaf(0.75f, out.zAsp, pullDraw(wA));
-		out.zFric = fmaf(0.75f, out.zFric, pullDraw(wF));
+		out.zAsp = colourNoise(out.zAsp, wA);
+		out.zFric = colourNoise(out.zFric, wF);
 		out.decay *= 0.75f;
 		const double pinc = w.phaseInc(X, srD, srInv);
 		X.inc[at] = pinc;
@@ -588,17 +518,9 @@ KLATT_HD void pullSourcePass2(const PullCtx &X, uint32_t ch, float aspStart, flo
 		pullNoiseWords(X, g0 + t, blk, blkIndex, wA, wF);
 		const PullSeg &S = X.segs[cur.s];
 		const uint32_t c = cur.c;
-		const float voice = (float)X.inc[at];
-		aspLast = fmaf(0.75f, aspLast, pullDraw(wA));
-		float asp = aspLast * (0.2f * kDrawScale);
-		float turb = asp * pullDirAt(S, dVoiceTurbulenceAmplitude, c);
-		if (voice < pullDirAt(S, dGlottalOpenQuotient, c)) turb *= 0.01f;
-		float v = (fmaf(voice, 2.0f, -1.0f) + turb) * pullDirAt(S, dVoiceAmplitude, c);
-		float src = fmaf(asp, pullDirAt(S, dAspirationAmplitude, c), v);
-		const float halfGain = pullDirAt(S, dPreFormantGain, c) * 0.5f;
-		X.sigA[at] = src * halfGain;
-		fricLast = fmaf(0.75f, fricLast, pullDraw(wF));
-		X.sigB[at] = fricLast * (((0.3f * kDrawScale) * pullDirAt(S, dFricationAmplitude, c)) * halfGain);
+		excitation((float)X.inc[at], wA, wF, pullDirAt(S, dVoiceTurbulenceAmplitude, c), pullDirAt(S, dGlottalOpenQuotient, c),
+		           pullDirAt(S, dVoiceAmplitude, c), pullDirAt(S, dAspirationAmplitude, c), pullDirAt(S, dFricationAmplitude, c),
+		           pullDirAt(S, dPreFormantGain, c), aspLast, fricLast, X.sigA[at], X.sigB[at]);
 		cur.next(X);
 	}
 	if (t1 == X.n) {  // the pull's last chunk leaves the carry
@@ -608,13 +530,8 @@ KLATT_HD void pullSourcePass2(const PullCtx &X, uint32_t ch, float aspStart, flo
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// resonator stages (reference src/speechWaveGenerator.cpp:112-182, :207-208)
+// resonator stages (klatt_tick_core.cuh StageTick): the parallel stage reads and rewrites sigB, the others sigA
 // ---------------------------------------------------------------------------------------------------------------
-enum PullStage : int { kPullParallel = 0, kPullNasal = 1, kPullCascade = 2, kPullLast = 3 };
-template <int STAGE> struct PullStageTraits {
-	static constexpr int NR = STAGE == kPullParallel ? 6 : 1;  // scanned sections
-};
-
 // input of the FIR section before tick t of the pull (t may reach 2 ticks into the previous pull)
 KLATT_HD float pullFirInput(const PullCtx &X, int64_t t) {
 	if (t >= 0) return X.sigA[pullIdx(X, (uint32_t)t)];
@@ -624,37 +541,31 @@ KLATT_HD float pullFirInput(const PullCtx &X, int64_t t) {
 
 // One chunk of one stage.  PASS 1: from zero state, accumulate the affine map.  PASS 2: from the scanned start state,
 // overwrite the stage's input signal with its output (or, for the last stage, store the int16 samples).
-//   kPullParallel: sigB = frication input -> sections 8..13 -> parallel output (:170-180)
-//   kPullNasal   : sigA = cascade input -> rN0 (FIR) -> rNP (section 1) -> caNP mix (:148-150)
-//   kPullCascade : sigA -> section `res` (:151-155)
-//   kPullLast    : like kPullCascade for r1, then (x + par) * outputGain * 4000, clamp, truncate (:207-208)
 // fir[2]: the two inputs before the chunk, read in pass 1 (before any thread overwrites sigA) and handed to pass 2.
 // poles[NR + 1]: zeta of the sections at the start of the chunk (and of rN0 in the last slot), found in pass 1 -- inside
 // a fade that is an exponential and a sine / cosine per section -- and handed to pass 2.
 template <int STAGE, int PASS>
-KLATT_HD void pullStage(const PullCtx &X, uint32_t ch, int res, PullAffine *maps, const PullStart *start, float *fir,
-                        PullPole *poles) {
-	constexpr int NR = PullStageTraits<STAGE>::NR;
+KLATT_HD void pullStage(const PullCtx &X, uint32_t ch, int res, Affine *maps, const PullStart *start, float *fir,
+                        PoleWalk *poles) {
+	constexpr int NR = StageTraits<STAGE>::NR;
 	uint32_t t0, t1;
 	pullChunkRange(X, ch, t0, t1);
 	if (PASS == 1) {
 #pragma unroll
-		for (int k = 0; k < NR; ++k) {
-			maps[k].p00 = 1.0f; maps[k].p01 = 0.0f; maps[k].p10 = 0.0f; maps[k].p11 = 1.0f; maps[k].zy = 0.0f; maps[k].zd = 0.0f;
-		}
+		for (int k = 0; k < NR; ++k) maps[k] = Affine{1.0f, 0.0f, 0.0f, 1.0f, 0.0f, 0.0f};
 	}
 	if (t0 >= t1) return;
 	const double srInv = 1.0 / (double)X.sampleRate;
-	float *sig = STAGE == kPullParallel ? X.sigB : X.sigA;
+	float *sig = STAGE == kStageParallel ? X.sigB : X.sigA;
 	PullCursor cur;
 	cur.seek(X, t0);
-	PullPole pw[NR], pw0;  // pw0: the FIR anti-resonator of the nasal stage
+	PoleWalk pw[NR], pw0;  // pw0: the FIR anti-resonator of the nasal stage
 	if (PASS == 1) {
 		const PullSeg &S = X.segs[cur.s];
 #pragma unroll
-		for (int k = 0; k < NR; ++k) pw[k].seek(S, cur.c, STAGE == kPullParallel ? kResParallel + k : res, srInv);
-		if (STAGE == kPullNasal) pw0.seek(S, cur.c, kResN0, srInv);
-		else { pw0.zr = pw0.zi = pw0.wr = pw0.wi = 0.0f; }
+		for (int k = 0; k < NR; ++k) pullPoleSeek(pw[k], S, cur.c, STAGE == kStageParallel ? kResParallel + k : res, srInv);
+		if (STAGE == kStageNasal) pullPoleSeek(pw0, S, cur.c, kResN0, srInv);
+		else pw0 = PoleWalk{0.0f, 0.0f, 0.0f, 0.0f};
 #pragma unroll
 		for (int k = 0; k < NR; ++k) poles[k] = pw[k];
 		poles[NR] = pw0;
@@ -663,108 +574,66 @@ KLATT_HD void pullStage(const PullCtx &X, uint32_t ch, int res, PullAffine *maps
 		for (int k = 0; k < NR; ++k) pw[k] = poles[k];
 		pw0 = poles[NR];
 	}
-	float y[NR], d[NR];
-	float p00[NR], p01[NR], p10[NR], p11[NR];
+	StageTick<STAGE, PASS> st;
+	st.start();
+	if (PASS == 2) {
 #pragma unroll
-	for (int k = 0; k < NR; ++k) {
-		if (PASS == 2) { y[k] = start[k].y; d[k] = start[k].d; }
-		else { y[k] = 0.0f; d[k] = 0.0f; }
-		p00[k] = 1.0f; p01[k] = 0.0f; p10[k] = 0.0f; p11[k] = 1.0f;
+		for (int k = 0; k < NR; ++k) { st.y[k] = start[k].y; st.d[k] = start[k].d; }
 	}
-	float in1 = 0.0f, in2 = 0.0f;
-	if (STAGE == kPullNasal) {
+	if (STAGE == kStageNasal) {
 		if (PASS == 1) {
 			fir[0] = pullFirInput(X, (int64_t)t0 - 1);
 			fir[1] = pullFirInput(X, (int64_t)t0 - 2);
 		}
-		in1 = fir[0]; in2 = fir[1];
+		st.in1 = fir[0]; st.in2 = fir[1];
 	}
 	// What a tick reads besides its input and the section memories: coefficients and mixing gains, functions of
 	// (segment, counter).  Behind the landing tick of a request they are constants, so a chunk that lies inside one hold
 	// (most chunks do: a fade is a third of the ticks and 512 consecutive ticks share a warp) evaluates them once.
-	float ca[NR], crho[NR], cmix[NR], cextra = 0.0f, ca0 = 0.0f, crho0 = 0.0f, crcp0 = 0.0f;
-	bool cinv = false;
+	StageCoefs<STAGE> co;
+	co.extra = co.a0 = co.rho0 = co.rcp0 = 0.0f;
+	co.inv = false;
 	auto loadCoefs = [&](const PullSeg &S, uint32_t c) {
-		if (STAGE == kPullNasal) {
-			pw0.tick(S, c, kResN0, srInv);
-			pw0.coef(ca0, crho0);
-			cinv = pullN0InvAt(S, c);
-			crcp0 = cinv ? fastRcp(ca0) : 0.0f;
-			cextra = pullDirAt(S, dCaNP, c);
+		if (STAGE == kStageNasal) {
+			pullPoleTick(pw0, S, c, kResN0, srInv);
+			pw0.coef(co.a0, co.rho0);
+			co.inv = n0InvLaw(c, S.F, S.n0InvStale, S.plan.n0InvFade, S.plan.n0InvFinal);
+			co.rcp0 = co.inv ? fastRcp(co.a0) : 0.0f;
+			co.extra = pullDirAt(S, dCaNP, c);
 		}
 #pragma unroll
 		for (int k = 0; k < NR; ++k) {
-			pw[k].tick(S, c, STAGE == kPullParallel ? kResParallel + k : res, srInv);
-			pw[k].coef(ca[k], crho[k]);
-			cmix[k] = STAGE == kPullParallel ? pullDirAt(S, dPa1 + k, c) : 0.0f;
+			pullPoleTick(pw[k], S, c, STAGE == kStageParallel ? kResParallel + k : res, srInv);
+			pw[k].coef(co.a[k], co.rho[k]);
+			co.mix[k] = STAGE == kStageParallel ? pullDirAt(S, dPa1 + k, c) : 0.0f;
 		}
-		if (STAGE == kPullParallel) cextra = pullDirAt(S, dParallelBypass, c);
-		if (STAGE == kPullLast) cextra = pullDirAt(S, dOutputGain, c) * 4000.0f;
+		if (STAGE == kStageParallel) co.extra = pullDirAt(S, dParallelBypass, c);
+		if (STAGE == kStageLast) co.extra = pullDirAt(S, dOutputGain, c);
 	};
 	const bool hold = cur.c > X.segs[cur.s].F && cur.left >= t1 - t0;
-	if (hold) loadCoefs(X.segs[cur.s], cur.c);
 	uint32_t at = ch;
 	for (uint32_t t = t0; t < t1; ++t, at += kPullThreads) {
-		if (!hold) loadCoefs(X.segs[cur.s], cur.c);
-		float x = sig[at];
-		const float xin = x;
-		if (STAGE == kPullNasal) {  // rN0 on inputs: src/speechWaveGenerator.cpp:129-135 with anti == true
-			const float dprev = in1 - in2;
-			const float dx = x - in1;
-			const float dx1 = fmaf(-crho0, dprev, dprev);
-			x = cinv ? fmaf(dx - dx1, crcp0, in1) : fmaf(ca0, dx, dx1 + in1);
-			in2 = in1;
-			in1 = xin;
-		}
-		float acc = 0.0f;
-#pragma unroll
-		for (int k = 0; k < NR; ++k) {
-			const float a = ca[k], rho = crho[k];
-			float w = fmaf(-rho, d[k], d[k]);
-			w = fmaf(-a, y[k], w);
-			const float dn = fmaf(a, x, w);
-			d[k] = dn;
-			y[k] += dn;
-			if (PASS == 1) {  // P <- A P with A = [[1-a, 1-rho], [-a, 1-rho]] acting on (y, d)
-				const float g = 1.0f - rho;
-				const float n10 = fmaf(-a, p00[k], g * p10[k]), n11 = fmaf(-a, p01[k], g * p11[k]);
-				p00[k] += n10; p01[k] += n11;
-				p10[k] = n10; p11[k] = n11;
-			}
-			if (STAGE == kPullParallel) acc = fmaf(y[k] - x, cmix[k], acc);
-		}
+		if (!hold || t == t0) loadCoefs(X.segs[cur.s], cur.c);
+		const float o = st(sig[at], STAGE == kStageLast && PASS == 2 ? X.sigB[at] : 0.0f, co);
 		if (PASS == 2) {
-			if (STAGE == kPullParallel) {
-				sig[at] = fmaf(x - acc, cextra, acc);
-			} else if (STAGE == kPullNasal) {
-				sig[at] = fmaf(y[0] - xin, cextra, xin);
-			} else if (STAGE == kPullCascade) {
-				sig[at] = y[0];
-			} else {
-				float s = (y[0] + X.sigB[at]) * cextra;
-				s = fminf(s, 32000.0f);
-				s = fmaxf(s, -32000.0f);
-				X.pcm[t] = (int16_t)(int)s;
-			}
+			if (STAGE == kStageLast) X.pcm[t] = (int16_t)(int)o;
+			else sig[at] = o;
 		}
 		if (!hold) cur.next(X);
 	}
 	if (PASS == 1) {
 #pragma unroll
-		for (int k = 0; k < NR; ++k) {
-			maps[k].p00 = p00[k]; maps[k].p01 = p01[k]; maps[k].p10 = p10[k]; maps[k].p11 = p11[k];
-			maps[k].zy = y[k]; maps[k].zd = d[k];
-		}
+		for (int k = 0; k < NR; ++k) maps[k] = st.map(k);
 	} else if (t1 == X.n) {  // the pull's last chunk leaves the carry
 #pragma unroll
 		for (int k = 0; k < NR; ++k) {
-			const int r = STAGE == kPullParallel ? kResParallel + k : res;
-			X.state->y[r] = y[k];
-			X.state->d[r] = d[k];
+			const int r = STAGE == kStageParallel ? kResParallel + k : res;
+			X.state->y[r] = st.y[k];
+			X.state->d[r] = st.d[k];
 		}
-		if (STAGE == kPullNasal) {
-			X.state->y[kResN0] = in1;
-			X.state->d[kResN0] = in1 - in2;
+		if (STAGE == kStageNasal) {
+			X.state->y[kResN0] = st.in1;
+			X.state->d[kResN0] = st.in1 - st.in2;
 		}
 	}
 }
@@ -784,7 +653,7 @@ struct PullAffineD {
 	PullScalar p00, p01, p10, p11, zy, zd;
 };
 KLATT_HD PullAffineD pullIdentity() { return PullAffineD{1, 0, 0, 1, 0, 0}; }
-KLATT_HD PullAffineD pullToD(const PullAffine &m) { return PullAffineD{m.p00, m.p01, m.p10, m.p11, m.zy, m.zd}; }
+KLATT_HD PullAffineD pullToD(const Affine &m) { return PullAffineD{m.p00, m.p01, m.p10, m.p11, m.zy, m.zd}; }
 KLATT_HD PullAffineD pullSeed(float y, float d) { return PullAffineD{1, 0, 0, 1, y, d}; }
 // `second` after `first`
 KLATT_HD PullAffineD pullCompose(const PullAffineD &second, const PullAffineD &first) {

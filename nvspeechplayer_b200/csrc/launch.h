@@ -92,11 +92,6 @@ struct LongTable {
 	LongStream one;              // streams[0] by value: a one-stream launch reads its stream from the parameter bank
 };
 
-// affine map of one section over one chunk, (y, d)_end = P (y, d)_start + z, row-major P
-struct Affine {
-	float p00, p01, p10, p11, zy, zd;
-};
-
 // Launchers: everything device-resident, scratch sized by the caller (api_long.cu).
 // ticks[s] = the ticks stream s's whole queue yields (the occupancy law of timelineTicks, host.h); offsets [numStreams + 1]
 // as validated by the host
