@@ -113,12 +113,17 @@ int speechPlayer_queueFrames(speechPlayer_handle_t playerHandle, const speechPla
 /* Render numHandles independent players at once (one launch).  sampleBuf is HOST memory,
  * [numHandles][sampleCount] row-major; samplesWritten[i] (may be NULL) receives what
  * speechPlayer_synthesize would have returned for handles[i].  All handles must share precision and
- * sample rate.  Returns the total number of samples written, or -1 on error. */
+ * sample rate.  Returns the total number of samples written, or -1 on error.
+ * With SPEECHPLAYER_NOISE_GLIBC the handles are not rendered in parallel: they render one after another, in
+ * handle order, so each row and the process-global generator end up exactly as the same speechPlayer_synthesize
+ * calls made one by one would leave them (the reference's shared rand() is sequential by nature). */
 long long speechPlayer_synthesizeBatch(speechPlayer_handle_t *handles, unsigned int numHandles,
                                        unsigned int sampleCount, sample *sampleBuf, unsigned int *samplesWritten);
 
 /* SPEECHPLAYER_NOISE_REPLAY: the draw sequence (values 0..2^31-1, aspiration then frication per generated
- * sample) this handle consumes from now on; copied to the device. */
+ * sample) of this handle, indexed from its first sample: the g-th sample the handle generates since it was
+ * created reads draws[2g] and draws[2g+1], also when the sequence is set after the handle has rendered.  Draws
+ * past numDraws are 0.  Copied to the device. */
 int speechPlayer_setNoiseReplay(speechPlayer_handle_t playerHandle, const int32_t *draws, size_t numDraws);
 
 /* SPEECHPLAYER_NOISE_GLIBC: reseed the process-global generator (what srand() is to the reference). */

@@ -110,6 +110,8 @@ int speechPlayer_batchGetLaunchStats(speechPlayer_batch_t *batch, unsigned long 
  *   SetFramesHost: same arguments as speechPlayer_batchSetFramesHost; (re)partitions the streams and uploads every shard's
  *                 queues from its own thread
  *   GetShards   : firstStream[numDevices + 1] -- shard d owns streams [firstStream[d], firstStream[d + 1])
+ *   Create refuses what speechPlayer_batchCreate refuses (STREAM precision, GLIBC noise), and REPLAY noise too: a
+ *                 multi-batch has no entry that takes replay draws.  precision is FP64 or FP32, noiseMode PHILOX.
  * Everything a single batch guarantees holds per stream (same kernels, same bits as one batch on one GPU). */
 typedef struct speechPlayer_multiBatch speechPlayer_multiBatch_t;
 speechPlayer_multiBatch_t *speechPlayer_multiBatchCreate(int sampleRate, unsigned int numStreams, int precision, int noiseMode,

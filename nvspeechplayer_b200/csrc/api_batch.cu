@@ -450,6 +450,13 @@ speechPlayer_multiBatch_t *speechPlayer_multiBatchCreate(int sampleRate, unsigne
                                                          unsigned int numDevices) {
 	g_lastError.clear();
 	if (sampleRate <= 0 || numStreams == 0 || numDevices == 0 || !devices) { fail("bad sampleRate / numStreams / devices"); return nullptr; }
+	// the shards are made at the first SetFrames: refuse here what speechPlayer_batchCreate would refuse there, and REPLAY, for
+	// which a multi-batch has no entry that takes the draws
+	if (precision != kPrecisionF64 && precision != kPrecisionF32) {
+		fail(precision == kPrecisionStream ? "SPEECHPLAYER_PRECISION_STREAM is a per-handle mode (speechPlayer_initializeEx)" : "unknown precision");
+		return nullptr;
+	}
+	if (noiseMode != kNoisePhilox) { fail("multi-batch noise mode must be PHILOX"); return nullptr; }
 	int have = 0;
 	if (cudaGetDeviceCount(&have) != cudaSuccess || have <= 0) { fail("no usable CUDA device (this library has no CPU fallback)"); return nullptr; }
 	for (unsigned d = 0; d < numDevices; ++d)

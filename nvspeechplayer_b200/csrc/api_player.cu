@@ -389,8 +389,8 @@ static long long synthesizePull(Player *p, unsigned int sampleCount, int16_t *ou
 
 // speechPlayer_synthesizeBatch over SPEECHPLAYER_PRECISION_STREAM handles: ONE launch per kPullMaxTicks for all players, one
 // block per player (klatt_pull_batch_kernel) -- 148 interactive players at the latency of one.  Each row is what the player's
-// own speechPlayer_synthesize would have produced (same kernel body, same carried state).  With the process-global glibc noise
-// the players draw in handle order, as sequential calls would.
+// own speechPlayer_synthesize would have produced (same kernel body, same carried state).  Players with the process-global
+// glibc noise never come here: speechPlayer_synthesizeBatch renders them one after another.
 static std::mutex g_pullBatchMu;
 static PullBatchItem *g_pullItemsHost = nullptr, *g_pullItemsDev = nullptr;
 static size_t g_pullItemsCap = 0;
@@ -416,10 +416,10 @@ static long long synthesizePullBatch(std::vector<Player *> &ps, unsigned int sam
 	std::vector<uint32_t> got(n, 0);
 	std::vector<char> done(n, 0), zero(n, 1);
 	// The per-player host work runs on the helper threads when it touches no shared state and makes no CUDA call: zero-copy
-	// staging, no process-global rand() sequence (its draws are handed out in player order), no replay upload pending.
+	// staging, no replay upload pending.
 	bool parallel = pullZeroCopy() && !pullDebugPhases() && n >= 8 && HostPool::get().helpers() > 0;
 	for (size_t i = 0; i < n && parallel; ++i)
-		if (ps[i]->noiseMode == kNoiseGlibc || (ps[i]->noiseMode == kNoiseReplay && ps[i]->replayDirty)) parallel = false;
+		if (ps[i]->noiseMode == kNoiseReplay && ps[i]->replayDirty) parallel = false;
 	const size_t grain = parallel ? std::max<size_t>(1, n / (4 * (HostPool::get().helpers() + 1))) : n;
 	auto forEach = [&](const std::function<void(size_t)> &fn) {
 		if (parallel) HostPool::get().parallelFor(n, grain, fn);
@@ -485,37 +485,10 @@ static long long synthesizePullBatch(std::vector<Player *> &ps, unsigned int sam
 	return sum;
 }
 
-long long speechPlayer_synthesizeBatch(speechPlayer_handle_t *handles, unsigned int numHandles, unsigned int sampleCount,
-                                       sample *sampleBuf, unsigned int *samplesWritten) {
-	g_lastError.clear();
-	if (numHandles == 0 || sampleCount == 0) return 0;
-	if (!handles || !sampleBuf) return fail("null argument");
-	std::vector<Player *> ps(numHandles);
-	bool anyPull = false;
-	for (unsigned i = 0; i < numHandles; ++i) {
-		ps[i] = lookup(handles[i]);
-		if (!ps[i]) return fail("bad handle in batch");
-		anyPull = anyPull || ps[i]->pull != nullptr;
-	}
-	if (!anyPull)
-		for (unsigned i = 0; i < numHandles; ++i) {
-			if (ps[i]->precision != ps[0]->precision || ps[i]->sampleRate != ps[0]->sampleRate ||
-			    ps[i]->device != ps[0]->device || ps[i]->noiseMode != ps[0]->noiseMode || ps[i]->seed != ps[0]->seed)
-				return fail("handles of one batch must share device, sample rate, precision and noise mode");
-		}
-	PlayerLocks locks;
-	if (!locks.lock(ps)) return fail("duplicate handle in batch");
-	if (anyPull) {  // low-latency players: one block per player, one launch for all of them
-		for (unsigned i = 0; i < numHandles; ++i)
-			if (!ps[i]->pull || ps[i]->device != ps[0]->device)
-				return fail("handles of one batch must share device and precision");
-		if (numHandles == 1) {
-			long long w = synthesizePull(ps[0], sampleCount, reinterpret_cast<int16_t *>(sampleBuf));
-			if (w >= 0 && samplesWritten) samplesWritten[0] = (unsigned int)w;
-			return w;
-		}
-		return synthesizePullBatch(ps, sampleCount, reinterpret_cast<int16_t *>(sampleBuf), samplesWritten);
-	}
+// One launch for the FP64 / FP32 handles ps[0..n) (the caller holds their locks and has checked that they share device, sample
+// rate, precision, noise mode and seed).
+static long long synthesizeHandles(Player *const *ps, unsigned int n, unsigned int sampleCount, sample *sampleBuf,
+                                   unsigned int *samplesWritten) {
 	Player *lead = ps[0];
 	DeviceGuard g(lead->device);
 	if (!lead->pipe.init()) return -1;
@@ -526,32 +499,82 @@ long long speechPlayer_synthesizeBatch(speechPlayer_handle_t *handles, unsigned 
 		noiseLock.lock();
 		checkpoint = g_noise;
 	}
-	std::vector<StreamDesc> descs(numHandles);
-	for (unsigned i = 0; i < numHandles; ++i)
+	std::vector<StreamDesc> descs(n);
+	for (unsigned i = 0; i < n; ++i)
 		if (ps[i]->prepare(descs[i], sampleCount, stream) != 0) return -1;
-	if (!lead->dDesc.reserve(sizeof(StreamDesc) * (size_t)numHandles)) return -1;
-	CU(cudaMemcpyAsync(lead->dDesc.p, descs.data(), sizeof(StreamDesc) * (size_t)numHandles, cudaMemcpyHostToDevice, stream));
+	if (!lead->dDesc.reserve(sizeof(StreamDesc) * (size_t)n)) return -1;
+	CU(cudaMemcpyAsync(lead->dDesc.p, descs.data(), sizeof(StreamDesc) * (size_t)n, cudaMemcpyHostToDevice, stream));
 	CU(cudaStreamSynchronize(stream));
-	std::vector<uint32_t> written(numHandles);
-	std::vector<StreamResult> results(numHandles);
+	std::vector<uint32_t> written(n);
+	std::vector<StreamResult> results(n);
 	NoiseConfig nc{lead->noiseMode, lead->seed};
 	// The reference's generate() returns the count and leaves sampleBuf[count..] untouched (src/speechWaveGenerator.cpp:210),
 	// so the rows land in a scratch buffer first and only the written prefix of each row is handed to the caller.
 	std::vector<int16_t> &scratch = lead->hostScratch;
-	scratch.resize((size_t)numHandles * sampleCount);
-	long long total = renderToHost(lead->pipe, lead->precision, lead->dDesc.as<StreamDesc>(), numHandles, lead->sampleRate,
+	scratch.resize((size_t)n * sampleCount);
+	long long total = renderToHost(lead->pipe, lead->precision, lead->dDesc.as<StreamDesc>(), n, lead->sampleRate,
 	                               sampleCount, scratch.data(), written.data(), results.data(), nc, nullptr);
 	if (total < 0) return -1;
-	for (unsigned i = 0; i < numHandles; ++i) {
+	for (unsigned i = 0; i < n; ++i) {
 		ps[i]->absorb(results[i], written[i]);
 		if (samplesWritten) samplesWritten[i] = written[i];
 		memcpy(reinterpret_cast<int16_t *>(sampleBuf) + (size_t)i * sampleCount, scratch.data() + (size_t)i * sampleCount,
 		       sizeof(int16_t) * (size_t)written[i]);
 	}
-	if (lead->noiseMode == kNoiseGlibc && numHandles == 1) {
-		// the reference consumes exactly two rand() calls per generated sample: rewind to that point
+	if (lead->noiseMode == kNoiseGlibc) {
+		// the reference consumes exactly two rand() calls per generated sample: rewind to that point (one handle only, see
+		// speechPlayer_synthesizeBatch)
 		g_noise = checkpoint;
 		g_noise.skip((uint64_t)written[0] * 2);
+	}
+	return total;
+}
+
+long long speechPlayer_synthesizeBatch(speechPlayer_handle_t *handles, unsigned int numHandles, unsigned int sampleCount,
+                                       sample *sampleBuf, unsigned int *samplesWritten) {
+	g_lastError.clear();
+	if (numHandles == 0 || sampleCount == 0) return 0;
+	if (!handles || !sampleBuf) return fail("null argument");
+	std::vector<Player *> ps(numHandles);
+	bool anyPull = false, anyGlibc = false;
+	for (unsigned i = 0; i < numHandles; ++i) {
+		ps[i] = lookup(handles[i]);
+		if (!ps[i]) return fail("bad handle in batch");
+		anyPull = anyPull || ps[i]->pull != nullptr;
+		anyGlibc = anyGlibc || ps[i]->noiseMode == kNoiseGlibc;
+	}
+	if (!anyPull)
+		for (unsigned i = 0; i < numHandles; ++i) {
+			if (ps[i]->precision != ps[0]->precision || ps[i]->sampleRate != ps[0]->sampleRate ||
+			    ps[i]->device != ps[0]->device || ps[i]->noiseMode != ps[0]->noiseMode || ps[i]->seed != ps[0]->seed)
+				return fail("handles of one batch must share device, sample rate, precision and noise mode");
+		}
+	PlayerLocks locks;
+	if (!locks.lock(ps)) return fail("duplicate handle in batch");
+	// The process-global glibc sequence is handed out in call order: a player takes two draws per sample it generates, and
+	// how many it generates is known only once it has rendered.  So with glibc noise the handles render one after another, in
+	// handle order, each exactly as its own speechPlayer_synthesize would.
+	const bool oneByOne = anyGlibc && numHandles > 1;
+	if (anyPull) {  // low-latency players: one block per player, one launch for all of them
+		for (unsigned i = 0; i < numHandles; ++i)
+			if (!ps[i]->pull || ps[i]->device != ps[0]->device)
+				return fail("handles of one batch must share device and precision");
+		if (numHandles > 1 && !oneByOne) return synthesizePullBatch(ps, sampleCount, reinterpret_cast<int16_t *>(sampleBuf), samplesWritten);
+		long long total = 0;
+		for (unsigned i = 0; i < numHandles; ++i) {
+			long long w = synthesizePull(ps[i], sampleCount, reinterpret_cast<int16_t *>(sampleBuf) + (size_t)i * sampleCount);
+			if (w < 0) return -1;
+			if (samplesWritten) samplesWritten[i] = (unsigned int)w;
+			total += w;
+		}
+		return total;
+	}
+	if (!oneByOne) return synthesizeHandles(ps.data(), numHandles, sampleCount, sampleBuf, samplesWritten);
+	long long total = 0;
+	for (unsigned i = 0; i < numHandles; ++i) {
+		long long w = synthesizeHandles(&ps[i], 1, sampleCount, sampleBuf + (size_t)i * sampleCount, samplesWritten ? samplesWritten + i : nullptr);
+		if (w < 0) return -1;
+		total += w;
 	}
 	return total;
 }

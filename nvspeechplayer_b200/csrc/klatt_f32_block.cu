@@ -53,12 +53,12 @@ struct BlockCtl {
 
 namespace {
 
-__device__ __forceinline__ uint32_t classifyLite(const StreamStateLite &st, uint32_t sampleCount, uint32_t holdTicks) {
+__device__ __forceinline__ uint32_t classifyLite(const StreamStateLite &st, uint32_t sampleCount, uint32_t holdTicks, const NoiseConfig &noise) {
 	const uint32_t pos = st.f32.callPos;
 	if (pos >= sampleCount || st.f32.callDrained != 0) return kClsDone;
 	const uint32_t left = sampleCount - pos;
 	if (left >= holdTicks && canHoldF32T(st.fm, st.f32, holdTicks)) return kClsHold;
-	if (left >= kCellTicks && canFadeF32T(st.fm, st.f32, kCellTicks)) return kClsFade;
+	if (left >= kCellTicks && canFadeF32T(st.fm, st.f32, kCellTicks, noise)) return kClsFade;
 	return kClsGen;
 }
 
@@ -205,7 +205,7 @@ klatt_f32_block_kernel(const StreamDesc *__restrict__ descs, StreamStateLite *__
 	}
 	__syncthreads();
 	for (uint32_t l = tid; l < owned; l += kBlkThreads) {
-		const uint32_t cls = classifyLite(lite[blockIdx.x + l * gridDim.x], sampleCount, holdTicks);
+		const uint32_t cls = classifyLite(lite[blockIdx.x + l * gridDim.x], sampleCount, holdTicks, noise);
 		if (cls < kClsDone) {
 			const uint32_t idx = atomicAdd(&ctl->count[cls], 1u);
 			ring[cls * cap + (idx & mask)] = (uint16_t)l;
@@ -351,7 +351,7 @@ klatt_f32_block_kernel(const StreamDesc *__restrict__ descs, StreamStateLite *__
 		}
 		xc.sync();  // both halves of every stream of this cell are in the staged records
 		uint32_t next = kClsExit;
-		if (cascade && valid) next = classifyLite(*st, sampleCount, holdTicks);
+		if (cascade && valid) next = classifyLite(*st, sampleCount, holdTicks, noise);
 		// ---- shared -> global (the idle lanes' dummy is not written back) ----
 #pragma unroll 1
 		for (uint32_t idx = tw; idx < 32u * kRecPieces; idx += 64u) {

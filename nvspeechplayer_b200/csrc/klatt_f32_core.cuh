@@ -687,11 +687,17 @@ KLATT_HD bool canHoldF32T(const FM &fm, const GS &gs, uint32_t ticks) {
 }
 KLATT_HD bool canHoldF32(const StreamState &st, uint32_t ticks) { return canHoldF32T(st.fm, st.gen.f32, ticks); }
 // `ticks` ticks ahead are all INTERIOR fade ticks (frame.cpp:49-52 with 1 <= sampleCounter < fade length, no event among
-// them) and the first of them falls on the 64-sample grid of the drift control: renderFadeF32T may run them
+// them) and the first of them falls on the 64-sample grid of the drift control
 template <class FM, class GS>
 KLATT_HD bool canFadeF32T(const FM &fm, const GS &gs, uint32_t ticks) {
 	return fm.hasNew && !fm.purgePending && fm.counter >= 1 && (uint64_t)fm.counter + ticks < (uint64_t)fm.newF &&
 	       (gs.samplesGenerated & (uint64_t)(kCoarseTicks - 1)) == 0;
+}
+// ... and the stream's noise is Philox: renderFadeF32T may run them.  The fade loop draws Philox noise only, so a stream under
+// any other noise mode takes the general loop for its interior fades.  Every caller that picks the loop for a stream asks this.
+template <class FM, class GS>
+KLATT_HD bool canFadeF32T(const FM &fm, const GS &gs, uint32_t ticks, const NoiseConfig &noise) {
+	return noise.mode == kNoisePhilox && canFadeF32T(fm, gs, ticks);
 }
 
 template <int ROLE, class Out, class Xchg, class FM, class GS>
@@ -1101,7 +1107,8 @@ KLATT_HD uint32_t renderGeneralF32(const StreamDesc &desc, int sampleRate, uint3
 // re-basing happens before the loop and a tick is pole recurrences -> coefficients -> the DSP with no branch.  The
 // arithmetic of every tick is renderGeneralF32T's, operation for operation: a stream may change between the two (and the
 // hold loop) at any chunk boundary without changing an output bit.  ticks is a multiple of kGroupTicks (any number of
-// kCoarseTicks cells); Philox noise only (pre-queued batches); even `samplesGenerated` follows from the grid condition.
+// kCoarseTicks cells); Philox noise only (canFadeF32T refuses every other mode); even `samplesGenerated` follows from the
+// grid condition.
 // ---------------------------------------------------------------------------------------------------
 template <int ROLE, class Out, class Xchg, class FM, class GS>
 KLATT_HD void renderFadeF32T(FM &fm, GS &gs, const StreamDesc &desc, int sampleRate, uint32_t ticks, Out &out, const NoiseConfig &noise,

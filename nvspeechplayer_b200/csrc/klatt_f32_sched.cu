@@ -103,15 +103,16 @@ __device__ __forceinline__ void stVolatile(uint32_t *p, uint32_t v) { *reinterpr
 
 // class of a stream's next chunk, or kClassExit when the call is complete for it
 template <class FM, class GS>
-__device__ __forceinline__ uint32_t classifyNextT(const FM &fm, const GS &gs, uint32_t sampleCount, uint32_t holdTicks, uint32_t fadeTicks) {
+__device__ __forceinline__ uint32_t classifyNextT(const FM &fm, const GS &gs, uint32_t sampleCount, uint32_t holdTicks, uint32_t fadeTicks,
+                                                   const NoiseConfig &noise) {
 	const uint32_t pos = gs.callPos;
 	if (pos >= sampleCount || gs.callDrained != 0) return kClassExit;
 	if (sampleCount - pos >= holdTicks && canHoldF32T(fm, gs, holdTicks)) return kClassHold;
-	if (fadeTicks != 0u && sampleCount - pos >= fadeTicks && canFadeF32T(fm, gs, fadeTicks)) return kClassFade;
+	if (fadeTicks != 0u && sampleCount - pos >= fadeTicks && canFadeF32T(fm, gs, fadeTicks, noise)) return kClassFade;
 	return kClassGen;
 }
-__device__ __forceinline__ uint32_t classifyNext(const StreamState *st, uint32_t sampleCount, uint32_t holdTicks) {
-	return classifyNextT(st->fm, st->gen.f32, sampleCount, holdTicks, 0u);
+__device__ __forceinline__ uint32_t classifyNext(const StreamState *st, uint32_t sampleCount, uint32_t holdTicks, const NoiseConfig &noise) {
+	return classifyNextT(st->fm, st->gen.f32, sampleCount, holdTicks, 0u, noise);
 }
 constexpr uint32_t kRecPieces = sizeof(StreamStateLite) / 16, kStageStride = sizeof(StreamStateLite) + 8, kStageBytes = 32 * kStageStride;
 constexpr uint32_t kHoldPiecesOut = (uint32_t)(offsetof(StreamStateLite, f32) + offsetof(GenStateF32Lite, zre)) / 16;  // everything before the pole state
@@ -257,18 +258,19 @@ __device__ __forceinline__ uint32_t schedClaim(SchedCtl *ctl, uint32_t *ring, ui
 // start of a call: reset the per-call cursors of every stream and seed the rings
 __global__ void __launch_bounds__(256)
 klatt_sched_seed_kernel(const StreamDesc *__restrict__ descs, const StreamStateLite *__restrict__ lite, uint32_t numStreams,
-                        uint32_t sampleCount, uint32_t holdTicks, uint32_t fadeTicks, SchedCtl *ctl, uint32_t *ring, uint32_t ringCap) {
+                        uint32_t sampleCount, uint32_t holdTicks, uint32_t fadeTicks, NoiseConfig noise, SchedCtl *ctl, uint32_t *ring,
+                        uint32_t ringCap) {
 	const uint32_t s = blockIdx.x * blockDim.x + threadIdx.x;
 	const bool valid = s < numStreams;
 	uint32_t cls = kClassExit;
 	if (valid) {
 		if (lite) {  // (the import kernel has reset the per-call cursors)
-			cls = classifyNextT(lite[s].fm, lite[s].f32, sampleCount, holdTicks, fadeTicks);
+			cls = classifyNextT(lite[s].fm, lite[s].f32, sampleCount, holdTicks, fadeTicks, noise);
 		} else {
 			StreamState *st = descs[s].state;
 			st->gen.f32.callPos = 0;
 			st->gen.f32.callDrained = 0;
-			cls = classifyNext(st, sampleCount, holdTicks);
+			cls = classifyNext(st, sampleCount, holdTicks, noise);
 		}
 	}
 	schedPush<true>(ctl, ring, ringCap, cls, s, valid);
@@ -425,7 +427,7 @@ klatt_f32_sched_kernel(const StreamDesc *__restrict__ descs, StreamStateLite *__
 		}
 #if KLATT_SCHED_LITE
 		xc.sync();  // both halves of every stream of this chunk are in the staged records
-		const uint32_t next = (cascade && valid) ? classifyNextT(fm, gs, sampleCount, holdTicks, fadeTicks) : kClassExit;
+		const uint32_t next = (cascade && valid) ? classifyNextT(fm, gs, sampleCount, holdTicks, fadeTicks, noise) : kClassExit;
 		// (a hold chunk only moves the frame-manager counters, the oscillators, the noise memories and the section memories:
 		// the first 256 bytes of a record; the pole state, the direct parameters and the drift-control record are unchanged)
 		const uint32_t piecesOut = cls == kClassHold ? kHoldPiecesOut : kRecPieces;
@@ -448,7 +450,7 @@ klatt_f32_sched_kernel(const StreamDesc *__restrict__ descs, StreamStateLite *__
 #endif
 		if (cascade) {
 #if !KLATT_SCHED_LITE
-			const uint32_t next = valid ? classifyNext(desc.state, sampleCount, holdTicks) : kClassExit;
+			const uint32_t next = valid ? classifyNext(desc.state, sampleCount, holdTicks, noise) : kClassExit;
 #endif
 			schedPush<false>(ctl, ring, ringCap, next, s, valid);
 		}
@@ -497,7 +499,7 @@ cudaError_t launchKlattF32Sched(const StreamDesc *descs, uint32_t numStreams, in
 	// paired workers: two warps per batch, two batches per block
 	const uint32_t blocksWanted = (batches + 1) / 2, grid = blocksWanted < numBlocks ? blocksWanted : numBlocks;
 	if (lite && (e = launchKlattLiteImport(descs, numStreams, 2 * grid, lite, stream)) != cudaSuccess) return e;
-	klatt_sched_seed_kernel<<<(numStreams + 255) / 256, 256, 0, stream>>>(descs, lite, numStreams, sampleCount, holdTicks, fadeTicks, ctl, ring, ringCap);
+	klatt_sched_seed_kernel<<<(numStreams + 255) / 256, 256, 0, stream>>>(descs, lite, numStreams, sampleCount, holdTicks, fadeTicks, noise, ctl, ring, ringCap);
 	// NVSP_L2_PERSIST=1: pin the record array in the L2 (persisting access-policy window on the launching stream).  Measured
 	// (DESIGN.md section 5d): DRAM traffic of a config-3 step 59.7 -> 51.5 GB, but every workload gets SLOWER in warm
 	// back-to-back steps (config 3 +1.2 %, config 5 +3.3 %, config 2 -- 190 MB of records against a 79 MB set-aside -- +8 %),

@@ -8,6 +8,8 @@
 //   mode 0  one general-kernel pass per `chunk` ticks, plans made inline at the pop tick (per-handle API)
 //   mode 1  plans precomputed for the whole queue (klatt_plan_kernel), then ROUNDS: a stream with at least holdTicks
 //           pure hold ticks ahead runs renderHoldF32(holdTicks), otherwise renderGeneralF32(genTicks)
+// Both render entries take Philox noise keyed (seed, streamId), or, given `replay`, the caller's draws (draw 2g / 2g+1 of
+// generated sample g, 0 past replayLen) as a batch under SPEECHPLAYER_NOISE_REPLAY feeds them.
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -27,7 +29,8 @@ struct ArrayOut {
 extern "C" int hostsim_render_f32(int sampleRate, const double *frames, const uint32_t *minDur, const uint32_t *fadeDur,
                                   const int32_t *userIndex, const uint8_t *isNull, uint32_t nFrames, uint64_t seed,
                                   uint64_t streamId, uint32_t maxSamples, int16_t *out, uint32_t chunk, int32_t *lastIndexOut,
-                                  int mode, uint32_t holdTicks, uint32_t genTicks, uint32_t *holdTicksUsedOut) {
+                                  int mode, uint32_t holdTicks, uint32_t genTicks, uint32_t *holdTicksUsedOut, const int32_t *replay,
+                                  uint64_t replayLen) {
 	StreamState *st = (StreamState *)calloc(1, sizeof(StreamState));
 	st->fm.lastUserIndex = -1;
 	st->fm.curIsNull = 1;
@@ -36,6 +39,7 @@ extern "C" int hostsim_render_f32(int sampleRate, const double *frames, const ui
 	memset(&d, 0, sizeof d);
 	d.state = st; d.frames = frames; d.minDur = minDur; d.fadeDur = fadeDur; d.userIndex = userIndex; d.isNull = isNull;
 	d.qCount = nFrames; d.qBase = 0; d.streamId = streamId;
+	d.replay = replay; d.replayLen = replay ? replayLen : 0; d.replayBase = 0;
 	std::vector<FadePlanF32> plans;
 	if (mode == 1) {
 		plans.resize(nFrames);
@@ -53,7 +57,7 @@ extern "C" int hostsim_render_f32(int sampleRate, const double *frames, const ui
 		d.plans = plans.data();
 	}
 	NoiseConfig nc;
-	nc.mode = kNoisePhilox; nc.seed = seed;
+	nc.mode = replay ? kNoiseReplay : kNoisePhilox; nc.seed = seed;
 	uint32_t total = 0, holdUsed = 0;
 	int32_t lui = -1;
 	uint32_t qh = 0;
@@ -89,7 +93,8 @@ extern "C" int hostsim_render_f32(int sampleRate, const double *frames, const ui
 extern "C" int hostsim_render_f32_cells(int sampleRate, const double *frames, const uint32_t *minDur, const uint32_t *fadeDur,
                                         const int32_t *userIndex, const uint8_t *isNull, uint32_t nFrames, uint64_t seed,
                                         uint64_t streamId, uint32_t maxSamples, int16_t *out, uint32_t holdTicks, uint32_t fadeTicks,
-                                        uint32_t *ticksByClass /* [3]: hold, fade, general */, int32_t *lastIndexOut, uint32_t fadeMax) {
+                                        uint32_t *ticksByClass /* [3]: hold, fade, general */, int32_t *lastIndexOut, uint32_t fadeMax,
+                                        const int32_t *replay, uint64_t replayLen) {
 	StreamStateLite *st = (StreamStateLite *)calloc(1, sizeof(StreamStateLite));
 	st->fm.lastUserIndex = -1;
 	st->fm.curIsNull = 1;
@@ -98,6 +103,7 @@ extern "C" int hostsim_render_f32_cells(int sampleRate, const double *frames, co
 	memset(&d, 0, sizeof d);
 	d.state = nullptr; d.frames = frames; d.minDur = minDur; d.fadeDur = fadeDur; d.userIndex = userIndex; d.isNull = isNull;
 	d.qCount = nFrames; d.qBase = 0; d.streamId = streamId;
+	d.replay = replay; d.replayLen = replay ? replayLen : 0; d.replayBase = 0;
 	std::vector<FadePlanF32> plans(nFrames);
 	int prevReal = -1;
 	for (uint32_t j = 0; j < nFrames; ++j) {
@@ -111,7 +117,7 @@ extern "C" int hostsim_render_f32_cells(int sampleRate, const double *frames, co
 	}
 	d.plans = plans.data();
 	NoiseConfig nc;
-	nc.mode = kNoisePhilox; nc.seed = seed;
+	nc.mode = replay ? kNoiseReplay : kNoisePhilox; nc.seed = seed;
 	uint32_t total = 0;
 	uint32_t used[3] = {0, 0, 0};
 	int32_t lui = -1;
@@ -126,7 +132,7 @@ extern "C" int hostsim_render_f32_cells(int sampleRate, const double *frames, co
 			lui = st->fm.lastUserIndex;
 			continue;
 		}
-		if (left >= fadeTicks && canFadeF32T(st->fm, st->f32, fadeTicks)) {
+		if (left >= fadeTicks && canFadeF32T(st->fm, st->f32, fadeTicks, nc)) {
 			// (the ring scheduler stretches a fade chunk to the interior fade ticks its streams have left, in whole cells)
 			uint32_t ticks = fadeTicks;
 			if (fadeMax > fadeTicks) {

@@ -18,18 +18,26 @@ def lib():
         vp = ctypes.c_void_p
         L.hostsim_render_f32.restype = ctypes.c_int
         L.hostsim_render_f32.argtypes = [ctypes.c_int, vp, vp, vp, vp, vp, ctypes.c_uint, ctypes.c_uint64, ctypes.c_uint64,
-                                         ctypes.c_uint, vp, ctypes.c_uint, vp, ctypes.c_int, ctypes.c_uint, ctypes.c_uint, vp]
+                                         ctypes.c_uint, vp, ctypes.c_uint, vp, ctypes.c_int, ctypes.c_uint, ctypes.c_uint, vp, vp,
+                                         ctypes.c_uint64]
         L.hostsim_render_f32_cells.restype = ctypes.c_int
         L.hostsim_render_f32_cells.argtypes = [ctypes.c_int, vp, vp, vp, vp, vp, ctypes.c_uint, ctypes.c_uint64, ctypes.c_uint64,
-                                               ctypes.c_uint, vp, ctypes.c_uint, ctypes.c_uint, vp, vp]
+                                               ctypes.c_uint, vp, ctypes.c_uint, ctypes.c_uint, vp, vp, ctypes.c_uint, vp, ctypes.c_uint64]
         _lib = L
     return _lib
 
 
+def _replay_args(replay):
+    if replay is None:
+        return None, 0
+    d = np.ascontiguousarray(replay, dtype=np.int32)
+    return d.ctypes.data_as(ctypes.c_void_p), d.size
+
+
 def render_f32_cells(sr, frames, min_dur, fade_dur, is_null=None, user_index=None, max_samples=None, seed=0, stream=0,
-                     hold_ticks=128, fade_ticks=64, fade_max=0):
+                     hold_ticks=128, fade_ticks=64, fade_max=0, replay=None):
     """The block scheduler's execution model on one stream: compact state, hold / fade / general cells.  Returns
-    (pcm, last_index, [hold ticks, fade ticks, general ticks])."""
+    (pcm, last_index, [hold ticks, fade ticks, general ticks]).  replay: int32 draws instead of Philox noise (seed, stream)."""
     frames = np.ascontiguousarray(frames, dtype=np.float64).reshape(-1, 47)
     m = np.ascontiguousarray(min_dur, dtype=np.uint32)
     f = np.ascontiguousarray(fade_dur, dtype=np.uint32)
@@ -44,14 +52,15 @@ def render_f32_cells(sr, frames, min_dur, fade_dur, is_null=None, user_index=Non
     li = ctypes.c_int32(0)
     used = (ctypes.c_uint32 * 3)()
     n = lib().hostsim_render_f32_cells(sr, ptr(frames), ptr(m), ptr(f), ptr(ux), ptr(nul), len(m), seed, stream, max_samples,
-                                       ptr(out), hold_ticks, fade_ticks, used, ctypes.byref(li), fade_max)
+                                       ptr(out), hold_ticks, fade_ticks, used, ctypes.byref(li), fade_max, *_replay_args(replay))
     return out[:n], li.value, list(used)
 
 
 def render_f32(sr, frames, min_dur, fade_dur, is_null=None, user_index=None, max_samples=None, seed=0, stream=0, chunk=0,
-               planned=False, hold_ticks=0, gen_ticks=0, return_hold=False):
+               planned=False, hold_ticks=0, gen_ticks=0, return_hold=False, replay=None):
     """planned=False: inline plans, one general pass per `chunk` ticks.  planned=True: precomputed plans and rounds of
-    hold_ticks pure-hold / gen_ticks general chunks, as the batch engine schedules them."""
+    hold_ticks pure-hold / gen_ticks general chunks, as the batch engine schedules them.  replay: int32 draws instead of
+    Philox noise (seed, stream)."""
     frames = np.ascontiguousarray(frames, dtype=np.float64).reshape(-1, 47)
     m = np.ascontiguousarray(min_dur, dtype=np.uint32)
     f = np.ascontiguousarray(fade_dur, dtype=np.uint32)
@@ -67,7 +76,7 @@ def render_f32(sr, frames, min_dur, fade_dur, is_null=None, user_index=None, max
     hold = ctypes.c_uint32(0)
     n = lib().hostsim_render_f32(sr, ptr(frames), ptr(m), ptr(f), ptr(ux), ptr(nul), len(m), seed, stream, max_samples,
                                  ptr(out), chunk, ctypes.byref(li), int(bool(planned)), hold_ticks, gen_ticks,
-                                 ctypes.byref(hold))
+                                 ctypes.byref(hold), *_replay_args(replay))
     if return_hold:
         return out[:n], li.value, hold.value
     return out[:n], li.value

@@ -8,6 +8,7 @@ import pytest
 from nvspeechplayer_b200 import workloads
 from tests import parity, scenarios
 from tests.hostsim import sim
+from tests.noise import noisy, philox_draws
 
 
 def test_config1_f32_arithmetic(port, golden_config1):
@@ -85,6 +86,25 @@ def test_cells_equal_one_shot_bitwise(golden_config1, hold, fade):
         got, _, used = sim.render_f32_cells(16000, fr, m, f, nul, ux, seed=8, stream=s, hold_ticks=hold, fade_ticks=fade)
         np.testing.assert_array_equal(got, one)
         assert used[1] > 0.4 * len(one), used   # 60 % of these ticks are fade ticks
+    _replay_cells_equal_one_shot(hold, fade, 0)
+
+
+def _replay_cells_equal_one_shot(hold, fade, fade_max):
+    """A replay stream under the cells model renders its caller's draws: the fade loop draws Philox noise only, so interior
+    fades must go to the general loop.  The draws are the Philox words of another key (>> 1): a fade cell that drew the
+    stream's own key would change the bits, and the one-shot render under that other key is the answer."""
+    fb = workloads.vowel_chart(1, pairs=2)
+    for s in range(fb.num_streams):
+        fr, m, f, nul, ux = fb.stream(s)
+        fr = noisy(fr)   # the vowels are voiced only: give the noise a way into the output
+        one, _ = sim.render_f32(16000, fr, m, f, nul, ux, seed=0x51, stream=(1 << 40) + s)
+        draws = philox_draws(0x51, (1 << 40) + s, 2 * len(one))
+        rep, _ = sim.render_f32(16000, fr, m, f, nul, ux, seed=8, stream=s, replay=draws)
+        np.testing.assert_array_equal(rep, one)
+        got, _, used = sim.render_f32_cells(16000, fr, m, f, nul, ux, seed=8, stream=s, hold_ticks=hold, fade_ticks=fade,
+                                            fade_max=fade_max, replay=draws)
+        np.testing.assert_array_equal(got, one)
+        assert used[1] == 0, used
 
 
 @pytest.mark.parametrize("hold,fade,fade_max", [(256, 128, 0), (256, 128, 512), (256, 64, 4096), (256, 192, 320)])
@@ -109,3 +129,4 @@ def test_long_fade_chunks_equal_one_shot_bitwise(hold, fade, fade_max):
         got, _, used = sim.render_f32_cells(16000, fr, m, f, nul, ux, seed=8, stream=s, hold_ticks=hold, fade_ticks=fade, fade_max=fade_max)
         np.testing.assert_array_equal(got, one)
         assert used[1] > 0.4 * len(one), used
+    _replay_cells_equal_one_shot(hold, fade, fade_max)
